@@ -2,6 +2,7 @@
 """bench.py -- GCUPS of the database-search hot path on N B200s, beside the reference on host cores.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload config3|config2]
+                  [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[2], the largest single-GPU configuration: the 20 customary query
 lengths 144 ... 5478 in the modes NW, HW and OV (score + end location) against the synthetic 570k-sequence /
@@ -219,6 +220,25 @@ def run_reference_arm(args, rank):
     print(json.dumps(line), flush=True)
 
 
+# ----------------------------------------------------------------------------- output dump
+DUMP_TARGETS = 32768  # 60 searches x 3 arrays x 32,768 targets in float64 = 47 MB: a dump stays under 64 MB
+DUMP_UNWRITTEN = np.iinfo(np.int32).min  # in a dump: an entry the last step did not write (no score or location)
+
+
+def dump_outputs(path, arrays, n):
+    """Writes the result arrays of the last timed step as <path>/<name>.npy in float64 (int32 values, exact), for
+    comparing two builds output for output.  A database of more than DUMP_TARGETS targets is sampled: the same seeded
+    choice of target indices every run, written beside them as target_index.npy.  Rows of a batch are the searches in
+    the order they were issued."""
+    cols = np.arange(n)
+    if n > DUMP_TARGETS:
+        cols = np.sort(np.random.default_rng(0).choice(n, DUMP_TARGETS, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "target_index.npy"), cols.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a[..., cols].astype(np.float64))
+
+
 # ----------------------------------------------------------------------------- B200 arm
 def run_b200_arm(args, rank, local_rank, world):
     import torch
@@ -264,18 +284,20 @@ def run_b200_arm(args, rank, local_rank, world):
         order = [order[k // 2] if k % 2 == 0 else order[nq - 1 - k // 2] for k in range(nq)]
     searches = [(w.queries[k], mode) for k in order for mode in w.modes]
     out = None if single else tuple(np.zeros((len(searches), n), dtype=np.int32) for _ in range(3))
+    last = {}  # what the latest step returned to its caller: score, end in query, end in target
 
     def step_resident():
         """One sweep against the resident database; returns (device ms, kernel launches)."""
         flush.zero_()
         torch.cuda.synchronize()
         if single:
-            rc, sc, _, _, ms = handle.search(w.queries[0], GAP_OPEN, GAP_EXT, mat, A, w.search_type, w.modes[0])
+            rc, sc, eq, et, ms = handle.search(w.queries[0], GAP_OPEN, GAP_EXT, mat, A, w.search_type, w.modes[0])
         else:  # one batch: every (query, mode) of the step, several in flight
-            rc, sc, _, _, ms = handle.search_batch([q for q, _ in searches], GAP_OPEN, GAP_EXT, mat, A, w.search_type,
-                                                   [m for _, m in searches], in_flight=args.in_flight, out=out)
+            rc, sc, eq, et, ms = handle.search_batch([q for q, _ in searches], GAP_OPEN, GAP_EXT, mat, A, w.search_type,
+                                                     [m for _, m in searches], in_flight=args.in_flight, out=out)
         if rc != 0:
             raise SystemExit(f"search failed rc={rc}: {eng.last_error()}")
+        last.update(score=sc, end_query=eq, end_target=et)
         return ms, handle.last_stats()["kernel_launches"]
 
     # ---- device-timed value (database resident)
@@ -285,14 +307,22 @@ def run_b200_arm(args, rank, local_rank, world):
     barrier()
     clocks.start()
     wall0 = time.perf_counter()
-    dev_ms, launches = 0.0, 0
-    for _ in range(args.steps):
+    dev_ms, launches, untimed = 0.0, 0, 0.0
+    for step in range(args.steps):
+        if args.dump_outputs and out is not None and step == args.steps - 1:
+            # the batch keeps old values where it computes nothing: a sentinel makes the dump show only the last step
+            t0 = time.perf_counter()
+            for a in out:
+                a.fill(DUMP_UNWRITTEN)
+            untimed += time.perf_counter() - t0
         ms, ln = step_resident()
         dev_ms += ms
         launches += ln
     barrier()
-    wall_resident = time.perf_counter() - wall0
+    wall_resident = time.perf_counter() - wall0 - untimed
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, n)
     t_dev = reduce(dev_ms / 1e3, "MAX")
     t_wall = reduce(wall_resident, "MAX")
     total_cells = reduce(cells_rank, "SUM") * args.steps
@@ -469,7 +499,13 @@ def main():
     ap.add_argument("--shard-of", type=int, default=0, help="development: run one shard of an M-way deal on one GPU")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/<name>.npy "
+                    "(rank 0's shard; float64, a fixed sample of the targets of a large database)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the B200 arm (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -13,6 +13,10 @@ Vectors (each one also names the reference fixture it comes from):
                  OPAL_OVERFLOW_SIMPLE: per-target score/end/start + alignment digest, and `Maximum`
   protein.json   seeded random protein DB (BLOSUM62 11/1), 4 modes score+end; SW alignments
   api.json       reuse rule, CharSW, invalid mode (SURVEY.md section 4, probes B-D)
+  oracle_vs_ref.json
+                 every call tests/test_oracle_vs_ref.py compares (seeded random protein and small-alphabet cases,
+                 score+end, SW alignments, per-target NW/HW/OV alignments): (rc, records), null where the
+                 reference crashed.  `python tests/golden/make_golden.py oracle_vs_ref` writes this file alone.
 """
 import json
 import os
@@ -118,7 +122,16 @@ def main():
     rc, res = ref.search_database(README_QUERY, db, 3, 1, README_MATRIX, 4, res, 0, 7, OPAL_OVERFLOW_SIMPLE)
     out["invalid_mode"] = {"rc": rc, "results": dump_results(res)}
     save("api.json", out)
+    oracle_vs_ref(ref)
+
+
+def oracle_vs_ref(ref):
+    from test_oracle_vs_ref import all_cases, run_reference
+    save("oracle_vs_ref.json", {key: run_reference(ref, args) for key, args in all_cases()})
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["oracle_vs_ref"]:
+        oracle_vs_ref(OpalCLibrary(REF_SO))
+    else:
+        main()

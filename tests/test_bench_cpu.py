@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -42,6 +43,26 @@ def test_reference_arm_other_ranks_exit_without_work():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--workload", "config2"],
                        capture_output=True, text=True, timeout=300, env=env, cwd=ROOT)
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+@pytest.mark.parametrize("shape", [(1000,), (60, 100000)])
+def test_dump_outputs_writes_the_same_float64_sample_every_run(tmp_path, shape):
+    import bench
+    n = shape[-1]
+    rng = np.random.default_rng(5)
+    arrays = {name: rng.integers(-2 ** 20, 2 ** 20, shape, dtype=np.int32) for name in ("score", "end_query", "end_target")}
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays, n)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["end_query.npy", "end_target.npy", "score.npy", "target_index.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 << 20
+    cols = np.load(tmp_path / "a" / "target_index.npy").astype(np.int64)
+    assert len(cols) == min(n, bench.DUMP_TARGETS) and (np.diff(cols) > 0).all()
+    for f in files:
+        got = np.load(tmp_path / "a" / f)
+        assert got.dtype == np.float64 and (got == np.load(tmp_path / "b" / f)).all()
+    for name, a in arrays.items():
+        assert (np.load(tmp_path / "a" / f"{name}.npy") == a[..., cols]).all()
 
 
 def test_product_arm_fails_loudly_without_a_gpu():

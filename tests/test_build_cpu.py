@@ -5,16 +5,23 @@ import os
 import re
 import shutil
 import subprocess
+import sys
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BUILD = os.path.join(ROOT, "opal_b200", "csrc", "build")
+# cuobjdump of the toolkit whose nvcc opal_b200/csrc/Makefile compiles with (NVCC ?= /usr/local/cuda/bin/nvcc), else
+# from PATH; the tools below call it by name
+CUOBJDUMP = os.path.join(os.path.dirname(os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")), "cuobjdump")
+if not os.path.exists(CUOBJDUMP):
+    CUOBJDUMP = shutil.which("cuobjdump") or CUOBJDUMP
+TOOL_ENV = dict(os.environ, PATH=os.path.dirname(CUOBJDUMP) + os.pathsep + os.environ.get("PATH", ""))
 
 
 def _objects():
     objs = sorted(glob.glob(os.path.join(BUILD, "kernels_R*.o")))
-    if not objs or shutil.which("cuobjdump") is None:
+    if not objs or not os.path.exists(CUOBJDUMP):
         pytest.skip("no built kernel objects / cuobjdump (run __graft_entry__.build() first)")
     return objs
 
@@ -23,7 +30,7 @@ def test_kernel_objects_are_sm_100a_packed_dpx_code():
     obj = os.path.join(BUILD, "kernels_R17.o")
     if obj not in _objects():
         pytest.skip("R = 17 not built")
-    sass = subprocess.run(["cuobjdump", "-sass", obj], capture_output=True, text=True, check=True).stdout
+    sass = subprocess.run([CUOBJDUMP, "-sass", obj], capture_output=True, text=True, check=True).stdout
     assert "sm_100a" in sass or "SM100a" in sass or "EF_CUDA_SM100" in sass
     for mnemonic in ("VIADDMNMX.S16x2", "VIADDMNMX.S16x2.RELU", "VIMNMX3.S16x2", "VIADD.16x2", "LDS.128", "SHFL.IDX"):
         assert mnemonic in sass, mnemonic
@@ -37,8 +44,8 @@ def test_sweep_loop_instruction_mix_matches_the_design():
     obj = os.path.join(BUILD, "kernels_R17.o")
     if obj not in _objects():
         pytest.skip("R = 17 not built")
-    out = subprocess.run(["python", os.path.join(ROOT, "tools", "sass_loop.py"), obj, "3"], capture_output=True, text=True,
-                         check=True).stdout
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "sass_loop.py"), obj, "3"], capture_output=True, text=True,
+                         check=True, env=TOOL_ENV).stdout
     first = out.split("  loop ")[1]
     counts = {m.group(1): int(m.group(2)) for m in re.finditer(r"ALU\s+(\S+)\s+(\d+)", first)}
     assert counts.get("VIADDMNMX.16x2") == 68
@@ -72,8 +79,8 @@ def test_tall_global_strips_keep_their_loop_invariants_in_registers():
     obj = os.path.join(BUILD, "kernels_R32.o")
     if obj not in _objects():
         pytest.skip("R = 32 not built")
-    out = subprocess.run(["python", os.path.join(ROOT, "tools", "sass_hot_path.py"), obj, "2", "Packed16", "384"], capture_output=True,
-                         text=True, check=True).stdout
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "sass_hot_path.py"), obj, "2", "Packed16", "384"], capture_output=True,
+                         text=True, check=True, env=TOOL_ENV).stdout
     loops = re.findall(r"hot path (\d+): ALU=(\d+).*\n\s+(.*)", out)
     # (the tool also lists the task loop around them, which holds the epilogue and several hundred instructions more)
     sweeps = [(int(n), int(alu), ops) for n, alu, ops in loops if "VIADDMNMX=128" in ops and int(n) < 320]
