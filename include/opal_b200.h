@@ -81,6 +81,26 @@ int opalb200_db_search(OpalB200Db* handle, const unsigned char query[], int quer
                        int* scores, int* endQuery, int* endTarget, float* deviceMs);
 
 /*
+ * Searches with a position-specific scoring matrix (PSSM) instead of a query and a substitution matrix: pssm is
+ * queryLength x alphabetLength ints, row-major, and pssm[r * alphabetLength + y] is the score of query position r
+ * against database residue code y (as from PSI-BLAST, a family alignment or any per-position scoring).  Everything
+ * else is the matrix search: modes, gaps, search types, end-location tie-breaking, skip rule, results of empty
+ * queries / targets.  pssm[r * A + y] = scoreMatrix[query[r] * A + y] gives exactly the scores and end locations of
+ * the matrix search with (query, scoreMatrix).  Argument rules are the matrix rules, with the extremes taken over all
+ * queryLength x alphabetLength entries (OPAL_ERR_OVERFLOW for an entry outside (INT_MIN / 2, INT_MAX / 2));
+ * pssm may be NULL only when queryLength is 0 (otherwise OPAL_ERR_INVALID_ARGUMENT).
+ * The alignment stage (the _results_pssm / _topk_pssm calls below, OPAL_SEARCH_ALIGNMENT) restates the reference's band
+ * (calculateBandBorders) with M = the largest of all PSSM entries instead of the largest matrix entry.  It also takes
+ * the residues the PSSM was built for (query, codes < alphabetLength, required at OPAL_SEARCH_ALIGNMENT and ignored
+ * otherwise); they are used only to label diagonal steps OPAL_ALIGN_MATCH / OPAL_ALIGN_MISMATCH.
+ *
+ * Same outputs as opalb200_db_search.
+ */
+int opalb200_db_search_pssm(OpalB200Db* handle, const int* pssm, int queryLength, int alphabetLength,
+                            int gapOpen, int gapExt, int searchType, int mode, const unsigned char* skip,
+                            int* scores, int* endQuery, int* endTarget, float* deviceMs);
+
+/*
  * numQueries searches against the resident database (config 3's protocol: many queries, one database), with up
  * to `inFlight` (1..16) queries on the device at a time so that the tail of one query overlaps the bulk of the
  * next and host-side planning / result publishing overlaps kernels.  Same arguments as opalb200_db_search;
@@ -101,6 +121,13 @@ int opalb200_db_search_batch_modes(OpalB200Db* handle, int numSearches, const un
                                    const int* scoreMatrix, int alphabetLength, int searchType,
                                    int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs);
 
+/* opalb200_db_search_batch_modes with one PSSM per search (pssms[s]: queryLengths[s] x alphabetLength, see
+ * opalb200_db_search_pssm). */
+int opalb200_db_search_batch_pssm(OpalB200Db* handle, int numSearches, const int* const pssms[],
+                                  const int queryLengths[], const int modes[], int alphabetLength,
+                                  int gapOpen, int gapExt, int searchType,
+                                  int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs);
+
 /*
  * opalSearchDatabase (reference src/opal.h:150-154) against the resident database: same result records, same
  * reuse rule for prefilled entries (:118-122), all three search levels including OPAL_SEARCH_ALIGNMENT --
@@ -110,6 +137,12 @@ int opalb200_db_search_batch_modes(OpalB200Db* handle, int numSearches, const un
 int opalb200_db_search_results(OpalB200Db* handle, const unsigned char query[], int queryLength,
                                int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength,
                                struct OpalSearchResult* results[], int searchType, int mode);
+
+/* opalb200_db_search_results with a PSSM (see opalb200_db_search_pssm; query labels the alignments' diagonal steps and
+ * may be NULL below OPAL_SEARCH_ALIGNMENT). */
+int opalb200_db_search_results_pssm(OpalB200Db* handle, const unsigned char query[], const int* pssm,
+                                    int queryLength, int alphabetLength, int gapOpen, int gapExt,
+                                    struct OpalSearchResult* results[], int searchType, int mode);
 
 /*
  * Score -> top-k -> alignment in one call on the resident database (BASELINE configs[3]: "SCORE pass, take the
@@ -123,6 +156,13 @@ int opalb200_db_search_results(OpalB200Db* handle, const unsigned char query[], 
 int opalb200_db_search_topk(OpalB200Db* handle, const unsigned char query[], int queryLength,
                             int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength,
                             int searchType, int mode, int k, int* indices, struct OpalSearchResult* results[], int* found);
+
+/* opalb200_db_search_topk with a PSSM (see opalb200_db_search_pssm; query labels the alignments' diagonal steps and may
+ * be NULL below OPAL_SEARCH_ALIGNMENT). */
+int opalb200_db_search_topk_pssm(OpalB200Db* handle, const unsigned char query[], const int* pssm,
+                                 int queryLength, int alphabetLength, int gapOpen, int gapExt,
+                                 int searchType, int mode, int k, int* indices,
+                                 struct OpalSearchResult* results[], int* found);
 
 /* Statistics of the last search on this handle: kernels launched, targets re-run in 32 bits, and the
  * geometry of the last launched class (threads per target pair, query rows per thread, passes over the

@@ -57,14 +57,16 @@ struct AlignOut {
 __device__ __forceinline__ int sat_sub(int x, int g) { return max(x - g, kNegInf); }
 
 // ---------------------------------------------------------------- kernel 1: DP + decision bits
+// With a PSSM (pssm non-NULL, Q x A) reversed row r is scored by PSSM row endQ - r instead of the matrix row of its query
+// letter; `matrixInSmem` then means that a pass's 32 x kRows rows of it are staged in shared memory.
 __global__ void __launch_bounds__(32) align_dp_kernel(const AlignTask* tasks, AlignOut* outs, const uint8_t* residues,
-                                                      const uint8_t* query, const int* matrix, int A, int Go, int Ge, int mode,
-                                                      uint32_t* flags, uint8_t* eqRows, int* bnd, int matrixInSmem) {
+                                                      const uint8_t* query, const int* matrix, const int* pssm, int A, int Go, int Ge,
+                                                      int mode, uint32_t* flags, uint8_t* eqRows, int* bnd, int matrixInSmem) {
     extern __shared__ int smemMatrix[];
     const AlignTask task = tasks[blockIdx.x];
     const int t = threadIdx.x;
-    const int* S = matrix;
-    if (matrixInSmem) {
+    const int* S = pssm ? pssm : matrix;
+    if (matrixInSmem && !pssm) {
         for (int i = t; i < A * A; i += 32) smemMatrix[i] = matrix[i];
         __syncwarp();
         S = smemMatrix;
@@ -78,13 +80,21 @@ __global__ void __launch_bounds__(32) align_dp_kernel(const AlignTask* tasks, Al
 
     for (int pass = 0; pass < passes; pass++) {
         const int row0 = (pass * 32 + t) * kRows;  // first reversed-query row of this thread
+        const int passRow0 = pass * 32 * kRows;
+        if (pssm && matrixInSmem) {  // this pass's PSSM rows, reversed: staged row i = PSSM row endQ - passRow0 - i
+            const int n = min(32 * kRows, Qp - passRow0) * A;
+            for (int i = t; i < n; i += 32) smemMatrix[i] = pssm[(size_t)(task.endQ - passRow0 - i / A) * A + i % A];
+            __syncwarp();
+            S = smemMatrix;
+        }
         int H[kRows], E[kRows], qoff[kRows];
 #pragma unroll
         for (int j = 0; j < kRows; j++) {
             const int r = row0 + j;
             H[j] = -Go - r * Ge;  // column -1 (src/opal.cpp:1266-1269)
             E[j] = kNegInf;
-            qoff[j] = (r < Qp) ? (int)query[task.endQ - r] * A : 0;
+            if (!pssm) qoff[j] = (r < Qp) ? (int)query[task.endQ - r] * A : 0;
+            else qoff[j] = (r < Qp) ? (matrixInSmem ? r - passRow0 : task.endQ - r) * A : 0;
         }
         int diag = (row0 == 0) ? 0 : -Go - (row0 - 1) * Ge;  // H[row0-1][-1]; the corner is 0
         int outH = kNegInf, outF = kNegInf;
@@ -261,16 +271,18 @@ bool band_borders(int k, int mode, int Q, int T, int Go, int Ge, int M, int* bot
 
 // Replay of an operation string (the check of reference src/test.cpp:348-422): does it start at
 // (sq, st), end at (endQ, endT) and score exactly `score`?
+// With a PSSM, query position qi scores by its row of the PSSM; q only labels the diagonal steps.
 bool replay_ok(const unsigned char* q, int Q, const unsigned char* t, int T, const unsigned char* ops, int n, int sq, int st,
-               int endQ, int endT, int score, int Go, int Ge, const int* S, int A) {
+               int endQ, int endT, int score, int Go, int Ge, const int* S, int A, const int* pssm) {
     i64 sc = 0;
     int qi = sq, ti = st, prev = -1;
     if (qi < 0 || ti < 0) return false;
+    auto cell = [&](int r, int y) -> i64 { return pssm ? pssm[(size_t)r * A + y] : S[q[r] * A + y]; };
     for (int i = 0; i < n; i++) {
         const int op = ops[i];
         if ((op != OPAL_ALIGN_DEL && ti >= T) || (op != OPAL_ALIGN_INS && qi >= Q)) return false;
-        if (op == OPAL_ALIGN_MATCH) { if (q[qi] != t[ti]) return false; sc += S[q[qi] * A + t[ti]]; qi++; ti++; }
-        else if (op == OPAL_ALIGN_MISMATCH) { if (q[qi] == t[ti]) return false; sc += S[q[qi] * A + t[ti]]; qi++; ti++; }
+        if (op == OPAL_ALIGN_MATCH) { if (q[qi] != t[ti]) return false; sc += cell(qi, t[ti]); qi++; ti++; }
+        else if (op == OPAL_ALIGN_MISMATCH) { if (q[qi] == t[ti]) return false; sc += cell(qi, t[ti]); qi++; ti++; }
         else if (op == OPAL_ALIGN_DEL) { sc -= (prev == OPAL_ALIGN_DEL ? Ge : Go); qi++; }
         else if (op == OPAL_ALIGN_INS) { sc -= (prev == OPAL_ALIGN_INS ? Ge : Go); ti++; }
         else return false;
@@ -293,7 +305,8 @@ bool replay_ok(const unsigned char* q, int Q, const unsigned char* t, int T, con
 }  // namespace
 
 int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned char* const* db, int n, const int* lens,
-                   int Go, int Ge, const int* matrix, int A, OpalSearchResult* results[], int mode, const int* subset) {
+                   int Go, int Ge, const int* matrix, int A, OpalSearchResult* results[], int mode, const int* subset,
+                   const int* pssm) {
     if (!ddb || !ddb->ensure_uploaded()) return OPAL_B200_ERR_CUDA;
     // target i on the host: the caller's pointer, or (resident-handle calls) the database's own sorted copy
     // record j describes database entry entry(j): all of them, or the given subset (top-k pipelines)
@@ -302,8 +315,11 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
     auto target_ptr = [&](int j) -> const unsigned char* {
         return db ? db[entry(j)] : ddb->h_residues() + ddb->offsets()[ddb->sorted_position()[entry(j)]];
     };
-    int M = matrix[0];
-    for (int i = 1; i < A * A; i++) M = std::max(M, matrix[i]);
+    // the band's M: the largest entry that can score a cell (matrix, or PSSM)
+    const int* scoreEntries = pssm ? pssm : matrix;
+    const long long numEntries = pssm ? (long long)Q * A : (long long)A * A;
+    int M = numEntries > 0 ? scoreEntries[0] : 0;
+    for (long long i = 1; i < numEntries; i++) M = std::max(M, scoreEntries[i]);
 
     // ---- entries that have an alignment at all (src/opal.cpp:1479-1483)
     std::vector<int> todo;
@@ -325,7 +341,7 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
     cudaSetDevice(ddb->device());
     bool ok = true;
     unsigned char* dQuery = nullptr;
-    int* dMatrix = nullptr;
+    int* dMatrix = nullptr;  // the matrix, or the PSSM
     AlignTask* dTasks = nullptr;
     AlignOut* dOuts = nullptr;
     uint32_t* dFlags = nullptr;
@@ -333,7 +349,9 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
     int* dBnd = nullptr;
     std::vector<unsigned char> hOps;
     std::vector<AlignOut> hOuts;
-    const int matrixInSmem = (size_t)A * A * 4 <= 40000 ? 1 : 0;
+    // matrix, or a pass's 32 x kRows PSSM rows, in shared memory when it fits
+    const size_t smemBytes = sizeof(int) * (size_t)A * (pssm ? 32 * kRows : A);
+    const int matrixInSmem = smemBytes <= 40000 ? 1 : 0;
     size_t freeB = 0, totalB = 0;
     cudaMemGetInfo(&freeB, &totalB);
     const long long budgetWords = (long long)std::max<size_t>(64u << 20, std::min<size_t>(freeB / 3, (size_t)16 << 30)) / 4;
@@ -346,9 +364,9 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
         dTasks = nullptr; dOuts = nullptr; dFlags = nullptr; dEq = nullptr; dOps = nullptr; dBnd = nullptr;
     };
     ALIGN_OK(dalloc(&dQuery, (size_t)Q + 16));
-    ALIGN_OK(dalloc(&dMatrix, sizeof(int) * A * A));
+    ALIGN_OK(dalloc(&dMatrix, sizeof(int) * (size_t)numEntries));
     ALIGN_TRY(cudaMemcpyAsync(dQuery, query, Q, cudaMemcpyHostToDevice, stream));
-    ALIGN_TRY(cudaMemcpyAsync(dMatrix, matrix, sizeof(int) * A * A, cudaMemcpyHostToDevice, stream));
+    ALIGN_TRY(cudaMemcpyAsync(dMatrix, scoreEntries, sizeof(int) * (size_t)numEntries, cudaMemcpyHostToDevice, stream));
 
     {
         // Two rounds at most: the reference's band first, the full band for entries whose replay fails.
@@ -389,8 +407,9 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
                 ALIGN_TRY(cudaMemcpyAsync(dTasks, tasks.data(), sizeof(AlignTask) * nt, cudaMemcpyHostToDevice, stream));
                 // an alignment is shorter than its slot: the unused tail travels back with the rest, so it is defined
                 ALIGN_TRY(cudaMemsetAsync(dOps, 0, (size_t)opsBytes, stream));
-                align_dp_kernel<<<nt, 32, matrixInSmem ? A * A * 4 : 0, stream>>>(dTasks, dOuts, ddb->d_residues(), dQuery, dMatrix, A, Go,
-                                                                                   Ge, mode, dFlags, dEq, dBnd, matrixInSmem);
+                align_dp_kernel<<<nt, 32, matrixInSmem ? smemBytes : 0, stream>>>(dTasks, dOuts, ddb->d_residues(), dQuery,
+                                                                                   pssm ? nullptr : dMatrix, pssm ? dMatrix : nullptr, A,
+                                                                                   Go, Ge, mode, dFlags, dEq, dBnd, matrixInSmem);
                 ALIGN_TRY(cudaGetLastError());
                 align_traceback_kernel<<<(nt + 63) / 64, 64, 0, stream>>>(dTasks, dOuts, nt, ddb->d_residues(), dQuery, mode, dFlags, dEq,
                                                                            dOps);
@@ -408,7 +427,7 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
                     const unsigned char* ops = hOps.data() + tk.opsOffset;
                     const int sq = tk.endQ - o.endRow, st = tk.endT - o.stopCol;  // src/opal.cpp:1499-1500
                     const bool good = o.status == 0 && replay_ok(query, Q, target_ptr(i), target_len(i), ops, o.opsLen, sq, st, tk.endQ, tk.endT,
-                                                                 tk.score, Go, Ge, matrix, A);
+                                                                 tk.score, Go, Ge, matrix, A, pssm);
                     if (!good && round == 0 && (tk.bottom != tk.Qp - 1 || tk.top != tk.Tp - 1)) { failed.push_back(i); continue; }
                     if (o.status != 0) {  // prefilled score / end inconsistent with the sequences: no alignment exists
                         r->alignment = NULL; r->alignmentLength = 0;

@@ -178,7 +178,7 @@ struct CreateGate {
 static int search_into_results(DeviceDb* ddb, const unsigned char* query, int queryLength, unsigned char* const* db, int dbLength,
                                const int* dbSeqLengths, int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength,
                                OpalSearchResult* results[], const int searchType, int mode, int device,
-                               CreateGate* gate = nullptr, int ticket = 0) {
+                               CreateGate* gate = nullptr, int ticket = 0, const int* pssm = nullptr) {
     if (mode != OPAL_MODE_NW && mode != OPAL_MODE_HW && mode != OPAL_MODE_OV && mode != OPAL_MODE_SW)
         return OPAL_ERR_INVALID_MODE;  // :1469-1473, results untouched
     if (dbLength <= 0) return 0;
@@ -214,11 +214,11 @@ static int search_into_results(DeviceDb* ddb, const unsigned char* query, int qu
     int status = 0;
     if (anyWork)  // results go straight into the records (same pass also sets the no-alignment fields, :1508-1515)
         status = ddb->search(query, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd, mode, skip.data(), nullptr,
-                             nullptr, nullptr, nullptr, results, searchType != OPAL_SEARCH_ALIGNMENT);
+                             nullptr, nullptr, nullptr, results, searchType != OPAL_SEARCH_ALIGNMENT, pssm);
     const auto t2 = now();
     if (status == 0 && searchType == OPAL_SEARCH_ALIGNMENT)
         status = align_database(ddb, query, queryLength, db, dbLength, dbSeqLengths, gapOpen, gapExt, scoreMatrix, alphabetLength,
-                                results, mode);
+                                results, mode, nullptr, pssm);
     const auto t3 = now();
     delete owned;
     if (trace)
@@ -328,6 +328,21 @@ int opalSearchDatabaseCharSW(unsigned char query[], int queryLength, unsigned ch
 }
 
 // ------------------------------------------------------------------ opal_b200.h
+// PSSM entry points: the rows of a search of queryLength 0 (pssm may then be NULL; nothing is read through it).
+static const int kNoPssmRows = 0;
+
+// Arguments only the PSSM entry points have: the PSSM itself, and -- for OPAL_SEARCH_ALIGNMENT -- the residues it was
+// built for, which label the diagonal steps of an alignment MATCH / MISMATCH.  0 or OPAL_ERR_INVALID_ARGUMENT.
+static int check_pssm_args(const int* pssm, const unsigned char* query, int queryLength, int alphabetLength, int searchType) {
+    if (!pssm && queryLength > 0) { set_error("pssm is NULL"); return OPAL_ERR_INVALID_ARGUMENT; }
+    if (searchType == OPAL_SEARCH_ALIGNMENT && queryLength > 0) {
+        if (!query) { set_error("OPAL_SEARCH_ALIGNMENT with a PSSM needs the query residues"); return OPAL_ERR_INVALID_ARGUMENT; }
+        for (int r = 0; r < queryLength; r++)
+            if (query[r] >= alphabetLength) { set_error("query holds residue codes >= alphabetLength"); return OPAL_ERR_INVALID_ARGUMENT; }
+    }
+    return 0;
+}
+
 int opalb200_device_count(void) {
     int n = 0;
     return cudaGetDeviceCount(&n) == cudaSuccess ? n : 0;
@@ -398,16 +413,17 @@ long long opalb200_db_residues(const OpalB200Db* h) { return reinterpret_cast<co
 
 int opalb200_db_devices(const OpalB200Db* h) { return reinterpret_cast<const DbHandle*>(h)->parts(); }
 
-int opalb200_db_search(OpalB200Db* hh, const unsigned char query[], int queryLength, int gapOpen, int gapExt,
-                       const int* scoreMatrix, int alphabetLength, int searchType, int mode, const unsigned char* skip,
-                       int* scores, int* endQuery, int* endTarget, float* deviceMs) {
+// opalb200_db_search and opalb200_db_search_pssm (pssm non-NULL: query and scoreMatrix unused)
+static int db_search(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int gapOpen, int gapExt,
+                     const int* scoreMatrix, int alphabetLength, int searchType, int mode, const unsigned char* skip,
+                     int* scores, int* endQuery, int* endTarget, float* deviceMs) {
     if (!hh || !scores) return OPAL_ERR_NO_SIMD_SUPPORT;
     DeviceGuard guard;
     DbHandle* h = reinterpret_cast<DbHandle*>(hh);
     const int wantEnd = searchType != OPAL_SEARCH_SCORE && endQuery && endTarget;
     if (h->index.empty()) {
         const int rc = h->shards[0]->search(query, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd, mode, skip, scores,
-                                            endQuery, endTarget, deviceMs);
+                                            endQuery, endTarget, deviceMs, nullptr, false, pssm);
         h->collect_stats();
         return rc;
     }
@@ -419,7 +435,7 @@ int opalb200_db_search(OpalB200Db* hh, const unsigned char query[], int queryLen
         std::vector<unsigned char> sk;
         if (skip) { sk.resize(m); for (size_t k = 0; k < m; k++) sk[k] = skip[idx[k]]; }
         const int r = h->shards[s]->search(query, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd, mode,
-                                           skip ? sk.data() : nullptr, sc.data(), eq.data(), et.data(), &ms[s]);
+                                           skip ? sk.data() : nullptr, sc.data(), eq.data(), et.data(), &ms[s], nullptr, false, pssm);
         if (r) return r;
         for (size_t k = 0; k < m; k++) {
             if (skip && sk[k]) continue;
@@ -434,9 +450,26 @@ int opalb200_db_search(OpalB200Db* hh, const unsigned char query[], int queryLen
     return rc;
 }
 
+int opalb200_db_search(OpalB200Db* hh, const unsigned char query[], int queryLength, int gapOpen, int gapExt,
+                       const int* scoreMatrix, int alphabetLength, int searchType, int mode, const unsigned char* skip,
+                       int* scores, int* endQuery, int* endTarget, float* deviceMs) {
+    return db_search(hh, query, nullptr, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, searchType, mode, skip, scores,
+                     endQuery, endTarget, deviceMs);
+}
+
+int opalb200_db_search_pssm(OpalB200Db* hh, const int* pssm, int queryLength, int alphabetLength, int gapOpen, int gapExt,
+                            int searchType, int mode, const unsigned char* skip, int* scores, int* endQuery, int* endTarget,
+                            float* deviceMs) {
+    if (deviceMs) *deviceMs = 0.f;
+    if (const int rc = check_pssm_args(pssm, nullptr, queryLength, alphabetLength, OPAL_SEARCH_SCORE)) return rc;
+    return db_search(hh, nullptr, pssm ? pssm : &kNoPssmRows, queryLength, gapOpen, gapExt, nullptr, alphabetLength, searchType, mode,
+                     skip, scores, endQuery, endTarget, deviceMs);
+}
+
 static int search_batch_modes(OpalB200Db* hh, int numQueries, const unsigned char* const queries[], const int queryLengths[],
                               int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength, int searchType, int mode,
-                              const int* modes, int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs);
+                              const int* modes, int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs,
+                              const int* const* pssms = nullptr);
 
 int opalb200_db_search_batch(OpalB200Db* hh, int numQueries, const unsigned char* const queries[], const int queryLengths[],
                              int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength, int searchType, int mode,
@@ -456,17 +489,36 @@ int opalb200_db_search_batch_modes(OpalB200Db* hh, int numSearches, const unsign
                               OPAL_MODE_SW, modes, scores, endQuery, endTarget, inFlight, batchMs);
 }
 
+int opalb200_db_search_batch_pssm(OpalB200Db* hh, int numSearches, const int* const pssms[], const int queryLengths[], const int modes[],
+                                  int alphabetLength, int gapOpen, int gapExt, int searchType, int* scores, int* endQuery,
+                                  int* endTarget, int inFlight, float* batchMs) {
+    if (batchMs) *batchMs = 0.f;
+    if (numSearches > 0 && !modes) return OPAL_ERR_INVALID_MODE;
+    if (numSearches > 0 && (!pssms || !queryLengths)) { set_error("pssms / queryLengths is NULL"); return OPAL_ERR_INVALID_ARGUMENT; }
+    for (int q = 0; q < numSearches; q++)
+        if (modes[q] != OPAL_MODE_NW && modes[q] != OPAL_MODE_HW && modes[q] != OPAL_MODE_OV && modes[q] != OPAL_MODE_SW)
+            return OPAL_ERR_INVALID_MODE;
+    std::vector<const int*> rows((size_t)std::max(numSearches, 0));
+    for (int q = 0; q < numSearches; q++) {
+        if (const int rc = check_pssm_args(pssms[q], nullptr, queryLengths[q], alphabetLength, OPAL_SEARCH_SCORE)) return rc;
+        rows[q] = pssms[q] ? pssms[q] : &kNoPssmRows;
+    }
+    return search_batch_modes(hh, numSearches, nullptr, queryLengths, gapOpen, gapExt, nullptr, alphabetLength, searchType,
+                              OPAL_MODE_SW, modes, scores, endQuery, endTarget, inFlight, batchMs, rows.data());
+}
+
 static int search_batch_modes(OpalB200Db* hh, int numQueries, const unsigned char* const queries[], const int queryLengths[],
                               int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength, int searchType, int mode,
-                              const int* modes, int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs) {
-    if (!hh || !scores || (numQueries > 0 && (!queries || !queryLengths))) return OPAL_ERR_NO_SIMD_SUPPORT;
+                              const int* modes, int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs,
+                              const int* const* pssms) {
+    if (!hh || !scores || (numQueries > 0 && ((!queries && !pssms) || !queryLengths))) return OPAL_ERR_NO_SIMD_SUPPORT;
     DeviceGuard guard;
     DbHandle* h = reinterpret_cast<DbHandle*>(hh);
     const int wantEnd = searchType != OPAL_SEARCH_SCORE && endQuery && endTarget;
     const int fl = inFlight <= 0 ? 3 : inFlight;
     if (h->index.empty()) {
         const int rc = h->shards[0]->search_batch(numQueries, queries, queryLengths, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd,
-                                                  mode, scores, endQuery, endTarget, fl, batchMs, modes);
+                                                  mode, scores, endQuery, endTarget, fl, batchMs, modes, pssms);
         h->collect_stats();
         return rc;
     }
@@ -477,7 +529,8 @@ static int search_batch_modes(OpalB200Db* hh, int numQueries, const unsigned cha
         const size_t m = idx.size(), all = m * (size_t)std::max(numQueries, 0);
         std::vector<int> sc(all), eq(wantEnd ? all : 0), et(wantEnd ? all : 0);
         const int r = h->shards[s]->search_batch(numQueries, queries, queryLengths, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd,
-                                                 mode, sc.data(), wantEnd ? eq.data() : nullptr, wantEnd ? et.data() : nullptr, fl, &ms[s], modes);
+                                                 mode, sc.data(), wantEnd ? eq.data() : nullptr, wantEnd ? et.data() : nullptr, fl, &ms[s], modes,
+                                                 pssms);
         if (r) return r;
         for (int q = 0; q < numQueries; q++)
             for (size_t k = 0; k < m; k++) {
@@ -493,27 +546,41 @@ static int search_batch_modes(OpalB200Db* hh, int numQueries, const unsigned cha
     return rc;
 }
 
-int opalb200_db_search_results(OpalB200Db* hh, const unsigned char query[], int queryLength, int gapOpen, int gapExt,
-                               const int* scoreMatrix, int alphabetLength, OpalSearchResult* results[], int searchType, int mode) {
+// opalb200_db_search_results and opalb200_db_search_results_pssm (pssm non-NULL: scoreMatrix unused)
+static int db_search_results(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int gapOpen, int gapExt,
+                             const int* scoreMatrix, int alphabetLength, OpalSearchResult* results[], int searchType, int mode) {
     if (!hh || !results) return OPAL_ERR_NO_SIMD_SUPPORT;
     DeviceGuard guard;
     DbHandle* h = reinterpret_cast<DbHandle*>(hh);
     if (h->index.empty())
         return search_into_results(h->shards[0], query, queryLength, nullptr, h->n, nullptr, gapOpen, gapExt, scoreMatrix, alphabetLength,
-                                   results, searchType, mode, h->shards[0]->device());
+                                   results, searchType, mode, h->shards[0]->device(), nullptr, 0, pssm);
     if (mode != OPAL_MODE_NW && mode != OPAL_MODE_HW && mode != OPAL_MODE_OV && mode != OPAL_MODE_SW) return OPAL_ERR_INVALID_MODE;
     return on_shards(h->parts(), [&](int s) -> int {
         const std::vector<int>& idx = h->index[s];
         std::vector<OpalSearchResult*> res(idx.size());
         for (size_t k = 0; k < idx.size(); k++) res[k] = results[idx[k]];
         return search_into_results(h->shards[s], query, queryLength, nullptr, (int)idx.size(), nullptr, gapOpen, gapExt, scoreMatrix,
-                                   alphabetLength, res.data(), searchType, mode, h->shards[s]->device());
+                                   alphabetLength, res.data(), searchType, mode, h->shards[s]->device(), nullptr, 0, pssm);
     });
 }
 
-int opalb200_db_search_topk(OpalB200Db* hh, const unsigned char query[], int queryLength, int gapOpen, int gapExt,
-                            const int* scoreMatrix, int alphabetLength, int searchType, int mode, int k, int* indices,
-                            OpalSearchResult* results[], int* found) {
+int opalb200_db_search_results(OpalB200Db* hh, const unsigned char query[], int queryLength, int gapOpen, int gapExt,
+                               const int* scoreMatrix, int alphabetLength, OpalSearchResult* results[], int searchType, int mode) {
+    return db_search_results(hh, query, nullptr, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, results, searchType, mode);
+}
+
+int opalb200_db_search_results_pssm(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int alphabetLength,
+                                    int gapOpen, int gapExt, OpalSearchResult* results[], int searchType, int mode) {
+    if (const int rc = check_pssm_args(pssm, query, queryLength, alphabetLength, searchType)) return rc;
+    return db_search_results(hh, searchType == OPAL_SEARCH_ALIGNMENT ? query : nullptr, pssm ? pssm : &kNoPssmRows, queryLength, gapOpen,
+                             gapExt, nullptr, alphabetLength, results, searchType, mode);
+}
+
+// opalb200_db_search_topk and opalb200_db_search_topk_pssm (pssm non-NULL: scoreMatrix unused)
+static int db_search_topk(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int gapOpen, int gapExt,
+                          const int* scoreMatrix, int alphabetLength, int searchType, int mode, int k, int* indices,
+                          OpalSearchResult* results[], int* found) {
     if (found) *found = 0;
     if (!hh || !indices || !results || k < 0) return OPAL_ERR_NO_SIMD_SUPPORT;
     DeviceGuard guard;
@@ -529,7 +596,7 @@ int opalb200_db_search_topk(OpalB200Db* hh, const unsigned char query[], int que
         std::vector<int> li((size_t)ks), sc((size_t)ks), eq((size_t)ks), et((size_t)ks);
         const int* map = h->index.empty() ? nullptr : h->index[s].data();
         const int r = h->shards[s]->search_topk(query, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd, mode, ks, map,
-                                                li.data(), sc.data(), eq.data(), et.data());
+                                                li.data(), sc.data(), eq.data(), et.data(), pssm);
         if (r) return r;
         for (int j = 0; j < ks; j++) perShard[s].push_back({sc[j], h->caller_index(s, li[j]), eq[j], et[j], s, li[j]});
         return 0;
@@ -558,9 +625,25 @@ int opalb200_db_search_topk(OpalB200Db* hh, const unsigned char query[], int que
                 if (hits[j].shard == s) { subset.push_back(hits[j].local); res.push_back(results[j]); }
             if (subset.empty()) return 0;
             return align_database(h->shards[s], query, queryLength, nullptr, (int)subset.size(), nullptr, gapOpen, gapExt, scoreMatrix,
-                                  alphabetLength, res.data(), mode, subset.data());
+                                  alphabetLength, res.data(), mode, subset.data(), pssm);
         });
     return status;
+}
+
+int opalb200_db_search_topk(OpalB200Db* hh, const unsigned char query[], int queryLength, int gapOpen, int gapExt,
+                            const int* scoreMatrix, int alphabetLength, int searchType, int mode, int k, int* indices,
+                            OpalSearchResult* results[], int* found) {
+    return db_search_topk(hh, query, nullptr, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, searchType, mode, k, indices,
+                          results, found);
+}
+
+int opalb200_db_search_topk_pssm(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int alphabetLength,
+                                 int gapOpen, int gapExt, int searchType, int mode, int k, int* indices, OpalSearchResult* results[],
+                                 int* found) {
+    if (found) *found = 0;
+    if (const int rc = check_pssm_args(pssm, query, queryLength, alphabetLength, searchType)) return rc;
+    return db_search_topk(hh, searchType == OPAL_SEARCH_ALIGNMENT ? query : nullptr, pssm ? pssm : &kNoPssmRows, queryLength, gapOpen,
+                          gapExt, nullptr, alphabetLength, searchType, mode, k, indices, results, found);
 }
 
 void opalb200_db_last_stats(const OpalB200Db* h, int* kernelLaunches, int* rerun32, int* G, int* R, int* passes,

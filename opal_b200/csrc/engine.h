@@ -104,9 +104,11 @@ public:
     // Several queries against the resident database, up to `inFlight` of them on the device at a time (each on a
     // search context of its own: streams, result and scratch buffers), so that the tail of one query overlaps the
     // bulk of the next and host-side planning / publishing overlaps kernels.  Outputs are [query][caller index].
+    // pssms: one position-specific scoring matrix per query (see search()); queries / matrix are then unused.
     int search_batch(int numQueries, const unsigned char* const* queries, const int* queryLengths, int Go, int Ge,
                      const int* matrix, int A, int wantEnd, int mode, int* scores, int* endQ, int* endT, int inFlight,
-                     float* batchMs, const int* modes = nullptr);  // modes: one per query (NULL: `mode` for all)
+                     float* batchMs, const int* modes = nullptr,  // modes: one per query (NULL: `mode` for all)
+                     const int* const* pssms = nullptr);
     // Blocks until the upload issued by create() has finished (create() returns with it in flight).
     bool ensure_uploaded();
 
@@ -114,14 +116,16 @@ public:
     // With `records` the results go straight into the caller's OpalSearchResult records instead of the three arrays
     // (one pass over half a million 40-byte records instead of two); noAlignmentFill also gives every computed record
     // the fields opalSearchDatabase sets below OPAL_SEARCH_ALIGNMENT (reference src/opal.cpp:1508-1515).
+    // With `pssm` (Q x A ints, row r = scores of query position r against every letter) the query is scored by it
+    // instead of by matrix rows of query letters; query and matrix are then unused (either may be NULL).
     int search(const unsigned char* query, int Q, int Go, int Ge, const int* matrix, int A, int wantEnd, int mode,
                const unsigned char* skip, int* scores, int* endQ, int* endT, float* deviceMs,
-               OpalSearchResult* const* records = nullptr, bool noAlignmentFill = false);
+               OpalSearchResult* const* records = nullptr, bool noAlignmentFill = false, const int* pssm = nullptr);
 
     // Score [+ end] search followed by the selection of the k best targets: score descending, then smallest
     // map[caller index] (map NULL: the caller index itself).  Writes k (<= size()) caller indices and their records.
     int search_topk(const unsigned char* query, int Q, int Go, int Ge, const int* matrix, int A, int wantEnd, int mode, int k,
-                    const int* map, int* outIndex, int* outScore, int* outEndQ, int* outEndT);
+                    const int* map, int* outIndex, int* outScore, int* outEndQ, int* outEndT, const int* pssm = nullptr);
 
     int size() const { return n_; }
     long long residues() const { return totalResidues_; }
@@ -171,7 +175,8 @@ private:
     int *dMaxCode_ = nullptr, *hMaxCode_ = nullptr;
     unsigned char *hBlock_ = nullptr, *dBlock_ = nullptr;  // offsets | pair offsets | lengths | max code | residues (pinned / device)
     int numPairs_ = 0, maxCode_ = 0;
-    unsigned char *dArgs_ = nullptr, *hArgs_ = nullptr;  // launch counters | score matrix | query (device / pinned)
+    unsigned char *dArgs_ = nullptr, *hArgs_ = nullptr;  // launch counters | score matrix | query, or counters | PSSM (device / pinned)
+    const int* dPssm_ = nullptr;  // the PSSM of the search in progress in dArgs_ (NULL: matrix search)
     size_t argsCapacity_ = 0;
     int *hScore_ = nullptr, *hEndQ_ = nullptr, *hEndT_ = nullptr;  // views into hResults_
     cudaStream_t stream_ = nullptr;

@@ -62,7 +62,7 @@ constexpr int kScoreOverflow = INT32_MIN + 1;  // 16-bit pass: re-run this targe
 struct SearchParams {
     // query side
     const uint8_t* query;  // Q alphabet indices
-    const int* matrix;     // A*A, row = query letter
+    const int* matrix;     // score rows read by the profile build: A*A, row = query letter (PSSM search: the PSSM, row = query row)
     int Q, A, gapOpen, gapExt, mode, wantEnd;
     // geometry of this pass
     int G, rowBase, padTop, pass, numPasses, rowStride, Rpad;
@@ -122,6 +122,10 @@ struct SearchParams {
     const int* chainOffsets;
     int* chainDone;       // [task * numPasses + pass]: that pass has written its results
     int* chainTicket;     // blocks take their place in the chain in the order they START (so a producer is never behind its consumer)
+    // Position-specific scoring matrix, Q x A row-major (row r = scores of query position r against every target letter),
+    // or NULL.  When set, `matrix` points at it as well and the profile build takes row r for query row r instead of the
+    // row of query letter query[r]; `query` is unused.  (Last member: the sweep's parameter offsets stay where they were.)
+    const int* pssm;
 };
 // Chained passes: "not written yet" in a boundary row.  Both half-words -32768 (or INT_MIN at 32 bits) lies outside
 // every range the kernels guarantee; a sweep that has already left that range (its target is flagged and re-run at 32
@@ -339,17 +343,20 @@ __global__ void __launch_bounds__(MAXT, 1) search_kernel(const SearchParams p) {
     // A + 1 target letters of that column, reading one row of the score matrix (a few cache lines).  (The earlier form,
     // one thread per profile WORD, paid the query load and its dependent matrix load for every word: ~40 us per launch
     // at 32 x 33 rows, which is 6 % of a BASELINE configs[1] search and 1 - 2 % of every pass on a database shard.)
+    // With a PSSM the column reads its own row of it.  (Written so that the sweep compiles to the same SASS as without
+    // PSSM support: a select of the row base here changed the register allocation of the R = 32 step.)
+    const bool byRow = p.pssm != nullptr;
     for (int pos = threadIdx.x; pos < p.rowStride; pos += blockDim.x) {
         const int t = pos / p.Rpad, j = pos - t * p.Rpad;
-        int q = -1, q2 = -1;  // query letters of the low / high half-word rows; -1 = padding row
+        int q = -1, q2 = -1;  // rows of `matrix` (query letters, or query rows) of the low / high half-word rows; -1 = padding
         const bool used = t < G && j < R;
         if (used) {
             const int r = rowBase + t * R + j - p.padTop;
-            if (r >= 0 && r < p.Q) q = p.query[r];
+            if (r >= 0 && r < p.Q) q = byRow ? r : p.query[r];
             q2 = q;
             if (LANES == 2 && p.folded) {  // high half-words: the rows 32 R further down
                 const int r2 = r + 32 * R;
-                q2 = (r2 >= 0 && r2 < p.Q) ? (int)p.query[r2] : -1;
+                q2 = (r2 >= 0 && r2 < p.Q) ? (byRow ? r2 : (int)p.query[r2]) : -1;
             }
         }
         // padding rows score 0 against everything (keeps H = 0 above the query); letter 0 is "no residue"

@@ -50,6 +50,14 @@ class OpalB200(OpalCLibrary):
         L.opalb200_db_residues.restype = ctypes.c_longlong
         L.opalb200_db_search.argtypes = [vp, vp, ci, ci, ci, vp, ci, ci, ci, vp, vp, vp, vp, vp]
         L.opalb200_db_search.restype = ci
+        L.opalb200_db_search_pssm.argtypes = [vp, vp, ci, ci, ci, ci, ci, ci, vp, vp, vp, vp, vp]
+        L.opalb200_db_search_pssm.restype = ci
+        L.opalb200_db_search_batch_pssm.argtypes = [vp, ci, vp, vp, vp, ci, ci, ci, ci, vp, vp, vp, ci, vp]
+        L.opalb200_db_search_batch_pssm.restype = ci
+        L.opalb200_db_search_results_pssm.argtypes = [vp, vp, vp, ci, ci, ci, ci, vp, ci, ci]
+        L.opalb200_db_search_results_pssm.restype = ci
+        L.opalb200_db_search_topk_pssm.argtypes = [vp, vp, vp, ci, ci, ci, ci, ci, ci, ci, vp, vp, ctypes.POINTER(ci)]
+        L.opalb200_db_search_topk_pssm.restype = ci
         L.opalb200_db_last_stats.argtypes = [vp] + [ctypes.POINTER(ci)] * 7
         L.opalb200_db_last_stats.restype = None
         L.opalb200_db_last_folded.argtypes = [vp]
@@ -189,6 +197,97 @@ class ResidentDb:
         rc = self.eng.lib.opalb200_db_search_topk(
             self.handle, qbuf.ctypes.data, int(query.size), int(gap_open), int(gap_ext), sm.ctypes.data,
             int(alphabet_length), int(search_type), int(mode), int(k), idx.ctypes.data, rp.ctypes.data, ctypes.byref(found))
+        return rc, idx[:found.value], results[:found.value]
+
+    # ---- position-specific scoring matrices: `pssm` is an int32 array of shape (Q, A); pssm[r, y] scores query position
+    # r against residue code y, and the alphabet length is pssm.shape[1].  pssm=None with `query_length` searches an empty
+    # query (or passes NULL, to see the call reject it for query_length > 0).
+    @staticmethod
+    def _pssm(pssm, query_length=None, alphabet_length=None):
+        """(C pointer or None, the array kept alive, Q, A)"""
+        if pssm is None:
+            return None, None, int(query_length or 0), int(alphabet_length or 1)
+        arr = np.ascontiguousarray(pssm, dtype=np.int32)
+        if arr.ndim != 2:
+            raise ValueError("pssm must have shape (queryLength, alphabetLength)")
+        buf = arr if arr.size else np.zeros(1, dtype=np.int32)
+        return buf.ctypes.data, buf, int(arr.shape[0]), int(arr.shape[1])
+
+    def search_pssm(self, pssm, gap_open, gap_ext, search_type, mode, skip=None, query_length=None, alphabet_length=None):
+        """opalb200_db_search_pssm. Returns (rc, scores, endQuery, endTarget, device_ms) like search()."""
+        ptr, keep, Q, A = self._pssm(pssm, query_length, alphabet_length)
+        sc = np.zeros(self.n, dtype=np.int32)
+        eq = np.full(self.n, -1, dtype=np.int32)
+        et = np.full(self.n, -1, dtype=np.int32)
+        ms = ctypes.c_float(0)
+        if isinstance(mode, str):
+            mode = MODES[mode]
+        skp = None if skip is None else np.ascontiguousarray(skip, dtype=np.uint8)
+        rc = self.eng.lib.opalb200_db_search_pssm(
+            self.handle, ptr, Q, A, int(gap_open), int(gap_ext), int(search_type), int(mode),
+            None if skp is None else skp.ctypes.data, sc.ctypes.data, eq.ctypes.data, et.ctypes.data, ctypes.byref(ms))
+        del keep
+        return rc, sc, eq, et, float(ms.value)
+
+    def search_batch_pssm(self, pssms, gap_open, gap_ext, search_type, modes, in_flight=3):
+        """opalb200_db_search_batch_pssm: one PSSM and one mode per search (all PSSMs have the same alphabet length).
+        Returns (rc, scores[ns, n], endQuery, endTarget, batch_ms)."""
+        arrs = [np.ascontiguousarray(x, dtype=np.int32) for x in pssms]
+        ns = len(arrs)
+        A = int(arrs[0].shape[1]) if ns else 1
+        if any(a.ndim != 2 or a.shape[1] != A for a in arrs):
+            raise ValueError("every pssm must have shape (queryLength, alphabetLength) with the same alphabetLength")
+        bufs = [a if a.size else np.zeros(1, dtype=np.int32) for a in arrs]
+        ptrs = np.array([b.ctypes.data for b in bufs], dtype=np.uint64)
+        qlens = np.array([a.shape[0] for a in arrs], dtype=np.int32)
+        if isinstance(modes, (str, int)):
+            modes = [modes] * ns
+        md = np.array([MODES[m] if isinstance(m, str) else int(m) for m in modes], dtype=np.int32)
+        assert len(md) == ns
+        sc = np.zeros((ns, self.n), dtype=np.int32)
+        eq = np.full((ns, self.n), -1, dtype=np.int32)
+        et = np.full((ns, self.n), -1, dtype=np.int32)
+        ms = ctypes.c_float(0)
+        rc = self.eng.lib.opalb200_db_search_batch_pssm(
+            self.handle, ns, ptrs.ctypes.data, qlens.ctypes.data, md.ctypes.data, A, int(gap_open), int(gap_ext),
+            int(search_type), sc.ctypes.data, eq.ctypes.data, et.ctypes.data, int(in_flight), ctypes.byref(ms))
+        return rc, sc, eq, et, float(ms.value)
+
+    def search_results_pssm(self, pssm, gap_open, gap_ext, search_type, mode, query=None, results=None, query_length=None,
+                            alphabet_length=None):
+        """opalb200_db_search_results_pssm; `query` (the residues the PSSM was built for) labels alignment steps
+        MATCH / MISMATCH and is required for OPAL_SEARCH_ALIGNMENT. Returns (rc, results)."""
+        ptr, keep, Q, A = self._pssm(pssm, query_length, alphabet_length)
+        qbuf = None if query is None else np.ascontiguousarray(query, dtype=np.uint8)
+        if qbuf is not None and not qbuf.size:
+            qbuf = np.zeros(1, dtype=np.uint8)
+        if results is None:
+            results = new_results(self.n)
+        rp = result_pointers(results)
+        if isinstance(mode, str):
+            mode = MODES[mode]
+        rc = self.eng.lib.opalb200_db_search_results_pssm(
+            self.handle, None if qbuf is None else qbuf.ctypes.data, ptr, Q, A, int(gap_open), int(gap_ext), rp.ctypes.data,
+            int(search_type), int(mode))
+        del keep
+        return rc, results
+
+    def search_topk_pssm(self, pssm, gap_open, gap_ext, search_type, mode, k, query=None):
+        """opalb200_db_search_topk_pssm. Returns (rc, indices[found], results[found])."""
+        ptr, keep, Q, A = self._pssm(pssm)
+        qbuf = None if query is None else np.ascontiguousarray(query, dtype=np.uint8)
+        if qbuf is not None and not qbuf.size:
+            qbuf = np.zeros(1, dtype=np.uint8)
+        results = new_results(max(int(k), 1))
+        rp = result_pointers(results)
+        idx = np.full(max(int(k), 1), -1, dtype=np.int32)
+        found = ctypes.c_int(0)
+        if isinstance(mode, str):
+            mode = MODES[mode]
+        rc = self.eng.lib.opalb200_db_search_topk_pssm(
+            self.handle, None if qbuf is None else qbuf.ctypes.data, ptr, Q, A, int(gap_open), int(gap_ext), int(search_type),
+            int(mode), int(k), idx.ctypes.data, rp.ctypes.data, ctypes.byref(found))
+        del keep
         return rc, idx[:found.value], results[:found.value]
 
     def devices(self):
