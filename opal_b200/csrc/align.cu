@@ -270,21 +270,19 @@ bool band_borders(int k, int mode, int Q, int T, int Go, int Ge, int M, int* bot
 }
 
 // Replay of an operation string (the check of reference src/test.cpp:348-422): does it start at
-// (sq, st), end at (endQ, endT) and score exactly `score`?
-// With a PSSM, query position qi scores by its row of the PSSM; q only labels the diagonal steps.
-bool replay_ok(const unsigned char* q, int Q, const unsigned char* t, int T, const unsigned char* ops, int n, int sq, int st,
-               int endQ, int endT, int score, int Go, int Ge, const int* S, int A, const int* pssm) {
+// (sq, st), end at (endQ, endT) and score exactly `score` under s?
+bool replay_ok(const Scoring& s, const unsigned char* t, int T, const unsigned char* ops, int n, int sq, int st, int endQ, int endT,
+               int score) {
     i64 sc = 0;
     int qi = sq, ti = st, prev = -1;
     if (qi < 0 || ti < 0) return false;
-    auto cell = [&](int r, int y) -> i64 { return pssm ? pssm[(size_t)r * A + y] : S[q[r] * A + y]; };
     for (int i = 0; i < n; i++) {
         const int op = ops[i];
-        if ((op != OPAL_ALIGN_DEL && ti >= T) || (op != OPAL_ALIGN_INS && qi >= Q)) return false;
-        if (op == OPAL_ALIGN_MATCH) { if (q[qi] != t[ti]) return false; sc += cell(qi, t[ti]); qi++; ti++; }
-        else if (op == OPAL_ALIGN_MISMATCH) { if (q[qi] == t[ti]) return false; sc += cell(qi, t[ti]); qi++; ti++; }
-        else if (op == OPAL_ALIGN_DEL) { sc -= (prev == OPAL_ALIGN_DEL ? Ge : Go); qi++; }
-        else if (op == OPAL_ALIGN_INS) { sc -= (prev == OPAL_ALIGN_INS ? Ge : Go); ti++; }
+        if ((op != OPAL_ALIGN_DEL && ti >= T) || (op != OPAL_ALIGN_INS && qi >= s.Q)) return false;
+        if (op == OPAL_ALIGN_MATCH) { if (s.query[qi] != t[ti]) return false; sc += s.cell(qi, t[ti]); qi++; ti++; }
+        else if (op == OPAL_ALIGN_MISMATCH) { if (s.query[qi] == t[ti]) return false; sc += s.cell(qi, t[ti]); qi++; ti++; }
+        else if (op == OPAL_ALIGN_DEL) { sc -= (prev == OPAL_ALIGN_DEL ? s.Ge : s.Go); qi++; }
+        else if (op == OPAL_ALIGN_INS) { sc -= (prev == OPAL_ALIGN_INS ? s.Ge : s.Go); ti++; }
         else return false;
         prev = op;
     }
@@ -304,9 +302,9 @@ bool replay_ok(const unsigned char* q, int Q, const unsigned char* t, int T, con
 
 }  // namespace
 
-int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned char* const* db, int n, const int* lens,
-                   int Go, int Ge, const int* matrix, int A, OpalSearchResult* results[], int mode, const int* subset,
-                   const int* pssm) {
+int align_database(DeviceDb* ddb, const Scoring& s, unsigned char* const* db, int n, const int* lens, OpalSearchResult* results[],
+                   const int* subset) {
+    const int Q = s.Q, A = s.A, Go = s.Go, Ge = s.Ge, mode = s.mode;
     if (!ddb || !ddb->ensure_uploaded()) return OPAL_B200_ERR_CUDA;
     // target i on the host: the caller's pointer, or (resident-handle calls) the database's own sorted copy
     // record j describes database entry entry(j): all of them, or the given subset (top-k pipelines)
@@ -315,11 +313,7 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
     auto target_ptr = [&](int j) -> const unsigned char* {
         return db ? db[entry(j)] : ddb->h_residues() + ddb->offsets()[ddb->sorted_position()[entry(j)]];
     };
-    // the band's M: the largest entry that can score a cell (matrix, or PSSM)
-    const int* scoreEntries = pssm ? pssm : matrix;
-    const long long numEntries = pssm ? (long long)Q * A : (long long)A * A;
-    int M = numEntries > 0 ? scoreEntries[0] : 0;
-    for (long long i = 1; i < numEntries; i++) M = std::max(M, scoreEntries[i]);
+    const int M = s.bounds().maxEntry;  // the band's M: the largest entry that can score a cell
 
     // ---- entries that have an alignment at all (src/opal.cpp:1479-1483)
     std::vector<int> todo;
@@ -350,7 +344,7 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
     std::vector<unsigned char> hOps;
     std::vector<AlignOut> hOuts;
     // matrix, or a pass's 32 x kRows PSSM rows, in shared memory when it fits
-    const size_t smemBytes = sizeof(int) * (size_t)A * (pssm ? 32 * kRows : A);
+    const size_t smemBytes = sizeof(int) * (size_t)A * (s.byPssm ? 32 * kRows : A);
     const int matrixInSmem = smemBytes <= 40000 ? 1 : 0;
     size_t freeB = 0, totalB = 0;
     cudaMemGetInfo(&freeB, &totalB);
@@ -364,9 +358,9 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
         dTasks = nullptr; dOuts = nullptr; dFlags = nullptr; dEq = nullptr; dOps = nullptr; dBnd = nullptr;
     };
     ALIGN_OK(dalloc(&dQuery, (size_t)Q + 16));
-    ALIGN_OK(dalloc(&dMatrix, sizeof(int) * (size_t)numEntries));
-    ALIGN_TRY(cudaMemcpyAsync(dQuery, query, Q, cudaMemcpyHostToDevice, stream));
-    ALIGN_TRY(cudaMemcpyAsync(dMatrix, scoreEntries, sizeof(int) * (size_t)numEntries, cudaMemcpyHostToDevice, stream));
+    ALIGN_OK(dalloc(&dMatrix, sizeof(int) * (size_t)s.num_entries()));
+    ALIGN_TRY(cudaMemcpyAsync(dQuery, s.query, Q, cudaMemcpyHostToDevice, stream));
+    ALIGN_TRY(cudaMemcpyAsync(dMatrix, s.entries, sizeof(int) * (size_t)s.num_entries(), cudaMemcpyHostToDevice, stream));
 
     {
         // Two rounds at most: the reference's band first, the full band for entries whose replay fails.
@@ -408,7 +402,7 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
                 // an alignment is shorter than its slot: the unused tail travels back with the rest, so it is defined
                 ALIGN_TRY(cudaMemsetAsync(dOps, 0, (size_t)opsBytes, stream));
                 align_dp_kernel<<<nt, 32, matrixInSmem ? smemBytes : 0, stream>>>(dTasks, dOuts, ddb->d_residues(), dQuery,
-                                                                                   pssm ? nullptr : dMatrix, pssm ? dMatrix : nullptr, A,
+                                                                                   s.byPssm ? nullptr : dMatrix, s.byPssm ? dMatrix : nullptr, A,
                                                                                    Go, Ge, mode, dFlags, dEq, dBnd, matrixInSmem);
                 ALIGN_TRY(cudaGetLastError());
                 align_traceback_kernel<<<(nt + 63) / 64, 64, 0, stream>>>(dTasks, dOuts, nt, ddb->d_residues(), dQuery, mode, dFlags, dEq,
@@ -426,8 +420,7 @@ int align_database(DeviceDb* ddb, const unsigned char* query, int Q, unsigned ch
                     const AlignTask& tk = tasks[k];
                     const unsigned char* ops = hOps.data() + tk.opsOffset;
                     const int sq = tk.endQ - o.endRow, st = tk.endT - o.stopCol;  // src/opal.cpp:1499-1500
-                    const bool good = o.status == 0 && replay_ok(query, Q, target_ptr(i), target_len(i), ops, o.opsLen, sq, st, tk.endQ, tk.endT,
-                                                                 tk.score, Go, Ge, matrix, A, pssm);
+                    const bool good = o.status == 0 && replay_ok(s, target_ptr(i), target_len(i), ops, o.opsLen, sq, st, tk.endQ, tk.endT, tk.score);
                     if (!good && round == 0 && (tk.bottom != tk.Qp - 1 || tk.top != tk.Tp - 1)) { failed.push_back(i); continue; }
                     if (o.status != 0) {  // prefilled score / end inconsistent with the sequences: no alignment exists
                         r->alignment = NULL; r->alignmentLength = 0;

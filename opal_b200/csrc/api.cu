@@ -175,12 +175,9 @@ struct CreateGate {
 
 // The body of opalSearchDatabase once the database is (or can be made) resident.  `ddb` may be NULL: it is
 // then created from db / dbSeqLengths if any entry needs work.  db / dbSeqLengths may be NULL for handle calls.
-static int search_into_results(DeviceDb* ddb, const unsigned char* query, int queryLength, unsigned char* const* db, int dbLength,
-                               const int* dbSeqLengths, int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength,
-                               OpalSearchResult* results[], const int searchType, int mode, int device,
-                               CreateGate* gate = nullptr, int ticket = 0, const int* pssm = nullptr) {
-    if (mode != OPAL_MODE_NW && mode != OPAL_MODE_HW && mode != OPAL_MODE_OV && mode != OPAL_MODE_SW)
-        return OPAL_ERR_INVALID_MODE;  // :1469-1473, results untouched
+static int search_into_results(DeviceDb* ddb, const Scoring& s, unsigned char* const* db, int dbLength, const int* dbSeqLengths,
+                               OpalSearchResult* results[], const int searchType, int device, CreateGate* gate = nullptr, int ticket = 0) {
+    if (!valid_mode(s.mode)) return OPAL_ERR_INVALID_MODE;  // :1469-1473, results untouched
     if (dbLength <= 0) return 0;
 
     // Entries that already hold what this search level needs are not recomputed (:1446-1451).
@@ -213,12 +210,10 @@ static int search_into_results(DeviceDb* ddb, const unsigned char* query, int qu
     const auto t1 = now();
     int status = 0;
     if (anyWork)  // results go straight into the records (same pass also sets the no-alignment fields, :1508-1515)
-        status = ddb->search(query, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd, mode, skip.data(), nullptr,
-                             nullptr, nullptr, nullptr, results, searchType != OPAL_SEARCH_ALIGNMENT, pssm);
+        status = ddb->search(s, wantEnd, skip.data(), SearchOut::into(results, searchType != OPAL_SEARCH_ALIGNMENT), nullptr);
     const auto t2 = now();
     if (status == 0 && searchType == OPAL_SEARCH_ALIGNMENT)
-        status = align_database(ddb, query, queryLength, db, dbLength, dbSeqLengths, gapOpen, gapExt, scoreMatrix, alphabetLength,
-                                results, mode, nullptr, pssm);
+        status = align_database(ddb, s, db, dbLength, dbSeqLengths, results);
     const auto t3 = now();
     delete owned;
     if (trace)
@@ -246,7 +241,8 @@ int opalSearchDatabase(unsigned char query[], int queryLength, unsigned char* db
     (void)overflowMethod;  // OPAL_OVERFLOW_SIMPLE / _BUCKETS only schedule the reference's passes; results are equal
     const std::vector<int> devices = env_devices();
     const int D = (int)std::min<size_t>(devices.size(), (size_t)std::max(dbLength / 2, 1));
-    const bool modeOk = mode == OPAL_MODE_NW || mode == OPAL_MODE_HW || mode == OPAL_MODE_OV || mode == OPAL_MODE_SW;
+    const bool modeOk = valid_mode(mode);
+    const Scoring scoring = Scoring::with_matrix(query, queryLength, scoreMatrix, alphabetLength, gapOpen, gapExt, mode);
     // A large database is cut into a few SLICES per device (longest sequences first) that are staged, uploaded and
     // searched as databases of their own, each on a host thread and streams of its own: the first slice is being
     // searched while the others are still on their way, and a slice's records are written while the next one's kernels
@@ -261,8 +257,7 @@ int opalSearchDatabase(unsigned char query[], int queryLength, unsigned char* db
     if (const char* e = getenv("OPAL_B200_SLICES")) K = std::max(1, std::min(atoi(e), 16));
     K = std::min(K, std::max(dbLength / (2 * std::max(D, 1)), 1));
     if (D * K <= 1 || !modeOk)
-        return search_into_results(nullptr, query, queryLength, db, dbLength, dbSeqLengths, gapOpen, gapExt, scoreMatrix,
-                                   alphabetLength, results, searchType, mode, devices[0]);
+        return search_into_results(nullptr, scoring, db, dbLength, dbSeqLengths, results, searchType, devices[0]);
     // One call = the whole database (reference src/opal.h:150-154), on every listed device: each searches the parts
     // dealt to it and fills the caller's records of those parts; the alignment stage stays on the owning device.
     std::shared_ptr<const Layout> lay = layout_for(dbSeqLengths, nullptr, dbLength, false, nullptr);
@@ -281,8 +276,8 @@ int opalSearchDatabase(unsigned char query[], int queryLength, unsigned char* db
         std::vector<OpalSearchResult*> res(idx.size());
         for (size_t j = 0; j < idx.size(); j++) { ptr[j] = db[idx[j]]; len[j] = dbSeqLengths[idx[j]]; res[j] = results[idx[j]]; }
         set_thread_overlapped(k + 1 < K);  // other slices follow on this device: plan for throughput, not for the last task's end
-        const int rc = search_into_results(nullptr, query, queryLength, ptr.data(), (int)idx.size(), len.data(), gapOpen, gapExt,
-                                           scoreMatrix, alphabetLength, res.data(), searchType, mode, devices[d], K > 1 ? &gates[d] : nullptr, k);
+        const int rc = search_into_results(nullptr, scoring, ptr.data(), (int)idx.size(), len.data(), res.data(), searchType, devices[d],
+                                           K > 1 ? &gates[d] : nullptr, k);
         set_thread_overlapped(false);
         return rc;
     });
@@ -308,8 +303,8 @@ int opalSearchDatabaseCharSW(unsigned char query[], int queryLength, unsigned ch
     if (argsFit) {
         DeviceDb* ddb = DeviceDb::create(db, dbLength, dbSeqLengths, env_devices()[0]);
         if (!ddb) return OPAL_ERR_NO_SIMD_SUPPORT;
-        const int st = ddb->search(query, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, 0, OPAL_MODE_SW, nullptr,
-                                   sc.data(), nullptr, nullptr, nullptr);
+        const int st = ddb->search(Scoring::with_matrix(query, queryLength, scoreMatrix, alphabetLength, gapOpen, gapExt, OPAL_MODE_SW), 0,
+                                   nullptr, SearchOut::arrays(sc.data(), nullptr, nullptr), nullptr);
         delete ddb;
         if (st == OPAL_ERR_NO_SIMD_SUPPORT) return st;
         if (st) std::fill(sc.begin(), sc.end(), -1);
@@ -328,9 +323,6 @@ int opalSearchDatabaseCharSW(unsigned char query[], int queryLength, unsigned ch
 }
 
 // ------------------------------------------------------------------ opal_b200.h
-// PSSM entry points: the rows of a search of queryLength 0 (pssm may then be NULL; nothing is read through it).
-static const int kNoPssmRows = 0;
-
 // Arguments only the PSSM entry points have: the PSSM itself, and -- for OPAL_SEARCH_ALIGNMENT -- the residues it was
 // built for, which label the diagonal steps of an alignment MATCH / MISMATCH.  0 or OPAL_ERR_INVALID_ARGUMENT.
 static int check_pssm_args(const int* pssm, const unsigned char* query, int queryLength, int alphabetLength, int searchType) {
@@ -413,17 +405,14 @@ long long opalb200_db_residues(const OpalB200Db* h) { return reinterpret_cast<co
 
 int opalb200_db_devices(const OpalB200Db* h) { return reinterpret_cast<const DbHandle*>(h)->parts(); }
 
-// opalb200_db_search and opalb200_db_search_pssm (pssm non-NULL: query and scoreMatrix unused)
-static int db_search(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int gapOpen, int gapExt,
-                     const int* scoreMatrix, int alphabetLength, int searchType, int mode, const unsigned char* skip,
-                     int* scores, int* endQuery, int* endTarget, float* deviceMs) {
+static int db_search(OpalB200Db* hh, const Scoring& scoring, int searchType, const unsigned char* skip, int* scores, int* endQuery,
+                     int* endTarget, float* deviceMs) {
     if (!hh || !scores) return OPAL_ERR_NO_SIMD_SUPPORT;
     DeviceGuard guard;
     DbHandle* h = reinterpret_cast<DbHandle*>(hh);
     const int wantEnd = searchType != OPAL_SEARCH_SCORE && endQuery && endTarget;
     if (h->index.empty()) {
-        const int rc = h->shards[0]->search(query, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd, mode, skip, scores,
-                                            endQuery, endTarget, deviceMs, nullptr, false, pssm);
+        const int rc = h->shards[0]->search(scoring, wantEnd, skip, SearchOut::arrays(scores, endQuery, endTarget), deviceMs);
         h->collect_stats();
         return rc;
     }
@@ -434,8 +423,8 @@ static int db_search(OpalB200Db* hh, const unsigned char query[], const int* pss
         std::vector<int> sc(m), eq(m, -1), et(m, -1);
         std::vector<unsigned char> sk;
         if (skip) { sk.resize(m); for (size_t k = 0; k < m; k++) sk[k] = skip[idx[k]]; }
-        const int r = h->shards[s]->search(query, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd, mode,
-                                           skip ? sk.data() : nullptr, sc.data(), eq.data(), et.data(), &ms[s], nullptr, false, pssm);
+        const int r = h->shards[s]->search(scoring, wantEnd, skip ? sk.data() : nullptr, SearchOut::arrays(sc.data(), eq.data(), et.data()),
+                                           &ms[s]);
         if (r) return r;
         for (size_t k = 0; k < m; k++) {
             if (skip && sk[k]) continue;
@@ -453,8 +442,8 @@ static int db_search(OpalB200Db* hh, const unsigned char query[], const int* pss
 int opalb200_db_search(OpalB200Db* hh, const unsigned char query[], int queryLength, int gapOpen, int gapExt,
                        const int* scoreMatrix, int alphabetLength, int searchType, int mode, const unsigned char* skip,
                        int* scores, int* endQuery, int* endTarget, float* deviceMs) {
-    return db_search(hh, query, nullptr, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, searchType, mode, skip, scores,
-                     endQuery, endTarget, deviceMs);
+    return db_search(hh, Scoring::with_matrix(query, queryLength, scoreMatrix, alphabetLength, gapOpen, gapExt, mode), searchType, skip,
+                     scores, endQuery, endTarget, deviceMs);
 }
 
 int opalb200_db_search_pssm(OpalB200Db* hh, const int* pssm, int queryLength, int alphabetLength, int gapOpen, int gapExt,
@@ -462,63 +451,20 @@ int opalb200_db_search_pssm(OpalB200Db* hh, const int* pssm, int queryLength, in
                             float* deviceMs) {
     if (deviceMs) *deviceMs = 0.f;
     if (const int rc = check_pssm_args(pssm, nullptr, queryLength, alphabetLength, OPAL_SEARCH_SCORE)) return rc;
-    return db_search(hh, nullptr, pssm ? pssm : &kNoPssmRows, queryLength, gapOpen, gapExt, nullptr, alphabetLength, searchType, mode,
-                     skip, scores, endQuery, endTarget, deviceMs);
+    return db_search(hh, Scoring::with_pssm(nullptr, pssm, queryLength, alphabetLength, gapOpen, gapExt, mode), searchType, skip, scores,
+                     endQuery, endTarget, deviceMs);
 }
 
-static int search_batch_modes(OpalB200Db* hh, int numQueries, const unsigned char* const queries[], const int queryLengths[],
-                              int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength, int searchType, int mode,
-                              const int* modes, int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs,
-                              const int* const* pssms = nullptr);
-
-int opalb200_db_search_batch(OpalB200Db* hh, int numQueries, const unsigned char* const queries[], const int queryLengths[],
-                             int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength, int searchType, int mode,
-                             int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs) {
-    return search_batch_modes(hh, numQueries, queries, queryLengths, gapOpen, gapExt, scoreMatrix, alphabetLength, searchType, mode,
-                              nullptr, scores, endQuery, endTarget, inFlight, batchMs);
-}
-
-int opalb200_db_search_batch_modes(OpalB200Db* hh, int numSearches, const unsigned char* const queries[], const int queryLengths[],
-                                   const int modes[], int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength,
-                                   int searchType, int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs) {
-    if (numSearches > 0 && !modes) return OPAL_ERR_INVALID_MODE;
-    for (int q = 0; q < numSearches; q++)
-        if (modes[q] != OPAL_MODE_NW && modes[q] != OPAL_MODE_HW && modes[q] != OPAL_MODE_OV && modes[q] != OPAL_MODE_SW)
-            return OPAL_ERR_INVALID_MODE;
-    return search_batch_modes(hh, numSearches, queries, queryLengths, gapOpen, gapExt, scoreMatrix, alphabetLength, searchType,
-                              OPAL_MODE_SW, modes, scores, endQuery, endTarget, inFlight, batchMs);
-}
-
-int opalb200_db_search_batch_pssm(OpalB200Db* hh, int numSearches, const int* const pssms[], const int queryLengths[], const int modes[],
-                                  int alphabetLength, int gapOpen, int gapExt, int searchType, int* scores, int* endQuery,
-                                  int* endTarget, int inFlight, float* batchMs) {
-    if (batchMs) *batchMs = 0.f;
-    if (numSearches > 0 && !modes) return OPAL_ERR_INVALID_MODE;
-    if (numSearches > 0 && (!pssms || !queryLengths)) { set_error("pssms / queryLengths is NULL"); return OPAL_ERR_INVALID_ARGUMENT; }
-    for (int q = 0; q < numSearches; q++)
-        if (modes[q] != OPAL_MODE_NW && modes[q] != OPAL_MODE_HW && modes[q] != OPAL_MODE_OV && modes[q] != OPAL_MODE_SW)
-            return OPAL_ERR_INVALID_MODE;
-    std::vector<const int*> rows((size_t)std::max(numSearches, 0));
-    for (int q = 0; q < numSearches; q++) {
-        if (const int rc = check_pssm_args(pssms[q], nullptr, queryLengths[q], alphabetLength, OPAL_SEARCH_SCORE)) return rc;
-        rows[q] = pssms[q] ? pssms[q] : &kNoPssmRows;
-    }
-    return search_batch_modes(hh, numSearches, nullptr, queryLengths, gapOpen, gapExt, nullptr, alphabetLength, searchType,
-                              OPAL_MODE_SW, modes, scores, endQuery, endTarget, inFlight, batchMs, rows.data());
-}
-
-static int search_batch_modes(OpalB200Db* hh, int numQueries, const unsigned char* const queries[], const int queryLengths[],
-                              int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength, int searchType, int mode,
-                              const int* modes, int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs,
-                              const int* const* pssms) {
-    if (!hh || !scores || (numQueries > 0 && ((!queries && !pssms) || !queryLengths))) return OPAL_ERR_NO_SIMD_SUPPORT;
+// The batch entry points once their searches are built: outputs are [search][caller index].
+static int db_search_batch(OpalB200Db* hh, const std::vector<Scoring>& searches, int searchType, int* scores, int* endQuery,
+                           int* endTarget, int inFlight, float* batchMs) {
+    if (!hh || !scores) return OPAL_ERR_NO_SIMD_SUPPORT;
     DeviceGuard guard;
     DbHandle* h = reinterpret_cast<DbHandle*>(hh);
     const int wantEnd = searchType != OPAL_SEARCH_SCORE && endQuery && endTarget;
     const int fl = inFlight <= 0 ? 3 : inFlight;
     if (h->index.empty()) {
-        const int rc = h->shards[0]->search_batch(numQueries, queries, queryLengths, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd,
-                                                  mode, scores, endQuery, endTarget, fl, batchMs, modes, pssms);
+        const int rc = h->shards[0]->search_batch(searches, wantEnd, scores, endQuery, endTarget, fl, batchMs);
         h->collect_stats();
         return rc;
     }
@@ -526,15 +472,14 @@ static int search_batch_modes(OpalB200Db* hh, int numQueries, const unsigned cha
     const size_t n = (size_t)h->n;
     const int rc = on_shards(h->parts(), [&](int s) -> int {
         const std::vector<int>& idx = h->index[s];
-        const size_t m = idx.size(), all = m * (size_t)std::max(numQueries, 0);
+        const size_t m = idx.size(), all = m * searches.size();
         std::vector<int> sc(all), eq(wantEnd ? all : 0), et(wantEnd ? all : 0);
-        const int r = h->shards[s]->search_batch(numQueries, queries, queryLengths, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd,
-                                                 mode, sc.data(), wantEnd ? eq.data() : nullptr, wantEnd ? et.data() : nullptr, fl, &ms[s], modes,
-                                                 pssms);
+        const int r = h->shards[s]->search_batch(searches, wantEnd, sc.data(), wantEnd ? eq.data() : nullptr, wantEnd ? et.data() : nullptr,
+                                                 fl, &ms[s]);
         if (r) return r;
-        for (int q = 0; q < numQueries; q++)
+        for (size_t q = 0; q < searches.size(); q++)
             for (size_t k = 0; k < m; k++) {
-                const size_t to = (size_t)q * n + (size_t)idx[k], from = (size_t)q * m + k;
+                const size_t to = q * n + (size_t)idx[k], from = q * m + k;
                 scores[to] = sc[from];
                 if (endQuery) endQuery[to] = wantEnd ? eq[from] : -1;
                 if (endTarget) endTarget[to] = wantEnd ? et[from] : -1;
@@ -546,41 +491,73 @@ static int search_batch_modes(OpalB200Db* hh, int numQueries, const unsigned cha
     return rc;
 }
 
-// opalb200_db_search_results and opalb200_db_search_results_pssm (pssm non-NULL: scoreMatrix unused)
-static int db_search_results(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int gapOpen, int gapExt,
-                             const int* scoreMatrix, int alphabetLength, OpalSearchResult* results[], int searchType, int mode) {
+int opalb200_db_search_batch(OpalB200Db* hh, int numQueries, const unsigned char* const queries[], const int queryLengths[],
+                             int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength, int searchType, int mode,
+                             int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs) {
+    if (numQueries > 0 && (!queries || !queryLengths)) return OPAL_ERR_NO_SIMD_SUPPORT;
+    std::vector<Scoring> searches;
+    for (int q = 0; q < numQueries; q++)
+        searches.push_back(Scoring::with_matrix(queries[q], queryLengths[q], scoreMatrix, alphabetLength, gapOpen, gapExt, mode));
+    return db_search_batch(hh, searches, searchType, scores, endQuery, endTarget, inFlight, batchMs);
+}
+
+int opalb200_db_search_batch_modes(OpalB200Db* hh, int numSearches, const unsigned char* const queries[], const int queryLengths[],
+                                   const int modes[], int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength,
+                                   int searchType, int* scores, int* endQuery, int* endTarget, int inFlight, float* batchMs) {
+    if (numSearches > 0 && !modes) return OPAL_ERR_INVALID_MODE;
+    for (int q = 0; q < numSearches; q++)
+        if (!valid_mode(modes[q])) return OPAL_ERR_INVALID_MODE;
+    if (numSearches > 0 && (!queries || !queryLengths)) return OPAL_ERR_NO_SIMD_SUPPORT;
+    std::vector<Scoring> searches;
+    for (int q = 0; q < numSearches; q++)
+        searches.push_back(Scoring::with_matrix(queries[q], queryLengths[q], scoreMatrix, alphabetLength, gapOpen, gapExt, modes[q]));
+    return db_search_batch(hh, searches, searchType, scores, endQuery, endTarget, inFlight, batchMs);
+}
+
+int opalb200_db_search_batch_pssm(OpalB200Db* hh, int numSearches, const int* const pssms[], const int queryLengths[], const int modes[],
+                                  int alphabetLength, int gapOpen, int gapExt, int searchType, int* scores, int* endQuery,
+                                  int* endTarget, int inFlight, float* batchMs) {
+    if (batchMs) *batchMs = 0.f;
+    if (numSearches > 0 && !modes) return OPAL_ERR_INVALID_MODE;
+    if (numSearches > 0 && (!pssms || !queryLengths)) { set_error("pssms / queryLengths is NULL"); return OPAL_ERR_INVALID_ARGUMENT; }
+    for (int q = 0; q < numSearches; q++)
+        if (!valid_mode(modes[q])) return OPAL_ERR_INVALID_MODE;
+    std::vector<Scoring> searches;
+    for (int q = 0; q < numSearches; q++) {
+        if (const int rc = check_pssm_args(pssms[q], nullptr, queryLengths[q], alphabetLength, OPAL_SEARCH_SCORE)) return rc;
+        searches.push_back(Scoring::with_pssm(nullptr, pssms[q], queryLengths[q], alphabetLength, gapOpen, gapExt, modes[q]));
+    }
+    return db_search_batch(hh, searches, searchType, scores, endQuery, endTarget, inFlight, batchMs);
+}
+
+static int db_search_results(OpalB200Db* hh, const Scoring& scoring, OpalSearchResult* results[], int searchType) {
     if (!hh || !results) return OPAL_ERR_NO_SIMD_SUPPORT;
     DeviceGuard guard;
     DbHandle* h = reinterpret_cast<DbHandle*>(hh);
     if (h->index.empty())
-        return search_into_results(h->shards[0], query, queryLength, nullptr, h->n, nullptr, gapOpen, gapExt, scoreMatrix, alphabetLength,
-                                   results, searchType, mode, h->shards[0]->device(), nullptr, 0, pssm);
-    if (mode != OPAL_MODE_NW && mode != OPAL_MODE_HW && mode != OPAL_MODE_OV && mode != OPAL_MODE_SW) return OPAL_ERR_INVALID_MODE;
+        return search_into_results(h->shards[0], scoring, nullptr, h->n, nullptr, results, searchType, h->shards[0]->device());
+    if (!valid_mode(scoring.mode)) return OPAL_ERR_INVALID_MODE;
     return on_shards(h->parts(), [&](int s) -> int {
         const std::vector<int>& idx = h->index[s];
         std::vector<OpalSearchResult*> res(idx.size());
         for (size_t k = 0; k < idx.size(); k++) res[k] = results[idx[k]];
-        return search_into_results(h->shards[s], query, queryLength, nullptr, (int)idx.size(), nullptr, gapOpen, gapExt, scoreMatrix,
-                                   alphabetLength, res.data(), searchType, mode, h->shards[s]->device(), nullptr, 0, pssm);
+        return search_into_results(h->shards[s], scoring, nullptr, (int)idx.size(), nullptr, res.data(), searchType, h->shards[s]->device());
     });
 }
 
 int opalb200_db_search_results(OpalB200Db* hh, const unsigned char query[], int queryLength, int gapOpen, int gapExt,
                                const int* scoreMatrix, int alphabetLength, OpalSearchResult* results[], int searchType, int mode) {
-    return db_search_results(hh, query, nullptr, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, results, searchType, mode);
+    return db_search_results(hh, Scoring::with_matrix(query, queryLength, scoreMatrix, alphabetLength, gapOpen, gapExt, mode), results,
+                             searchType);
 }
 
 int opalb200_db_search_results_pssm(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int alphabetLength,
                                     int gapOpen, int gapExt, OpalSearchResult* results[], int searchType, int mode) {
     if (const int rc = check_pssm_args(pssm, query, queryLength, alphabetLength, searchType)) return rc;
-    return db_search_results(hh, searchType == OPAL_SEARCH_ALIGNMENT ? query : nullptr, pssm ? pssm : &kNoPssmRows, queryLength, gapOpen,
-                             gapExt, nullptr, alphabetLength, results, searchType, mode);
+    return db_search_results(hh, Scoring::with_pssm(query, pssm, queryLength, alphabetLength, gapOpen, gapExt, mode), results, searchType);
 }
 
-// opalb200_db_search_topk and opalb200_db_search_topk_pssm (pssm non-NULL: scoreMatrix unused)
-static int db_search_topk(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int gapOpen, int gapExt,
-                          const int* scoreMatrix, int alphabetLength, int searchType, int mode, int k, int* indices,
-                          OpalSearchResult* results[], int* found) {
+static int db_search_topk(OpalB200Db* hh, const Scoring& scoring, int searchType, int k, int* indices, OpalSearchResult* results[], int* found) {
     if (found) *found = 0;
     if (!hh || !indices || !results || k < 0) return OPAL_ERR_NO_SIMD_SUPPORT;
     DeviceGuard guard;
@@ -595,8 +572,7 @@ static int db_search_topk(OpalB200Db* hh, const unsigned char query[], const int
         const int m = h->shards[s]->size(), ks = std::min(kk, m);
         std::vector<int> li((size_t)ks), sc((size_t)ks), eq((size_t)ks), et((size_t)ks);
         const int* map = h->index.empty() ? nullptr : h->index[s].data();
-        const int r = h->shards[s]->search_topk(query, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, wantEnd, mode, ks, map,
-                                                li.data(), sc.data(), eq.data(), et.data(), pssm);
+        const int r = h->shards[s]->search_topk(scoring, wantEnd, ks, map, li.data(), sc.data(), eq.data(), et.data());
         if (r) return r;
         for (int j = 0; j < ks; j++) perShard[s].push_back({sc[j], h->caller_index(s, li[j]), eq[j], et[j], s, li[j]});
         return 0;
@@ -624,8 +600,7 @@ static int db_search_topk(OpalB200Db* hh, const unsigned char query[], const int
             for (int j = 0; j < kk; j++)
                 if (hits[j].shard == s) { subset.push_back(hits[j].local); res.push_back(results[j]); }
             if (subset.empty()) return 0;
-            return align_database(h->shards[s], query, queryLength, nullptr, (int)subset.size(), nullptr, gapOpen, gapExt, scoreMatrix,
-                                  alphabetLength, res.data(), mode, subset.data(), pssm);
+            return align_database(h->shards[s], scoring, nullptr, (int)subset.size(), nullptr, res.data(), subset.data());
         });
     return status;
 }
@@ -633,8 +608,8 @@ static int db_search_topk(OpalB200Db* hh, const unsigned char query[], const int
 int opalb200_db_search_topk(OpalB200Db* hh, const unsigned char query[], int queryLength, int gapOpen, int gapExt,
                             const int* scoreMatrix, int alphabetLength, int searchType, int mode, int k, int* indices,
                             OpalSearchResult* results[], int* found) {
-    return db_search_topk(hh, query, nullptr, queryLength, gapOpen, gapExt, scoreMatrix, alphabetLength, searchType, mode, k, indices,
-                          results, found);
+    return db_search_topk(hh, Scoring::with_matrix(query, queryLength, scoreMatrix, alphabetLength, gapOpen, gapExt, mode), searchType, k,
+                          indices, results, found);
 }
 
 int opalb200_db_search_topk_pssm(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int alphabetLength,
@@ -642,8 +617,8 @@ int opalb200_db_search_topk_pssm(OpalB200Db* hh, const unsigned char query[], co
                                  int* found) {
     if (found) *found = 0;
     if (const int rc = check_pssm_args(pssm, query, queryLength, alphabetLength, searchType)) return rc;
-    return db_search_topk(hh, searchType == OPAL_SEARCH_ALIGNMENT ? query : nullptr, pssm ? pssm : &kNoPssmRows, queryLength, gapOpen,
-                          gapExt, nullptr, alphabetLength, searchType, mode, k, indices, results, found);
+    return db_search_topk(hh, Scoring::with_pssm(query, pssm, queryLength, alphabetLength, gapOpen, gapExt, mode), searchType, k, indices,
+                          results, found);
 }
 
 void opalb200_db_last_stats(const OpalB200Db* h, int* kernelLaunches, int* rerun32, int* G, int* R, int* passes,
