@@ -164,6 +164,28 @@ int opalb200_db_search_topk_pssm(OpalB200Db* handle, const unsigned char query[]
                                  int searchType, int mode, int k, int* indices,
                                  struct OpalSearchResult* results[], int* found);
 
+/*
+ * opalb200_db_search_topk for numSearches searches in one call, up to `inFlight` (1..16; <= 0: 3) of them on the device
+ * at a time as in opalb200_db_search_batch, with a mode per search (modes[s] = OPAL_MODE_*).  At
+ * OPAL_SEARCH_ALIGNMENT the hits of all searches are aligned in the same launches.  indices and results are
+ * numSearches x k, row-major: row s starts at s * k and holds exactly what opalb200_db_search_topk returns for search s
+ * alone.  *found (nullable) = min(k, dbLength), the count written in every row; later slots are untouched.  Every search
+ * is checked before any runs: a fault returns the code of the lowest-index search that has one, writes no record and
+ * leaves *found = 0.
+ */
+int opalb200_db_search_batch_topk(OpalB200Db* handle, int numSearches, const unsigned char* const queries[],
+                                  const int queryLengths[], const int modes[], int gapOpen, int gapExt,
+                                  const int* scoreMatrix, int alphabetLength, int searchType, int k,
+                                  int* indices, struct OpalSearchResult* results[], int* found, int inFlight);
+
+/* opalb200_db_search_batch_topk with one PSSM per search (pssms[s]: queryLengths[s] x alphabetLength, see
+ * opalb200_db_search_pssm).  queries[s] labels the alignments' diagonal steps; `queries` and any queries[s] may be NULL
+ * below OPAL_SEARCH_ALIGNMENT. */
+int opalb200_db_search_batch_topk_pssm(OpalB200Db* handle, int numSearches, const unsigned char* const queries[],
+                                       const int* const pssms[], const int queryLengths[], const int modes[],
+                                       int alphabetLength, int gapOpen, int gapExt, int searchType, int k,
+                                       int* indices, struct OpalSearchResult* results[], int* found, int inFlight);
+
 /* Statistics of the last search on this handle: kernels launched, targets re-run in 32 bits, and the
  * geometry of the last launched class (threads per target pair, query rows per thread, passes over the
  * query, resident warps per SM scheduler partition), and the number of concurrent launch groups. Any pointer may be NULL. */

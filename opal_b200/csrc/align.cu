@@ -45,6 +45,15 @@ struct AlignTask {
     int score;
     int bottom, top;         // band
     int rowBlocks;           // ceil(Qp / 8)
+    int search;              // its entry in the search table
+};
+
+// What the tasks of one search share (device pointers): the query, the entries (the A x A matrix, or with byPssm the
+// Q x A PSSM), the mode and the gap penalties.  One launch holds the tasks of every search in the table.
+struct AlignSearch {
+    const uint8_t* query;
+    const int* entries;
+    int A, Go, Ge, mode, byPssm;
 };
 
 struct AlignOut {
@@ -59,11 +68,14 @@ __device__ __forceinline__ int sat_sub(int x, int g) { return max(x - g, kNegInf
 // ---------------------------------------------------------------- kernel 1: DP + decision bits
 // With a PSSM (pssm non-NULL, Q x A) reversed row r is scored by PSSM row endQ - r instead of the matrix row of its query
 // letter; `matrixInSmem` then means that a pass's 32 x kRows rows of it are staged in shared memory.
-__global__ void __launch_bounds__(32) align_dp_kernel(const AlignTask* tasks, AlignOut* outs, const uint8_t* residues,
-                                                      const uint8_t* query, const int* matrix, const int* pssm, int A, int Go, int Ge,
-                                                      int mode, uint32_t* flags, uint8_t* eqRows, int* bnd, int matrixInSmem) {
+__global__ void __launch_bounds__(32) align_dp_kernel(const AlignTask* tasks, const AlignSearch* searches, AlignOut* outs,
+                                                      const uint8_t* residues, uint32_t* flags, uint8_t* eqRows, int* bnd, int matrixInSmem) {
     extern __shared__ int smemMatrix[];
     const AlignTask task = tasks[blockIdx.x];
+    const AlignSearch sr = searches[task.search];
+    const uint8_t* query = sr.query;
+    const int *matrix = sr.entries, *pssm = sr.byPssm ? sr.entries : nullptr;
+    const int A = sr.A, Go = sr.Go, Ge = sr.Ge, mode = sr.mode;
     const int t = threadIdx.x;
     const int* S = pssm ? pssm : matrix;
     if (matrixInSmem && !pssm) {
@@ -167,14 +179,15 @@ __global__ void __launch_bounds__(32) align_dp_kernel(const AlignTask* tasks, Al
 }
 
 // ---------------------------------------------------------------- kernel 2: traceback
-__global__ void align_traceback_kernel(const AlignTask* tasks, AlignOut* outs, int numTasks, const uint8_t* residues,
-                                       const uint8_t* query, int mode, const uint32_t* flags, const uint8_t* eqRows,
-                                       uint8_t* ops) {
+__global__ void align_traceback_kernel(const AlignTask* tasks, const AlignSearch* searches, AlignOut* outs, int numTasks,
+                                       const uint8_t* residues, const uint32_t* flags, const uint8_t* eqRows, uint8_t* ops) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= numTasks) return;
     const AlignTask task = tasks[i];
     AlignOut o = outs[i];
     if (o.status != 0) return;
+    const uint8_t* query = searches[task.search].query;
+    const int mode = searches[task.search].mode;
     const int ce = o.stopCol;
     int re;
     if (mode == OPAL_MODE_NW || mode == OPAL_MODE_HW) re = task.Qp - 1;  // src/opal.cpp:1341-1350
@@ -302,31 +315,35 @@ bool replay_ok(const Scoring& s, const unsigned char* t, int T, const unsigned c
 
 }  // namespace
 
-int align_database(DeviceDb* ddb, const Scoring& s, unsigned char* const* db, int n, const int* lens, OpalSearchResult* results[],
-                   const int* subset) {
-    const int Q = s.Q, A = s.A, Go = s.Go, Ge = s.Ge, mode = s.mode;
+int align_database(DeviceDb* ddb, const std::vector<AlignSet>& sets, unsigned char* const* db, const int* lens) {
     if (!ddb || !ddb->ensure_uploaded()) return OPAL_B200_ERR_CUDA;
-    // target i on the host: the caller's pointer, or (resident-handle calls) the database's own sorted copy
-    // record j describes database entry entry(j): all of them, or the given subset (top-k pipelines)
-    auto entry = [&](int j) { return subset ? subset[j] : j; };
-    auto target_len = [&](int j) { return lens ? lens[entry(j)] : ddb->sorted_lengths()[ddb->sorted_position()[entry(j)]]; };
-    auto target_ptr = [&](int j) -> const unsigned char* {
-        return db ? db[entry(j)] : ddb->h_residues() + ddb->offsets()[ddb->sorted_position()[entry(j)]];
+    const int ns = (int)sets.size();
+    // target of record j of search q on the host: the caller's pointer, or (resident-handle calls) the database's own
+    // sorted copy; the record describes database entry entry(q, j): all of them, or the search's subset (top-k pipelines)
+    auto entry = [&](int q, int j) { return sets[q].subset ? sets[q].subset[j] : j; };
+    auto target_len = [&](int q, int j) { return lens ? lens[entry(q, j)] : ddb->sorted_lengths()[ddb->sorted_position()[entry(q, j)]]; };
+    auto target_ptr = [&](int q, int j) -> const unsigned char* {
+        return db ? db[entry(q, j)] : ddb->h_residues() + ddb->offsets()[ddb->sorted_position()[entry(q, j)]];
     };
-    const int M = s.bounds().maxEntry;  // the band's M: the largest entry that can score a cell
+    std::vector<int> M((size_t)ns);  // the band's M of every search: the largest entry that can score a cell
 
     // ---- entries that have an alignment at all (src/opal.cpp:1479-1483)
-    std::vector<int> todo;
-    for (int i = 0; i < n; i++) {
-        OpalSearchResult* r = results[i];
-        if ((mode == OPAL_MODE_SW && r->score == 0) || r->endLocationQuery < 0 || r->endLocationTarget < 0 ||
-            r->endLocationQuery >= Q || r->endLocationTarget >= target_len(i)) {
-            r->alignment = NULL;
-            r->alignmentLength = 0;
-            r->startLocationQuery = r->startLocationTarget = -1;
-            r->endLocationQuery = r->endLocationTarget = -1;
-        } else {
-            todo.push_back(i);
+    struct Item { int q, j; };
+    std::vector<Item> todo;
+    for (int q = 0; q < ns; q++) {
+        const Scoring& s = *sets[q].s;
+        M[q] = s.bounds().maxEntry;
+        for (int j = 0; j < sets[q].n; j++) {
+            OpalSearchResult* r = sets[q].results[j];
+            if ((s.mode == OPAL_MODE_SW && r->score == 0) || r->endLocationQuery < 0 || r->endLocationTarget < 0 ||
+                r->endLocationQuery >= s.Q || r->endLocationTarget >= target_len(q, j)) {
+                r->alignment = NULL;
+                r->alignmentLength = 0;
+                r->startLocationQuery = r->startLocationTarget = -1;
+                r->endLocationQuery = r->endLocationTarget = -1;
+            } else {
+                todo.push_back({q, j});
+            }
         }
     }
     if (todo.empty()) return 0;
@@ -334,8 +351,7 @@ int align_database(DeviceDb* ddb, const Scoring& s, unsigned char* const* db, in
     const cudaStream_t stream = ddb->stream();
     cudaSetDevice(ddb->device());
     bool ok = true;
-    unsigned char* dQuery = nullptr;
-    int* dMatrix = nullptr;  // the matrix, or the PSSM
+    unsigned char* dArgs = nullptr;  // [search table | entries and query of every search]
     AlignTask* dTasks = nullptr;
     AlignOut* dOuts = nullptr;
     uint32_t* dFlags = nullptr;
@@ -343,9 +359,23 @@ int align_database(DeviceDb* ddb, const Scoring& s, unsigned char* const* db, in
     int* dBnd = nullptr;
     std::vector<unsigned char> hOps;
     std::vector<AlignOut> hOuts;
-    // matrix, or a pass's 32 x kRows PSSM rows, in shared memory when it fits
-    const size_t smemBytes = sizeof(int) * (size_t)A * (s.byPssm ? 32 * kRows : A);
+    // the table, then every search's entries (searches that share one matrix share one copy) and query: one upload
+    auto up16 = [](size_t x) { return (x + 15) / 16 * 16; };
+    std::vector<size_t> entOff((size_t)ns), qOff((size_t)ns);
+    size_t argsBytes = up16(sizeof(AlignSearch) * (size_t)ns), smemBytes = 0;
+    for (int q = 0; q < ns; q++) {
+        const Scoring& s = *sets[q].s;
+        entOff[q] = 0;
+        for (int p = 0; p < q && !entOff[q]; p++)
+            if (sets[p].s->entries == s.entries && sets[p].s->num_entries() == s.num_entries()) entOff[q] = entOff[p];
+        if (!entOff[q]) { entOff[q] = argsBytes; argsBytes += up16(sizeof(int) * (size_t)s.num_entries()); }
+        qOff[q] = argsBytes;
+        argsBytes += up16((size_t)s.Q + 16);
+        // matrix, or a pass's 32 x kRows PSSM rows, in shared memory when it fits
+        smemBytes = std::max(smemBytes, sizeof(int) * (size_t)s.A * (s.byPssm ? 32 * kRows : s.A));
+    }
     const int matrixInSmem = smemBytes <= 40000 ? 1 : 0;
+    std::vector<unsigned char> hArgs(argsBytes, 0);
     size_t freeB = 0, totalB = 0;
     cudaMemGetInfo(&freeB, &totalB);
     const long long budgetWords = (long long)std::max<size_t>(64u << 20, std::min<size_t>(freeB / 3, (size_t)16 << 30)) / 4;
@@ -357,37 +387,44 @@ int align_database(DeviceDb* ddb, const Scoring& s, unsigned char* const* db, in
         device_release(dev, dOps); device_release(dev, dBnd);
         dTasks = nullptr; dOuts = nullptr; dFlags = nullptr; dEq = nullptr; dOps = nullptr; dBnd = nullptr;
     };
-    ALIGN_OK(dalloc(&dQuery, (size_t)Q + 16));
-    ALIGN_OK(dalloc(&dMatrix, sizeof(int) * (size_t)s.num_entries()));
-    ALIGN_TRY(cudaMemcpyAsync(dQuery, s.query, Q, cudaMemcpyHostToDevice, stream));
-    ALIGN_TRY(cudaMemcpyAsync(dMatrix, s.entries, sizeof(int) * (size_t)s.num_entries(), cudaMemcpyHostToDevice, stream));
+    ALIGN_OK(dalloc(&dArgs, argsBytes));
+    for (int q = 0; q < ns; q++) {
+        const Scoring& s = *sets[q].s;
+        const AlignSearch sr{dArgs + qOff[q], reinterpret_cast<const int*>(dArgs + entOff[q]), s.A, s.Go, s.Ge, s.mode, s.byPssm ? 1 : 0};
+        memcpy(hArgs.data() + sizeof(AlignSearch) * q, &sr, sizeof(sr));
+        if (s.num_entries() > 0) memcpy(hArgs.data() + entOff[q], s.entries, sizeof(int) * (size_t)s.num_entries());
+        if (s.Q > 0 && s.query) memcpy(hArgs.data() + qOff[q], s.query, (size_t)s.Q);
+    }
+    ALIGN_TRY(cudaMemcpyAsync(dArgs, hArgs.data(), argsBytes, cudaMemcpyHostToDevice, stream));
 
     {
         // Two rounds at most: the reference's band first, the full band for entries whose replay fails.
-        std::vector<int> pending = todo;
+        std::vector<Item> pending = todo;
         for (int round = 0; round < 2 && !pending.empty(); round++) {
-            std::vector<int> failed;
+            std::vector<Item> failed;
             size_t cursor = 0;
             while (cursor < pending.size()) {
                 // ---- one batch within the memory budget
                 std::vector<AlignTask> tasks;
-                std::vector<int> ids;
+                std::vector<Item> ids;
                 long long flagWords = 0, opsBytes = 0, bndInts = 0;
                 while (cursor < pending.size()) {
-                    const int i = pending[cursor];
-                    const OpalSearchResult* r = results[i];
+                    const Item it = pending[cursor];
+                    const Scoring& s = *sets[it.q].s;
+                    const OpalSearchResult* r = sets[it.q].results[it.j];
                     AlignTask tk;
                     tk.Qp = r->endLocationQuery + 1; tk.Tp = r->endLocationTarget + 1;
                     tk.endQ = r->endLocationQuery; tk.endT = r->endLocationTarget; tk.score = r->score;
                     tk.rowBlocks = (tk.Qp + kRows - 1) / kRows;
+                    tk.search = it.q;
                     const long long words = (long long)tk.rowBlocks * tk.Tp;
                     if (!tasks.empty() && flagWords + words > budgetWords) break;
-                    if (round == 0 && band_borders(tk.score, mode, tk.Qp, tk.Tp, Go, Ge, M, &tk.bottom, &tk.top)) {}
+                    if (round == 0 && band_borders(tk.score, s.mode, tk.Qp, tk.Tp, s.Go, s.Ge, M[it.q], &tk.bottom, &tk.top)) {}
                     else { tk.bottom = tk.Qp - 1; tk.top = tk.Tp - 1; }
-                    tk.targetOffset = ddb->offsets()[ddb->sorted_position()[entry(i)]];
+                    tk.targetOffset = ddb->offsets()[ddb->sorted_position()[entry(it.q, it.j)]];
                     tk.flagOffset = flagWords; tk.eqOffset = flagWords; tk.opsOffset = opsBytes; tk.bndOffset = bndInts;
                     flagWords += words; opsBytes += tk.Qp + tk.Tp + 8; bndInts += 2LL * tk.Tp;
-                    tasks.push_back(tk); ids.push_back(i);
+                    tasks.push_back(tk); ids.push_back(it);
                     cursor++;
                 }
                 const int nt = (int)tasks.size();
@@ -401,12 +438,11 @@ int align_database(DeviceDb* ddb, const Scoring& s, unsigned char* const* db, in
                 ALIGN_TRY(cudaMemcpyAsync(dTasks, tasks.data(), sizeof(AlignTask) * nt, cudaMemcpyHostToDevice, stream));
                 // an alignment is shorter than its slot: the unused tail travels back with the rest, so it is defined
                 ALIGN_TRY(cudaMemsetAsync(dOps, 0, (size_t)opsBytes, stream));
-                align_dp_kernel<<<nt, 32, matrixInSmem ? smemBytes : 0, stream>>>(dTasks, dOuts, ddb->d_residues(), dQuery,
-                                                                                   s.byPssm ? nullptr : dMatrix, s.byPssm ? dMatrix : nullptr, A,
-                                                                                   Go, Ge, mode, dFlags, dEq, dBnd, matrixInSmem);
+                const AlignSearch* dSearches = reinterpret_cast<const AlignSearch*>(dArgs);
+                align_dp_kernel<<<nt, 32, matrixInSmem ? smemBytes : 0, stream>>>(dTasks, dSearches, dOuts, ddb->d_residues(), dFlags, dEq,
+                                                                                   dBnd, matrixInSmem);
                 ALIGN_TRY(cudaGetLastError());
-                align_traceback_kernel<<<(nt + 63) / 64, 64, 0, stream>>>(dTasks, dOuts, nt, ddb->d_residues(), dQuery, mode, dFlags, dEq,
-                                                                           dOps);
+                align_traceback_kernel<<<(nt + 63) / 64, 64, 0, stream>>>(dTasks, dSearches, dOuts, nt, ddb->d_residues(), dFlags, dEq, dOps);
                 ALIGN_TRY(cudaGetLastError());
                 hOps.resize((size_t)opsBytes);
                 hOuts.resize(nt);
@@ -414,14 +450,15 @@ int align_database(DeviceDb* ddb, const Scoring& s, unsigned char* const* db, in
                 ALIGN_TRY(cudaMemcpyAsync(hOuts.data(), dOuts, sizeof(AlignOut) * nt, cudaMemcpyDeviceToHost, stream));
                 ALIGN_TRY(cudaStreamSynchronize(stream));
                 for (int k = 0; k < nt; k++) {
-                    const int i = ids[k];
-                    OpalSearchResult* r = results[i];
+                    const Item it = ids[k];
+                    OpalSearchResult* r = sets[it.q].results[it.j];
                     const AlignOut& o = hOuts[k];
                     const AlignTask& tk = tasks[k];
                     const unsigned char* ops = hOps.data() + tk.opsOffset;
                     const int sq = tk.endQ - o.endRow, st = tk.endT - o.stopCol;  // src/opal.cpp:1499-1500
-                    const bool good = o.status == 0 && replay_ok(s, target_ptr(i), target_len(i), ops, o.opsLen, sq, st, tk.endQ, tk.endT, tk.score);
-                    if (!good && round == 0 && (tk.bottom != tk.Qp - 1 || tk.top != tk.Tp - 1)) { failed.push_back(i); continue; }
+                    const bool good = o.status == 0 && replay_ok(*sets[it.q].s, target_ptr(it.q, it.j), target_len(it.q, it.j), ops, o.opsLen, sq,
+                                                                 st, tk.endQ, tk.endT, tk.score);
+                    if (!good && round == 0 && (tk.bottom != tk.Qp - 1 || tk.top != tk.Tp - 1)) { failed.push_back(it); continue; }
                     if (o.status != 0) {  // prefilled score / end inconsistent with the sequences: no alignment exists
                         r->alignment = NULL; r->alignmentLength = 0;
                         r->startLocationQuery = r->startLocationTarget = -1;
@@ -439,7 +476,7 @@ int align_database(DeviceDb* ddb, const Scoring& s, unsigned char* const* db, in
     }
 done:
     cudaStreamSynchronize(stream);  // nothing may still be using the blocks when they go back to the cache
-    device_release(dev, dQuery); device_release(dev, dMatrix);
+    device_release(dev, dArgs);
     release_batch();
     return ok ? 0 : OPAL_B200_ERR_CUDA;
 }

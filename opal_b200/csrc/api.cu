@@ -213,7 +213,7 @@ static int search_into_results(DeviceDb* ddb, const Scoring& s, unsigned char* c
         status = ddb->search(s, wantEnd, skip.data(), SearchOut::into(results, searchType != OPAL_SEARCH_ALIGNMENT), nullptr);
     const auto t2 = now();
     if (status == 0 && searchType == OPAL_SEARCH_ALIGNMENT)
-        status = align_database(ddb, s, db, dbLength, dbSeqLengths, results);
+        status = align_database(ddb, {{&s, results, dbLength, nullptr}}, db, dbSeqLengths);
     const auto t3 = now();
     delete owned;
     if (trace)
@@ -557,50 +557,83 @@ int opalb200_db_search_results_pssm(OpalB200Db* hh, const unsigned char query[],
     return db_search_results(hh, Scoring::with_pssm(query, pssm, queryLength, alphabetLength, gapOpen, gapExt, mode), results, searchType);
 }
 
-static int db_search_topk(OpalB200Db* hh, const Scoring& scoring, int searchType, int k, int* indices, OpalSearchResult* results[], int* found) {
+// Score -> top-k -> alignment for a batch of searches; indices / results are [search][k] (row q starts at q * k).  Every
+// search is checked before any runs (the PSSM argument rule, then -- when anything is selected -- Scoring::validate and
+// the database's residue codes), in search order, so a fault reports the code of the lowest-index search that has one
+// and writes nothing.  Every shard searches and selects ITS k best of every search on the device (DeviceDb::search_batch_topk:
+// only k records per search and shard come back, not every score); the candidates are merged here: score descending,
+// caller index ascending among equals.  At OPAL_SEARCH_ALIGNMENT every shard then aligns the hits it owns, of all
+// searches in the same launches.
+static int db_search_batch_topk(OpalB200Db* hh, const std::vector<Scoring>& searches, int searchType, int k, int* indices,
+                                OpalSearchResult* results[], int* found, int inFlight) {
     if (found) *found = 0;
     if (!hh || !indices || !results || k < 0) return OPAL_ERR_NO_SIMD_SUPPORT;
     DeviceGuard guard;
     DbHandle* h = reinterpret_cast<DbHandle*>(hh);
-    const int n = h->n, kk = std::min(k, n), parts = h->parts();
+    const int n = h->n, kk = std::min(k, n), parts = h->parts(), ns = (int)searches.size();
     const int wantEnd = searchType != OPAL_SEARCH_SCORE;
-    // Every shard searches and selects ITS k best on the device (DeviceDb::search_topk: only k records per shard come
-    // back, not every score); the candidates are merged here: score descending, caller index ascending among equals.
+    for (const Scoring& sc : searches) {
+        if (sc.byPssm)
+            if (const int rc = check_pssm_args(sc.entries, sc.query, sc.Q, sc.A, searchType)) return rc;
+        for (int s = 0; s < parts && kk > 0; s++)
+            if (const int rc = h->shards[s]->check(sc)) return rc;
+    }
+    if (kk <= 0 || ns == 0) {
+        if (found) *found = kk;
+        return 0;
+    }
     struct Hit { int score, index, endQ, endT, shard, local; };
-    std::vector<std::vector<Hit>> perShard((size_t)parts);
+    std::vector<std::vector<Hit>> perShard((size_t)parts);  // [shard]: ks candidates of every search
+    auto shard_k = [&](int s) { return std::min(kk, h->shards[s]->size()); };
     int status = on_shards(parts, [&](int s) -> int {
-        const int m = h->shards[s]->size(), ks = std::min(kk, m);
-        std::vector<int> li((size_t)ks), sc((size_t)ks), eq((size_t)ks), et((size_t)ks);
+        const size_t all = (size_t)ns * (size_t)shard_k(s);
+        std::vector<int> li(all), sc(all), eq(all), et(all);
         const int* map = h->index.empty() ? nullptr : h->index[s].data();
-        const int r = h->shards[s]->search_topk(scoring, wantEnd, ks, map, li.data(), sc.data(), eq.data(), et.data());
+        const int r = h->shards[s]->search_batch_topk(searches, wantEnd, shard_k(s), map, li.data(), sc.data(), eq.data(), et.data(),
+                                                      inFlight <= 0 ? 3 : inFlight);
         if (r) return r;
-        for (int j = 0; j < ks; j++) perShard[s].push_back({sc[j], h->caller_index(s, li[j]), eq[j], et[j], s, li[j]});
+        for (size_t j = 0; j < all; j++) perShard[s].push_back({sc[j], h->caller_index(s, li[j]), eq[j], et[j], s, li[j]});
         return 0;
     });
     h->collect_stats();
     if (status) return status;
-    std::vector<Hit> hits;
-    for (auto& v : perShard) hits.insert(hits.end(), v.begin(), v.end());
     auto better = [](const Hit& a, const Hit& b) { return a.score != b.score ? a.score > b.score : a.index < b.index; };
-    std::sort(hits.begin(), hits.end(), better);
-    hits.resize((size_t)kk);
-    for (int j = 0; j < kk; j++) {
-        indices[j] = hits[j].index;
-        opalInitSearchResult(results[j]);
-        opalSearchResultSetScore(results[j], hits[j].score);
-        results[j]->endLocationQuery = wantEnd ? hits[j].endQ : -1;
-        results[j]->endLocationTarget = wantEnd ? hits[j].endT : -1;
-        results[j]->alignmentLength = -1;  // as opalSearchDatabase leaves it below OPAL_SEARCH_ALIGNMENT (:1508-1515)
+    std::vector<Hit> hits;  // [search][kk]
+    for (int q = 0; q < ns; q++) {
+        std::vector<Hit> cand;
+        for (int s = 0; s < parts; s++) {
+            const auto from = perShard[s].begin() + (size_t)q * shard_k(s);
+            cand.insert(cand.end(), from, from + shard_k(s));
+        }
+        std::sort(cand.begin(), cand.end(), better);
+        hits.insert(hits.end(), cand.begin(), cand.begin() + kk);
     }
+    auto slot = [&](int q, int j) { return (size_t)q * (size_t)k + (size_t)j; };
+    for (int q = 0; q < ns; q++)
+        for (int j = 0; j < kk; j++) {
+            const Hit& hit = hits[(size_t)q * kk + j];
+            OpalSearchResult* r = results[slot(q, j)];
+            indices[slot(q, j)] = hit.index;
+            opalInitSearchResult(r);
+            opalSearchResultSetScore(r, hit.score);
+            r->endLocationQuery = wantEnd ? hit.endQ : -1;
+            r->endLocationTarget = wantEnd ? hit.endT : -1;
+            r->alignmentLength = -1;  // as opalSearchDatabase leaves it below OPAL_SEARCH_ALIGNMENT (:1508-1515)
+        }
     if (found) *found = kk;
-    if (searchType == OPAL_SEARCH_ALIGNMENT && kk > 0)  // start + alignment on the device that owns the target
+    if (searchType == OPAL_SEARCH_ALIGNMENT)  // start + alignment on the device that owns the target
         status = on_shards(parts, [&](int s) -> int {
-            std::vector<int> subset;
-            std::vector<OpalSearchResult*> res;
-            for (int j = 0; j < kk; j++)
-                if (hits[j].shard == s) { subset.push_back(hits[j].local); res.push_back(results[j]); }
-            if (subset.empty()) return 0;
-            return align_database(h->shards[s], scoring, nullptr, (int)subset.size(), nullptr, res.data(), subset.data());
+            std::vector<std::vector<int>> subset((size_t)ns);
+            std::vector<std::vector<OpalSearchResult*>> res((size_t)ns);
+            for (int q = 0; q < ns; q++)
+                for (int j = 0; j < kk; j++) {
+                    const Hit& hit = hits[(size_t)q * kk + j];
+                    if (hit.shard == s) { subset[q].push_back(hit.local); res[q].push_back(results[slot(q, j)]); }
+                }
+            std::vector<AlignSet> sets;
+            for (int q = 0; q < ns; q++)
+                if (!subset[q].empty()) sets.push_back({&searches[q], res[q].data(), (int)subset[q].size(), subset[q].data()});
+            return sets.empty() ? 0 : align_database(h->shards[s], sets);
         });
     return status;
 }
@@ -608,17 +641,40 @@ static int db_search_topk(OpalB200Db* hh, const Scoring& scoring, int searchType
 int opalb200_db_search_topk(OpalB200Db* hh, const unsigned char query[], int queryLength, int gapOpen, int gapExt,
                             const int* scoreMatrix, int alphabetLength, int searchType, int mode, int k, int* indices,
                             OpalSearchResult* results[], int* found) {
-    return db_search_topk(hh, Scoring::with_matrix(query, queryLength, scoreMatrix, alphabetLength, gapOpen, gapExt, mode), searchType, k,
-                          indices, results, found);
+    return db_search_batch_topk(hh, {Scoring::with_matrix(query, queryLength, scoreMatrix, alphabetLength, gapOpen, gapExt, mode)},
+                                searchType, k, indices, results, found, 1);
 }
 
 int opalb200_db_search_topk_pssm(OpalB200Db* hh, const unsigned char query[], const int* pssm, int queryLength, int alphabetLength,
                                  int gapOpen, int gapExt, int searchType, int mode, int k, int* indices, OpalSearchResult* results[],
                                  int* found) {
+    return db_search_batch_topk(hh, {Scoring::with_pssm(query, pssm, queryLength, alphabetLength, gapOpen, gapExt, mode)}, searchType, k,
+                                indices, results, found, 1);
+}
+
+int opalb200_db_search_batch_topk(OpalB200Db* hh, int numSearches, const unsigned char* const queries[], const int queryLengths[],
+                                  const int modes[], int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength,
+                                  int searchType, int k, int* indices, OpalSearchResult* results[], int* found, int inFlight) {
     if (found) *found = 0;
-    if (const int rc = check_pssm_args(pssm, query, queryLength, alphabetLength, searchType)) return rc;
-    return db_search_topk(hh, Scoring::with_pssm(query, pssm, queryLength, alphabetLength, gapOpen, gapExt, mode), searchType, k, indices,
-                          results, found);
+    if (numSearches > 0 && !modes) return OPAL_ERR_INVALID_MODE;
+    if (numSearches > 0 && (!queries || !queryLengths)) return OPAL_ERR_NO_SIMD_SUPPORT;
+    std::vector<Scoring> searches;
+    for (int q = 0; q < numSearches; q++)
+        searches.push_back(Scoring::with_matrix(queries[q], queryLengths[q], scoreMatrix, alphabetLength, gapOpen, gapExt, modes[q]));
+    return db_search_batch_topk(hh, searches, searchType, k, indices, results, found, inFlight);
+}
+
+int opalb200_db_search_batch_topk_pssm(OpalB200Db* hh, int numSearches, const unsigned char* const queries[], const int* const pssms[],
+                                       const int queryLengths[], const int modes[], int alphabetLength, int gapOpen, int gapExt,
+                                       int searchType, int k, int* indices, OpalSearchResult* results[], int* found, int inFlight) {
+    if (found) *found = 0;
+    if (numSearches > 0 && !modes) return OPAL_ERR_INVALID_MODE;
+    if (numSearches > 0 && (!pssms || !queryLengths)) { set_error("pssms / queryLengths is NULL"); return OPAL_ERR_INVALID_ARGUMENT; }
+    std::vector<Scoring> searches;
+    for (int q = 0; q < numSearches; q++)
+        searches.push_back(Scoring::with_pssm(queries ? queries[q] : nullptr, pssms[q], queryLengths[q], alphabetLength, gapOpen, gapExt,
+                                              modes[q]));
+    return db_search_batch_topk(hh, searches, searchType, k, indices, results, found, inFlight);
 }
 
 void opalb200_db_last_stats(const OpalB200Db* h, int* kernelLaunches, int* rerun32, int* G, int* R, int* passes,

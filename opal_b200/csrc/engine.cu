@@ -1039,7 +1039,7 @@ DeviceDb* DeviceDb::clone_context() {
     c->lay_ = lay_;
     c->hResidues_ = hResidues_; c->dResidues_ = dResidues_; c->dOffsets_ = dOffsets_; c->dLengths_ = dLengths_;
     c->dPairStream_ = dPairStream_; c->dPairOffsets_ = dPairOffsets_; c->numPairs_ = numPairs_; c->maxCode_ = maxCode_;
-    c->dFoldStream_ = dFoldStream_; c->dFoldOffsets_ = dFoldOffsets_; c->numFold_ = numFold_;
+    c->dFoldStream_ = dFoldStream_; c->dFoldOffsets_ = dFoldOffsets_; c->numFold_ = numFold_; c->dOrder_ = dOrder_;
     if (cudaSetDevice(device_) != cudaSuccess || !c->alloc_search_buffers()) { delete c; return nullptr; }
     return c;
 }
@@ -1782,13 +1782,7 @@ int DeviceDb::search_topk(const Scoring& s, int wantEnd, int k, const int* map, 
     const size_t selectInts = (size_t)n_ + 4 * (size_t)kk + 16;
     int* dSelect = nullptr;  // [count | flagged positions (n) | k records]
     if (!device_alloc(device_, (void**)&dSelect, sizeof(int) * selectInts)) return OPAL_B200_ERR_CUDA;
-    if (!dOrder_) {
-        if (!ensure_uploaded() || !device_alloc(device_, (void**)&dOrder_, sizeof(int) * (size_t)std::max(n_, 1)) ||
-            cudaMemcpyAsync(dOrder_, lay_->order.data(), sizeof(int) * (size_t)n_, cudaMemcpyHostToDevice, stream_) != cudaSuccess ||
-            cudaStreamSynchronize(stream_) != cudaSuccess) {
-            set_error("upload of the index map failed"); device_release(device_, dSelect); return OPAL_B200_ERR_CUDA;
-        }
-    }
+    if (!ensure_order()) { device_release(device_, dSelect); return OPAL_B200_ERR_CUDA; }
     const int rc = search(s, wantEnd, nullptr, SearchOut::on_device(dSelect), nullptr);
     if (rc) { device_release(device_, dSelect); return rc; }
     int4* dRecords = reinterpret_cast<int4*>(dSelect + (((size_t)n_ + 4) & ~(size_t)3));
@@ -1809,12 +1803,35 @@ int DeviceDb::search_topk(const Scoring& s, int wantEnd, int k, const int* map, 
     return 0;
 }
 
-int DeviceDb::search_batch(const std::vector<Scoring>& searches, int wantEnd, int* scores, int* endQ, int* endT, int inFlight,
-                           float* batchMs) {
+// The device copy of the index map (sorted position -> caller index) that the selection reads, made once; the search
+// contexts borrow it as they borrow the database arrays.
+bool DeviceDb::ensure_order() {
+    if (dOrder_) return true;
+    if (!ensure_uploaded() || !device_alloc(device_, (void**)&dOrder_, sizeof(int) * (size_t)std::max(n_, 1)) ||
+        cudaMemcpyAsync(dOrder_, lay_->order.data(), sizeof(int) * (size_t)n_, cudaMemcpyHostToDevice, stream_) != cudaSuccess ||
+        cudaStreamSynchronize(stream_) != cudaSuccess) {
+        set_error("upload of the index map failed");
+        return false;
+    }
+    for (DeviceDb* c : contexts_) c->dOrder_ = dOrder_;
+    return true;
+}
+
+int DeviceDb::check(const Scoring& s) {
+    ScoreBounds b;
+    if (const int rc = s.validate(&b)) return rc;
+    if (s.Q <= 0 || lay_->nonEmpty == 0) return 0;  // nothing is swept, so no residue code is read (see run_classes)
+    if (!ensure_uploaded()) return OPAL_B200_ERR_CUDA;
+    if (maxCode_ >= s.A) { set_error("database holds residue codes >= alphabetLength"); return OPAL_B200_ERR_ARGUMENT; }
+    return 0;
+}
+
+// Searches claim the next index in order and stop claiming after a failure, so every search below the lowest failed
+// one has run: its code is the one a loop of single searches would have returned.
+int DeviceDb::in_flight(int num, int inFlight, const std::function<int(DeviceDb*, int)>& job, float* batchMs) {
     if (batchMs) *batchMs = 0.f;
-    const int numQueries = (int)searches.size();
-    if (numQueries <= 0) return 0;
-    const int K = std::max(1, std::min(std::min(inFlight, numQueries), 16));
+    if (num <= 0) return 0;
+    const int K = std::max(1, std::min(std::min(inFlight, num), 16));
     if (cudaSetDevice(device_) != cudaSuccess) { set_error("cudaSetDevice failed"); return OPAL_B200_ERR_CUDA; }
     while ((int)contexts_.size() < K - 1) {
         DeviceDb* c = clone_context();
@@ -1826,19 +1843,18 @@ int DeviceDb::search_batch(const std::vector<Scoring>& searches, int wantEnd, in
     if (!event_acquire(device_, &evBatch)) return OPAL_B200_ERR_CUDA;
     if (cudaEventRecord(evBatch, stream_) != cudaSuccess) { event_release(device_, evBatch); set_error("cudaEventRecord failed"); return OPAL_B200_ERR_CUDA; }
     std::atomic<int> next(0);
-    std::vector<int> rcs((size_t)K, 0);
-    std::vector<std::string> errors((size_t)K);
+    std::atomic<bool> stop(false);
+    std::vector<int> rcs((size_t)num, 0);
+    std::vector<std::string> errors((size_t)num);
     std::vector<float> lastStop((size_t)K, 0.f);
     std::vector<int> launches((size_t)K, 0), reruns((size_t)K, 0);
     auto worker = [&](int k) {
         DeviceDb* ctx = k == 0 ? this : contexts_[k - 1];
-        for (;;) {
+        while (!stop.load()) {
             const int q = next.fetch_add(1);
-            if (q >= numQueries) break;
-            const size_t base = (size_t)q * (size_t)n_;
-            const SearchOut out = SearchOut::arrays(scores + base, endQ ? endQ + base : nullptr, endT ? endT + base : nullptr);
-            const int rc = ctx->search(searches[q], wantEnd, nullptr, out, nullptr);
-            if (rc) { rcs[k] = rc; errors[k] = last_error(); break; }
+            if (q >= num) break;
+            const int rc = job(ctx, q);
+            if (rc) { rcs[q] = rc; errors[q] = last_error(); stop.store(true); break; }
             launches[k] += ctx->stats_.kernelLaunches; reruns[k] += ctx->stats_.rerun32;
             float ms = 0.f;
             if (ctx->startRecorded_ && cudaEventElapsedTime(&ms, evBatch, ctx->evStop_) == cudaSuccess) lastStop[k] = std::max(lastStop[k], ms);
@@ -1854,12 +1870,32 @@ int DeviceDb::search_batch(const std::vector<Scoring>& searches, int wantEnd, in
         for (auto& t : th) t.join();
     }
     event_release(device_, evBatch);
-    for (int k = 0; k < K; k++)
-        if (rcs[k]) { set_error(errors[k]); return rcs[k]; }
+    for (int q = 0; q < num; q++)
+        if (rcs[q]) { set_error(errors[q]); return rcs[q]; }
     if (batchMs) *batchMs = *std::max_element(lastStop.begin(), lastStop.end());
     stats_.kernelLaunches = stats_.rerun32 = 0;  // batch totals
     for (int k = 0; k < K; k++) { stats_.kernelLaunches += launches[k]; stats_.rerun32 += reruns[k]; }
     return 0;
+}
+
+int DeviceDb::search_batch(const std::vector<Scoring>& searches, int wantEnd, int* scores, int* endQ, int* endT, int inFlight,
+                           float* batchMs) {
+    return in_flight((int)searches.size(), inFlight, [&](DeviceDb* ctx, int q) {
+        const size_t base = (size_t)q * (size_t)n_;
+        const SearchOut out = SearchOut::arrays(scores + base, endQ ? endQ + base : nullptr, endT ? endT + base : nullptr);
+        return ctx->search(searches[q], wantEnd, nullptr, out, nullptr);
+    }, batchMs);
+}
+
+int DeviceDb::search_batch_topk(const std::vector<Scoring>& searches, int wantEnd, int k, const int* map, int* outIndex, int* outScore,
+                                int* outEndQ, int* outEndT, int inFlight) {
+    if (k <= 0 || searches.empty()) return 0;
+    if (cudaSetDevice(device_) != cudaSuccess) { set_error("cudaSetDevice failed"); return OPAL_B200_ERR_CUDA; }
+    if (!ensure_order()) return OPAL_B200_ERR_CUDA;  // before the contexts start: they borrow it
+    return in_flight((int)searches.size(), inFlight, [&](DeviceDb* ctx, int q) {
+        const size_t base = (size_t)q * (size_t)k;
+        return ctx->search_topk(searches[q], wantEnd, k, map, outIndex + base, outScore + base, outEndQ + base, outEndT + base);
+    }, nullptr);
 }
 
 // ------------------------------------------------------------------ DPX roofline probe

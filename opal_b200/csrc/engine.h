@@ -167,6 +167,13 @@ public:
     // Score [+ end] search followed by the selection of the k best targets: score descending, then smallest
     // map[caller index] (map NULL: the caller index itself).  Writes k (<= size()) caller indices and their records.
     int search_topk(const Scoring& s, int wantEnd, int k, const int* map, int* outIndex, int* outScore, int* outEndQ, int* outEndT);
+    // search_topk of every search, up to `inFlight` of them on the device at a time (as search_batch); k <= size().
+    // Outputs are [search][k].  0, or the code of the lowest-index search that failed.
+    int search_batch_topk(const std::vector<Scoring>& searches, int wantEnd, int k, const int* map, int* outIndex, int* outScore,
+                          int* outEndQ, int* outEndT, int inFlight);
+    // The checks a search makes before it sweeps: Scoring::validate, then (for a search that sweeps at all) the
+    // database's residue codes against the alphabet length.  0 or an OPAL_B200_ERR_* code.
+    int check(const Scoring& s);
 
     int size() const { return n_; }
     long long residues() const { return totalResidues_; }
@@ -186,6 +193,9 @@ private:
     DeviceDb() {}
     static DeviceDb* build(unsigned char* const* db, const unsigned char* packed, const int* lens, const int* order, int n, int device);
     DeviceDb* clone_context();
+    bool ensure_order();
+    // job(context, q) for every q in [0, num), up to inFlight at a time, each context on a host thread of its own.
+    int in_flight(int num, int inFlight, const std::function<int(DeviceDb*, int)>& job, float* batchMs);
     bool alloc_search_buffers();
     struct Group;
     struct Run;     // the search in progress (engine.cu)
@@ -231,7 +241,7 @@ private:
     SearchStats stats_;
     std::vector<void*> chainScratch_;  // device blocks of chained launches (boundary rows, flags), released by the next search
     bool startRecorded_ = false;
-    int* dOrder_ = nullptr;       // device copy of order_ (sorted position -> caller index), made by the first search_topk
+    int* dOrder_ = nullptr;       // device copy of order_ (sorted position -> caller index), made by the first top-k search, borrowed by the contexts
 };
 
 double measure_dpx_peak(int device, int mix, double* threadInstrPerSec, float* ms);  // mix 0 = SW recurrence, 1 = NW / HW / OV

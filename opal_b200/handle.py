@@ -58,6 +58,10 @@ class OpalB200(OpalCLibrary):
         L.opalb200_db_search_results_pssm.restype = ci
         L.opalb200_db_search_topk_pssm.argtypes = [vp, vp, vp, ci, ci, ci, ci, ci, ci, ci, vp, vp, ctypes.POINTER(ci)]
         L.opalb200_db_search_topk_pssm.restype = ci
+        L.opalb200_db_search_batch_topk.argtypes = [vp, ci, vp, vp, vp, ci, ci, vp, ci, ci, ci, vp, vp, ctypes.POINTER(ci), ci]
+        L.opalb200_db_search_batch_topk.restype = ci
+        L.opalb200_db_search_batch_topk_pssm.argtypes = [vp, ci, vp, vp, vp, vp, ci, ci, ci, ci, ci, vp, vp, ctypes.POINTER(ci), ci]
+        L.opalb200_db_search_batch_topk_pssm.restype = ci
         L.opalb200_db_last_stats.argtypes = [vp] + [ctypes.POINTER(ci)] * 7
         L.opalb200_db_last_stats.restype = None
         L.opalb200_db_last_folded.argtypes = [vp]
@@ -289,6 +293,66 @@ class ResidentDb:
             int(mode), int(k), idx.ctypes.data, rp.ctypes.data, ctypes.byref(found))
         del keep
         return rc, idx[:found.value], results[:found.value]
+
+    @staticmethod
+    def _modes(modes, ns):
+        if isinstance(modes, (str, int)):
+            modes = [modes] * ns
+        md = np.array([MODES[m] if isinstance(m, str) else int(m) for m in modes], dtype=np.int32)
+        assert len(md) == ns
+        return md
+
+    def _batch_topk(self, call, ns, k):
+        """Runs call(indices, result pointers, found) over ns x k slots; returns (rc, indices[ns, found], results[ns, found])."""
+        k = int(k)
+        results = new_results(max(ns * k, 1))
+        rp = result_pointers(results)
+        idx = np.full(max(ns * k, 1), -1, dtype=np.int32)
+        found = ctypes.c_int(0)
+        rc = call(idx.ctypes.data, rp.ctypes.data, ctypes.byref(found))
+        f = found.value
+        rows = idx[:ns * k].reshape(ns, k)[:, :f]
+        recs = results[:ns * k].reshape(ns, k)[:, :f]
+        return rc, np.ascontiguousarray(rows), np.ascontiguousarray(recs)
+
+    def search_batch_topk(self, queries, gap_open, gap_ext, score_matrix, alphabet_length, search_type, modes, k, in_flight=3):
+        """opalb200_db_search_batch_topk: one mode per search (or one mode for all). Returns (rc, indices[ns, found],
+        results[ns, found]); row s is what search_topk returns for queries[s] (free_alignments takes one row at a time)."""
+        qs = [np.ascontiguousarray(q, dtype=np.uint8) for q in queries]
+        bufs = [q if q.size else np.zeros(1, dtype=np.uint8) for q in qs]
+        ns = len(qs)
+        ptrs = np.array([b.ctypes.data for b in bufs] or [0], dtype=np.uint64)
+        qlens = np.array([q.size for q in qs] or [0], dtype=np.int32)
+        md = self._modes(modes, ns)
+        mdb = md if md.size else np.zeros(1, dtype=np.int32)
+        sm = np.ascontiguousarray(score_matrix, dtype=np.int32).ravel()
+        return self._batch_topk(lambda idx, rp, found: self.eng.lib.opalb200_db_search_batch_topk(
+            self.handle, ns, ptrs.ctypes.data, qlens.ctypes.data, mdb.ctypes.data, int(gap_open), int(gap_ext), sm.ctypes.data,
+            int(alphabet_length), int(search_type), int(k), idx, rp, found, int(in_flight)), ns, k)
+
+    def search_batch_topk_pssm(self, pssms, gap_open, gap_ext, search_type, modes, k, queries=None, in_flight=3):
+        """opalb200_db_search_batch_topk_pssm: one PSSM (shape (Q, A), the same A for all; None = a NULL PSSM) and one mode
+        per search; `queries` (the residues each PSSM was built for) is required for OPAL_SEARCH_ALIGNMENT. Returns
+        (rc, indices[ns, found], results[ns, found])."""
+        arrs = [None if x is None else np.ascontiguousarray(x, dtype=np.int32) for x in pssms]
+        ns = len(arrs)
+        shaped = [a for a in arrs if a is not None]
+        A = int(shaped[0].shape[1]) if shaped else 1
+        if any(a.ndim != 2 or a.shape[1] != A for a in shaped):
+            raise ValueError("every pssm must have shape (queryLength, alphabetLength) with the same alphabetLength")
+        bufs = [None if a is None else (a if a.size else np.zeros(1, dtype=np.int32)) for a in arrs]
+        ptrs = np.array([0 if b is None else b.ctypes.data for b in bufs] or [0], dtype=np.uint64)
+        qlens = np.array([1 if a is None else a.shape[0] for a in arrs] or [0], dtype=np.int32)
+        qbufs = None
+        if queries is not None:
+            qbufs = [np.ascontiguousarray(q, dtype=np.uint8) for q in queries]
+            qbufs = [q if q.size else np.zeros(1, dtype=np.uint8) for q in qbufs]
+            qptrs = np.array([q.ctypes.data for q in qbufs] or [0], dtype=np.uint64)
+        md = self._modes(modes, ns)
+        mdb = md if md.size else np.zeros(1, dtype=np.int32)
+        return self._batch_topk(lambda idx, rp, found: self.eng.lib.opalb200_db_search_batch_topk_pssm(
+            self.handle, ns, None if qbufs is None else qptrs.ctypes.data, ptrs.ctypes.data, qlens.ctypes.data, mdb.ctypes.data, A,
+            int(gap_open), int(gap_ext), int(search_type), int(k), idx, rp, found, int(in_flight)), ns, k)
 
     def devices(self):
         return int(self.eng.lib.opalb200_db_devices(self.handle))
