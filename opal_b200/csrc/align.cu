@@ -315,15 +315,14 @@ bool replay_ok(const Scoring& s, const unsigned char* t, int T, const unsigned c
 
 }  // namespace
 
-int align_database(DeviceDb* ddb, const std::vector<AlignSet>& sets, unsigned char* const* db, const int* lens) {
-    if (!ddb || !ddb->ensure_uploaded()) return OPAL_B200_ERR_CUDA;
+int align_database(const DbArrays& ddb, cudaStream_t stream, const std::vector<AlignSet>& sets, unsigned char* const* db, const int* lens) {
     const int ns = (int)sets.size();
     // target of record j of search q on the host: the caller's pointer, or (resident-handle calls) the database's own
     // sorted copy; the record describes database entry entry(q, j): all of them, or the search's subset (top-k pipelines)
     auto entry = [&](int q, int j) { return sets[q].subset ? sets[q].subset[j] : j; };
-    auto target_len = [&](int q, int j) { return lens ? lens[entry(q, j)] : ddb->sorted_lengths()[ddb->sorted_position()[entry(q, j)]]; };
+    auto target_len = [&](int q, int j) { return lens ? lens[entry(q, j)] : ddb.lay->sortedLen[ddb.lay->pos[entry(q, j)]]; };
     auto target_ptr = [&](int q, int j) -> const unsigned char* {
-        return db ? db[entry(q, j)] : ddb->h_residues() + ddb->offsets()[ddb->sorted_position()[entry(q, j)]];
+        return db ? db[entry(q, j)] : ddb.hResidues + ddb.lay->offsets[ddb.lay->pos[entry(q, j)]];
     };
     std::vector<int> M((size_t)ns);  // the band's M of every search: the largest entry that can score a cell
 
@@ -348,8 +347,7 @@ int align_database(DeviceDb* ddb, const std::vector<AlignSet>& sets, unsigned ch
     }
     if (todo.empty()) return 0;
 
-    const cudaStream_t stream = ddb->stream();
-    cudaSetDevice(ddb->device());
+    cudaSetDevice(ddb.device);
     bool ok = true;
     unsigned char* dArgs = nullptr;  // [search table | entries and query of every search]
     AlignTask* dTasks = nullptr;
@@ -380,7 +378,7 @@ int align_database(DeviceDb* ddb, const std::vector<AlignSet>& sets, unsigned ch
     cudaMemGetInfo(&freeB, &totalB);
     const long long budgetWords = (long long)std::max<size_t>(64u << 20, std::min<size_t>(freeB / 3, (size_t)16 << 30)) / 4;
 
-    const int dev = ddb->device();
+    const int dev = ddb.device;
     auto dalloc = [&](void* pp, size_t bytes) { return device_alloc(dev, (void**)pp, bytes); };
     auto release_batch = [&]() {
         device_release(dev, dTasks); device_release(dev, dOuts); device_release(dev, dFlags); device_release(dev, dEq);
@@ -421,7 +419,7 @@ int align_database(DeviceDb* ddb, const std::vector<AlignSet>& sets, unsigned ch
                     if (!tasks.empty() && flagWords + words > budgetWords) break;
                     if (round == 0 && band_borders(tk.score, s.mode, tk.Qp, tk.Tp, s.Go, s.Ge, M[it.q], &tk.bottom, &tk.top)) {}
                     else { tk.bottom = tk.Qp - 1; tk.top = tk.Tp - 1; }
-                    tk.targetOffset = ddb->offsets()[ddb->sorted_position()[entry(it.q, it.j)]];
+                    tk.targetOffset = ddb.lay->offsets[ddb.lay->pos[entry(it.q, it.j)]];
                     tk.flagOffset = flagWords; tk.eqOffset = flagWords; tk.opsOffset = opsBytes; tk.bndOffset = bndInts;
                     flagWords += words; opsBytes += tk.Qp + tk.Tp + 8; bndInts += 2LL * tk.Tp;
                     tasks.push_back(tk); ids.push_back(it);
@@ -439,10 +437,10 @@ int align_database(DeviceDb* ddb, const std::vector<AlignSet>& sets, unsigned ch
                 // an alignment is shorter than its slot: the unused tail travels back with the rest, so it is defined
                 ALIGN_TRY(cudaMemsetAsync(dOps, 0, (size_t)opsBytes, stream));
                 const AlignSearch* dSearches = reinterpret_cast<const AlignSearch*>(dArgs);
-                align_dp_kernel<<<nt, 32, matrixInSmem ? smemBytes : 0, stream>>>(dTasks, dSearches, dOuts, ddb->d_residues(), dFlags, dEq,
+                align_dp_kernel<<<nt, 32, matrixInSmem ? smemBytes : 0, stream>>>(dTasks, dSearches, dOuts, ddb.dResidues, dFlags, dEq,
                                                                                    dBnd, matrixInSmem);
                 ALIGN_TRY(cudaGetLastError());
-                align_traceback_kernel<<<(nt + 63) / 64, 64, 0, stream>>>(dTasks, dSearches, dOuts, nt, ddb->d_residues(), dFlags, dEq, dOps);
+                align_traceback_kernel<<<(nt + 63) / 64, 64, 0, stream>>>(dTasks, dSearches, dOuts, nt, ddb.dResidues, dFlags, dEq, dOps);
                 ALIGN_TRY(cudaGetLastError());
                 hOps.resize((size_t)opsBytes);
                 hOuts.resize(nt);

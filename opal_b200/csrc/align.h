@@ -16,7 +16,7 @@ struct AlignSet {
     const int* subset;
 };
 // For every record of every set: derive start location and alignment from its (score, end location), as reference
-// src/opal.cpp:1475-1507 does with findAlignment (:1236-1431).  The records of all sets share the launches.  db / lens
-// may be NULL (the database's own host copy is used).
-int align_database(DeviceDb* ddb, const std::vector<AlignSet>& sets, unsigned char* const* db = nullptr, const int* lens = nullptr);
+// src/opal.cpp:1475-1507 does with findAlignment (:1236-1431), on `stream` of the database's device, whose upload has
+// finished.  The records of all sets share the launches.  db / lens may be NULL (the database's own host copy is used).
+int align_database(const DbArrays& ddb, cudaStream_t stream, const std::vector<AlignSet>& sets, unsigned char* const* db = nullptr, const int* lens = nullptr);
 }  // namespace opalb200

@@ -213,7 +213,8 @@ static int search_into_results(DeviceDb* ddb, const Scoring& s, unsigned char* c
         status = ddb->search(s, wantEnd, skip.data(), SearchOut::into(results, searchType != OPAL_SEARCH_ALIGNMENT), nullptr);
     const auto t2 = now();
     if (status == 0 && searchType == OPAL_SEARCH_ALIGNMENT)
-        status = align_database(ddb, {{&s, results, dbLength, nullptr}}, db, dbSeqLengths);
+        status = ddb->ensure_uploaded() ? align_database(ddb->arrays(), ddb->stream(), {{&s, results, dbLength, nullptr}}, db, dbSeqLengths)
+                                        : OPAL_B200_ERR_CUDA;
     const auto t3 = now();
     delete owned;
     if (trace)
@@ -633,7 +634,9 @@ static int db_search_batch_topk(OpalB200Db* hh, const std::vector<Scoring>& sear
             std::vector<AlignSet> sets;
             for (int q = 0; q < ns; q++)
                 if (!subset[q].empty()) sets.push_back({&searches[q], res[q].data(), (int)subset[q].size(), subset[q].data()});
-            return sets.empty() ? 0 : align_database(h->shards[s], sets);
+            if (sets.empty()) return 0;
+            DeviceDb* d = h->shards[s];
+            return d->ensure_uploaded() ? align_database(d->arrays(), d->stream(), sets) : OPAL_B200_ERR_CUDA;
         });
     return status;
 }

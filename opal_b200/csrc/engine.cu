@@ -859,14 +859,14 @@ DeviceDb* DeviceDb::create_sorted(const unsigned char* residues, const int* sort
     return build(nullptr, residues, sortedLens, order, n, device);
 }
 
-bool DeviceDb::alloc_search_buffers() {
-    if (!stream_acquire(device_, &stream_) || !event_acquire(device_, &evStart_) || !event_acquire(device_, &evStop_) ||
-        !event_acquire(device_, &evFork_)) return false;
+bool SearchContext::alloc_search_buffers() {
+    if (!stream_acquire(db_.device, &stream_) || !event_acquire(db_.device, &evStart_) || !event_acquire(db_.device, &evStop_) ||
+        !event_acquire(db_.device, &evFork_)) return false;
     // One device block [score | endQ | endT | task list (2n)] and one pinned block [score | endQ | endT]: every
     // stream operation has a fixed cost that exceeds the transfer itself at these sizes, so results come back in
     // a single copy.
-    const size_t nWords = (size_t)std::max(n_, 1);
-    if (!device_alloc(device_, (void**)&dResults_, sizeof(int) * 5 * nWords)) return false;
+    const size_t nWords = (size_t)std::max(db_.n, 1);
+    if (!device_alloc(db_.device, (void**)&dResults_, sizeof(int) * 5 * nWords)) return false;
     // (the copy back covers entries no kernel writes -- skipped and zero-length targets, never read by the host)
     CUDA_TRY(cudaMemsetAsync(dResults_, 0xff, sizeof(int) * 3 * nWords, stream_));
     if (!pinned_alloc((void**)&hResults_, sizeof(int) * 3 * nWords)) return false;
@@ -883,17 +883,17 @@ DeviceDb* DeviceDb::build(unsigned char* const* db, const unsigned char* packed,
         set_error("no usable CUDA device");
         return nullptr;
     }
-    DeviceDb* d = new DeviceDb();
-    d->device_ = device;
-    d->n_ = n;
-    auto fail = [&]() -> DeviceDb* { delete d; return nullptr; };
+    std::unique_ptr<DeviceDb> d(new DeviceDb());
+    DbArrays& a = d->db_;
+    a.device = device;
+    a.n = n;
     auto ok = [&]() -> bool {
         CUDA_TRY(cudaSetDevice(device));
         DeviceInfo di;
         if (!device_info(device, &di)) return false;
         if (di.major < 10) { set_error("device is not sm_100 or newer"); return false; }
-        d->numSMs_ = di.numSMs;
-        d->smemLimit_ = di.smemLimit;
+        a.numSMs = di.numSMs;
+        a.smemLimit = di.smemLimit;
         PhaseTrace trace("build");
         trace.mark("setup");
 
@@ -902,37 +902,39 @@ DeviceDb* DeviceDb::build(unsigned char* const* db, const unsigned char* packed,
         bool cached = false;
         std::shared_ptr<const Layout> lay = layout_for(lens, order, n, packed != nullptr, &cached);
         if (!lay) return false;
-        d->lay_ = lay;
+        a.lay = lay;
         const long long total = lay->total;
         const std::vector<long long>& copyOff = lay->copyOff;
-        d->totalResidues_ = total;
+        a.totalResidues = total;
         trace.mark(cached ? "layout (cached)" : "layout");
-        if (!d->alloc_search_buffers()) return false;
+        d->contexts_.push_back(std::make_unique<SearchContext>(a));
+        SearchContext& ctx = *d->contexts_[0];
+        if (!ctx.alloc_search_buffers()) return false;
         trace.mark("buffers");
 
         // ---- one pinned block [offsets | pair offsets | lengths | max code | residues], one upload.  (Every stream
         // operation costs tens of microseconds on its own here, far more than its share of a few MB, so the
         // database goes up in a single copy once the gather is complete.)  The residues part stays as the host
         // copy the alignment stage replays against.  Paired stream: [32 zeros][pair 0 columns][32 zeros][pair 1 ...].
-        d->numPairs_ = lay->numPairs;
-        d->numFold_ = lay->numFold;
-        const size_t nOff = (size_t)n + 1, nPair = (size_t)std::max(d->numPairs_, 1), nLen = (size_t)std::max(n, 1);
-        const size_t nFold = (size_t)std::max(d->numFold_, 1);
+        a.numPairs = lay->numPairs;
+        a.numFold = lay->numFold;
+        const size_t nOff = (size_t)n + 1, nPair = (size_t)std::max(a.numPairs, 1), nLen = (size_t)std::max(n, 1);
+        const size_t nFold = (size_t)std::max(a.numFold, 1);
         const size_t indexBytes = (sizeof(long long) * (nOff + nPair + nFold) + sizeof(int) * (nLen + 1) + 255) / 256 * 256;
         const size_t bytes = indexBytes + (size_t)total + 64;
-        if (!pinned_alloc((void**)&d->hBlock_, bytes)) return false;
-        if (!device_alloc(device, (void**)&d->dBlock_, bytes)) return false;
-        long long* hOff = reinterpret_cast<long long*>(d->hBlock_);
+        if (!pinned_alloc((void**)&a.hBlock, bytes)) return false;
+        if (!device_alloc(device, (void**)&a.dBlock, bytes)) return false;
+        long long* hOff = reinterpret_cast<long long*>(a.hBlock);
         long long* hPair = hOff + nOff;
         long long* hFold = hPair + nPair;
         int* hLen = reinterpret_cast<int*>(hFold + nFold);
-        d->hResidues_ = d->hBlock_ + indexBytes;
-        d->dOffsets_ = reinterpret_cast<long long*>(d->dBlock_);
-        d->dPairOffsets_ = d->dOffsets_ + nOff;
-        d->dFoldOffsets_ = d->dPairOffsets_ + nPair;
-        d->dLengths_ = reinterpret_cast<int*>(d->dFoldOffsets_ + nFold);
-        d->dMaxCode_ = d->dLengths_ + nLen;
-        d->dResidues_ = d->dBlock_ + indexBytes;
+        a.hResidues = a.hBlock + indexBytes;
+        a.dOffsets = reinterpret_cast<long long*>(a.dBlock);
+        a.dPairOffsets = a.dOffsets + nOff;
+        a.dFoldOffsets = a.dPairOffsets + nPair;
+        a.dLengths = reinterpret_cast<int*>(a.dFoldOffsets + nFold);
+        a.dMaxCode = a.dLengths + nLen;
+        a.dResidues = a.dBlock + indexBytes;
         memcpy(hOff, lay->offsets.data(), sizeof(long long) * nOff);
         memcpy(hPair, lay->pairOff.data(), sizeof(long long) * nPair);
         memcpy(hFold, lay->foldOff.data(), sizeof(long long) * nFold);
@@ -940,7 +942,7 @@ DeviceDb* DeviceDb::build(unsigned char* const* db, const unsigned char* packed,
         if (n > 0) memcpy(hLen, lay->sortedLen.data(), sizeof(int) * (size_t)n);
         hLen[nLen] = 0;  // max code, raised by the pairing kernel
         const long long entries = lay->entries, foldEntries = lay->foldEntries;
-        uint8_t* staging = d->hResidues_;
+        uint8_t* staging = a.hResidues;
         memset(staging + total, 0, 64);
         // Parts of about equal residue count, cut at sequence boundaries; each is uploaded as soon as it and all
         // parts before it are staged, so the copy engine runs behind the host copy.  The copy engine reads lines
@@ -982,91 +984,80 @@ DeviceDb* DeviceDb::build(unsigned char* const* db, const unsigned char* packed,
         auto upload = [&](int k) {
             const size_t end = k == parts - 1 ? bytes : indexBytes + (size_t)copyOff[cut[k + 1]];
             for (size_t at = uploaded; at < end; at += (size_t)1 << 30) {
-                const cudaError_t ce = cudaMemcpyAsync(d->dBlock_ + at, d->hBlock_ + at, std::min(end - at, (size_t)1 << 30), cudaMemcpyHostToDevice, d->stream_);
+                const cudaError_t ce = cudaMemcpyAsync(a.dBlock + at, a.hBlock + at, std::min(end - at, (size_t)1 << 30), cudaMemcpyHostToDevice, ctx.stream_);
                 if (ce != cudaSuccess) copyError = ce;
             }
             uploaded = std::max(uploaded, end);
         };
         trace.mark("index");
-        if (trace.on) CUDA_TRY(cudaEventRecord(d->evStart_, d->stream_));
+        ctx.uploadPending_ = true;
+        if (trace.on) CUDA_TRY(cudaEventRecord(ctx.evStart_, ctx.stream_));
         if (threaded) pool.run(parts, stage, upload);
         else for (int k = 0; k < parts; k++) { stage(k); upload(k); }
         CUDA_TRY(copyError);
         trace.mark("stage+issue");
-        if (trace.on) CUDA_TRY(cudaEventRecord(d->evFork_, d->stream_));
-        if (!device_alloc(device, (void**)&d->dPairStream_, sizeof(uint16_t) * (size_t)entries)) return false;
-        if (!pinned_alloc((void**)&d->hMaxCode_, sizeof(int))) return false;
+        if (trace.on) CUDA_TRY(cudaEventRecord(ctx.evFork_, ctx.stream_));
+        if (!device_alloc(device, (void**)&a.dPairStream, sizeof(uint16_t) * (size_t)entries)) return false;
+        if (!pinned_alloc((void**)&a.hMaxCode, sizeof(int))) return false;
         {
             const long long blocks = (entries + kPackEntriesPerBlock - 1) / kPackEntriesPerBlock;
-            pack_pairs_kernel<<<(unsigned)blocks, 256, 0, d->stream_>>>(d->dResidues_, d->dOffsets_, d->dLengths_, n, d->dPairOffsets_,
-                                                                        d->numPairs_, entries, d->dPairStream_, d->dMaxCode_);
+            pack_pairs_kernel<<<(unsigned)blocks, 256, 0, ctx.stream_>>>(a.dResidues, a.dOffsets, a.dLengths, n, a.dPairOffsets,
+                                                                         a.numPairs, entries, a.dPairStream, a.dMaxCode);
             CUDA_TRY(cudaGetLastError());
         }
-        if (d->numFold_ > 0) {
-            if (!device_alloc(device, (void**)&d->dFoldStream_, sizeof(uint16_t) * (size_t)foldEntries)) return false;
-            pack_folded_kernel<<<(unsigned)((foldEntries + 255) / 256), 256, 0, d->stream_>>>(d->dResidues_, d->dOffsets_, d->dLengths_,
-                                                                                           d->dFoldOffsets_, d->numFold_, foldEntries, d->dFoldStream_);
+        if (a.numFold > 0) {
+            if (!device_alloc(device, (void**)&a.dFoldStream, sizeof(uint16_t) * (size_t)foldEntries)) return false;
+            pack_folded_kernel<<<(unsigned)((foldEntries + 255) / 256), 256, 0, ctx.stream_>>>(a.dResidues, a.dOffsets, a.dLengths,
+                                                                                            a.dFoldOffsets, a.numFold, foldEntries, a.dFoldStream);
             CUDA_TRY(cudaGetLastError());
         }
-        CUDA_TRY(cudaMemcpyAsync(d->hMaxCode_, d->dMaxCode_, sizeof(int), cudaMemcpyDeviceToHost, d->stream_));
-        if (trace.on) CUDA_TRY(cudaEventRecord(d->evStop_, d->stream_));
+        CUDA_TRY(cudaMemcpyAsync(a.hMaxCode, a.dMaxCode, sizeof(int), cudaMemcpyDeviceToHost, ctx.stream_));
+        if (trace.on) CUDA_TRY(cudaEventRecord(ctx.evStop_, ctx.stream_));
         trace.mark("issue");
         return true;  // upload still in flight: see ensure_uploaded()
     }();
-    return ok ? d : fail();
+    return ok ? d.release() : nullptr;
 }
 
-bool DeviceDb::ensure_uploaded() {
-    if (uploaded_) return true;
-    CUDA_TRY(cudaSetDevice(device_));
+// Only the first context ever waits here: build() issues the upload on its stream, and in_flight() waits for the
+// upload before it makes the others.
+bool SearchContext::ensure_uploaded() {
+    if (!uploadPending_) return true;
+    CUDA_TRY(cudaSetDevice(db_.device));
     CUDA_TRY(cudaStreamSynchronize(stream_));
-    if (getenv("OPAL_B200_TRACE") && ownsDb_) {
+    if (getenv("OPAL_B200_TRACE")) {
         float copies = 0.f, pack = 0.f;
         if (cudaEventElapsedTime(&copies, evStart_, evFork_) == cudaSuccess && cudaEventElapsedTime(&pack, evFork_, evStop_) == cudaSuccess)
             fprintf(stderr, "[opal-b200] upload on the device: copies %.0f us, pairing %.0f us\n", copies * 1e3, pack * 1e3);
     }
-    maxCode_ = hMaxCode_ ? *hMaxCode_ : 0;
-    uploaded_ = true;
+    uploadPending_ = false;
     return true;
 }
 
-// A search context over the same resident database: own stream, events, result and scratch buffers.
-DeviceDb* DeviceDb::clone_context() {
-    if (!ensure_uploaded()) return nullptr;
-    DeviceDb* c = new DeviceDb();
-    c->ownsDb_ = false; c->uploaded_ = true;
-    c->device_ = device_; c->n_ = n_; c->numSMs_ = numSMs_; c->smemLimit_ = smemLimit_; c->totalResidues_ = totalResidues_;
-    c->lay_ = lay_;
-    c->hResidues_ = hResidues_; c->dResidues_ = dResidues_; c->dOffsets_ = dOffsets_; c->dLengths_ = dLengths_;
-    c->dPairStream_ = dPairStream_; c->dPairOffsets_ = dPairOffsets_; c->numPairs_ = numPairs_; c->maxCode_ = maxCode_;
-    c->dFoldStream_ = dFoldStream_; c->dFoldOffsets_ = dFoldOffsets_; c->numFold_ = numFold_; c->dOrder_ = dOrder_;
-    if (cudaSetDevice(device_) != cudaSuccess || !c->alloc_search_buffers()) { delete c; return nullptr; }
-    return c;
-}
-
-DeviceDb::~DeviceDb() {
-    cudaSetDevice(device_);
-    for (DeviceDb* c : contexts_) delete c;
+SearchContext::~SearchContext() {
+    cudaSetDevice(db_.device);
     if (stream_) cudaStreamSynchronize(stream_);
     void* own[] = {dResults_, dArgs_, dBndH_, dBndF_};
-    for (void* p : own) device_release(device_, p);
-    for (void* b : chainScratch_) device_release(device_, b);
-    if (ownsDb_) {
-        void* shared[] = {dBlock_, dPairStream_, dFoldStream_, dOrder_};
-        for (void* p : shared) device_release(device_, p);
-        pinned_release(hBlock_); pinned_release(hMaxCode_);
-    }
+    for (void* p : own) device_release(db_.device, p);
+    for (void* b : chainScratch_) device_release(db_.device, b);
     pinned_release(hResults_); pinned_release(hArgs_);
-    event_release(device_, evStart_); event_release(device_, evStop_); event_release(device_, evFork_);
-    for (cudaStream_t st : auxStreams_) { cudaStreamSynchronize(st); stream_release(device_, st); }
-    for (cudaEvent_t e : auxEvents_) event_release(device_, e);
-    stream_release(device_, stream_);
+    event_release(db_.device, evStart_); event_release(db_.device, evStop_); event_release(db_.device, evFork_);
+    for (cudaStream_t st : auxStreams_) { cudaStreamSynchronize(st); stream_release(db_.device, st); }
+    for (cudaEvent_t e : auxEvents_) event_release(db_.device, e);
+    stream_release(db_.device, stream_);
 }
 
-bool DeviceDb::ensure_boundary() {
+DbArrays::~DbArrays() {
+    cudaSetDevice(device);
+    void* arrays[] = {dBlock, dPairStream, dFoldStream, dOrder};
+    for (void* p : arrays) device_release(device, p);
+    pinned_release(hBlock); pinned_release(hMaxCode);
+}
+
+bool SearchContext::ensure_boundary() {
     if (dBndH_) return true;
-    const size_t bytes = 2 * sizeof(uint32_t) * (size_t)(totalResidues_ + 64);  // two halves: ping-pong between passes
-    if (!device_alloc(device_, (void**)&dBndH_, bytes) || !device_alloc(device_, (void**)&dBndF_, bytes)) return false;
+    const size_t bytes = 2 * sizeof(uint32_t) * (size_t)(db_.totalResidues + 64);  // two halves: ping-pong between passes
+    if (!device_alloc(db_.device, (void**)&dBndH_, bytes) || !device_alloc(db_.device, (void**)&dBndF_, bytes)) return false;
     return true;
 }
 
@@ -1112,7 +1103,7 @@ void SearchOut::put(int i, int score, int endQuery, int endTarget) const {
 }
 
 // The search in progress as its planning and launches see it: built once its arguments have passed.
-struct DeviceDb::Run {
+struct SearchContext::Run {
     const Scoring& s;
     int wantEnd;
     ScoreBounds b;  // (args16 cleared when the database holds a code the 16-bit streams cannot carry, see search())
@@ -1132,13 +1123,13 @@ struct DeviceDb::Run {
 };
 
 // The targets of a search by precision class (sorted positions, ascending).
-struct DeviceDb::Routes {
+struct SearchContext::Routes {
     std::vector<int> list16, list32;
     int emptyFrom = 0;  // results on the device: first sorted position of the zero-length targets (n: none)
 };
 
 // One kernel-launch group: tasks that share a precision class and a geometry.
-struct DeviceDb::Group {
+struct SearchContext::Group {
     int type = 0;            // 0 = Packed16 (tasks are pair indices), 1 = Scalar32 (tasks are sorted-target indices)
     std::vector<int> tasks;  // longest first
     Geometry g;
@@ -1151,7 +1142,7 @@ struct DeviceDb::Group {
 // busy long after everything else has finished (the tail bound of pick_geometry) gets a "latency class":
 // its longest tasks run with 32 threads per task and one warp per scheduler partition on SMs of their own,
 // concurrently with the throughput-oriented bulk group on the remaining SMs.
-bool DeviceDb::plan_class(int type, const std::vector<int>& list, const Run& run, std::vector<Group>* groups, double deadline) {
+bool SearchContext::plan_class(int type, const std::vector<int>& list, const Run& run, std::vector<Group>* groups, double deadline) {
     if (list.empty()) return true;
     const int Q = run.s.Q, A = run.s.A, mode = run.s.mode, wantEnd = run.wantEnd;
     const int lanes = type == 0 ? 2 : 1;
@@ -1166,19 +1157,19 @@ bool DeviceDb::plan_class(int type, const std::vector<int>& list, const Run& run
     // The usual list is "every non-empty target": its prefix sums live with the layout (they cost more than the rest
     // of the planning for half a million targets and depend on nothing else).
     TaskLens own;
-    const bool everything = (int)list.size() == lay_->nonEmpty && list.front() == 0 && list.back() == lay_->nonEmpty - 1;
+    const bool everything = (int)list.size() == db_.lay->nonEmpty && list.front() == 0 && list.back() == db_.lay->nonEmpty - 1;
     if (!everything) {
         own.len.resize(tasks.size());
-        for (size_t k = 0; k < tasks.size(); k++) own.len[k] = lay_->sortedLen[lanes == 2 ? 2 * tasks[k] : tasks[k]];
+        for (size_t k = 0; k < tasks.size(); k++) own.len[k] = db_.lay->sortedLen[lanes == 2 ? 2 * tasks[k] : tasks[k]];
         own.build();
     }
-    const TaskLens& tl = everything ? (lanes == 2 ? lay_->pair_lens() : lay_->target_lens()) : own;
+    const TaskLens& tl = everything ? (lanes == 2 ? db_.lay->pair_lens() : db_.lay->target_lens()) : own;
     const size_t nT = tasks.size();
 
     Geometry gAll;
     double tAll = 0;
     const int flavorClass = mode == kModeSW ? (wantEnd ? 0 : 1) : 2;
-    if (!pick_geometry(Q, A, lanes, tl, 0, nT, smemLimit_, numSMs_, mode, false, flavorClass, &gAll, &tAll)) return false;
+    if (!pick_geometry(Q, A, lanes, tl, 0, nT, db_.smemLimit, db_.numSMs, mode, false, flavorClass, &gAll, &tAll)) return false;
     // A small class beside one that takes much longer (the sixteen targets of a global-mode search that need 32 bits
     // beside half a million that do not): it cannot end the search, so it holds the fewest SMs on which it still ends
     // well inside the other class's time instead of the many that end it soonest (measured on BASELINE configs[2],
@@ -1187,7 +1178,7 @@ bool DeviceDb::plan_class(int type, const std::vector<int>& list, const Run& run
         for (int sms = 1; sms <= 8; sms *= 2) {
             Geometry g;
             double t = 0;
-            if (!pick_geometry(Q, A, lanes, tl, 0, nT, smemLimit_, sms, mode, false, flavorClass, &g, &t) || t > 0.6 * deadline) continue;
+            if (!pick_geometry(Q, A, lanes, tl, 0, nT, db_.smemLimit, sms, mode, false, flavorClass, &g, &t) || t > 0.6 * deadline) continue;
             Group grp;
             grp.type = type; grp.estCycles = t; grp.tasks = tasks; grp.g = g; grp.maxBlocks = sms; grp.smemBytes = g.smemBytes;
             groups->push_back(std::move(grp));
@@ -1206,7 +1197,7 @@ bool DeviceDb::plan_class(int type, const std::vector<int>& list, const Run& run
             if (passes < 2 || passes > 64 || (long long)passes * rows * 3 > (long long)Q * 4 + 96) continue;
             const int Rpad = rpad_of(R), rowStride = 32 * Rpad;
             const size_t smem = (size_t)planes * (A + 1) * rowStride * 4;
-            if (smem > (size_t)smemLimit_ || passes * quads > numSMs_ / 3) continue;
+            if (smem > (size_t)db_.smemLimit || passes * quads > db_.numSMs / 3) continue;
             const double t = (tl.len[0] + 31 + 100.0 * (passes - 1)) * step_cycles(flavorClass, 1, R) * 1.08 + 40000.0;
             if (t < tAll * 0.90) {
                 tAll = t;
@@ -1223,12 +1214,12 @@ bool DeviceDb::plan_class(int type, const std::vector<int>& list, const Run& run
     Geometry bestL, bestB;
     // Folded variant of the latency class (16 bits, one pass): the 2 m longest TARGETS, one per warp in both half-words,
     // which halves the rows per thread and with them the time of the longest target.  Needs the folded stream
-    // (built for the numFold_ longest targets) and every one of those targets wanted.
+    // (built for the numFold longest targets) and every one of those targets wanted.
     TaskLens tlFold;
     size_t foldable = 0;
-    if (lanes == 2 && numFold_ > 0 && !getenv("OPAL_B200_NO_FOLD") && (mode == kModeSW || !getenv("OPAL_B200_NO_FOLD_GLOBAL"))) {
-        while (foldable < (size_t)numFold_ && foldable < list.size() && list[foldable] == (int)foldable) foldable++;
-        tlFold.len.assign(lay_->sortedLen.begin(), lay_->sortedLen.begin() + foldable);
+    if (lanes == 2 && db_.numFold > 0 && !getenv("OPAL_B200_NO_FOLD") && (mode == kModeSW || !getenv("OPAL_B200_NO_FOLD_GLOBAL"))) {
+        while (foldable < (size_t)db_.numFold && foldable < list.size() && list[foldable] == (int)foldable) foldable++;
+        tlFold.len.assign(db_.lay->sortedLen.begin(), db_.lay->sortedLen.begin() + foldable);
         tlFold.build();
     }
     if (!getenv("OPAL_B200_NO_SPLIT") && !getenv("OPAL_B200_GEOMETRY")) {
@@ -1244,19 +1235,19 @@ bool DeviceDb::plan_class(int type, const std::vector<int>& list, const Run& run
                 if (variant && tasksL > foldable) continue;
                 if (fm >= 0 && ((int)m != fm || variant != fv)) continue;
                 for (int div = 1; div <= 4; div *= 2) {
-                    int smL = (int)std::min<size_t>((tasksL + 4 * div - 1) / (4 * div), (size_t)numSMs_ / 2);
+                    int smL = (int)std::min<size_t>((tasksL + 4 * div - 1) / (4 * div), (size_t)db_.numSMs / 2);
                     if (fm >= 0) { if (div > 1) continue; smL = fsm; bestT = 1e300; }
                     if (smL < 1) continue;
                     Geometry gL, gB;
                     double tL = 0, tB = 0;
-                    if (!pick_geometry(Q, A, lanes, variant ? tlFold : tl, 0, tasksL, smemLimit_, smL, mode, true, flavorClass, &gL, &tL, variant != 0)) continue;
-                    if (!pick_geometry(Q, A, lanes, tl, m, nT, smemLimit_, numSMs_ - smL, mode, false, flavorClass, &gB, &tB)) continue;
+                    if (!pick_geometry(Q, A, lanes, variant ? tlFold : tl, 0, tasksL, db_.smemLimit, smL, mode, true, flavorClass, &gL, &tL, variant != 0)) continue;
+                    if (!pick_geometry(Q, A, lanes, tl, m, nT, db_.smemLimit, db_.numSMs - smL, mode, false, flavorClass, &gB, &tB)) continue;
                     // One search alone ends when its slower group ends.  With searches overlapping (search_batch) the SMs a
                     // group leaves are taken by the next search, so a plan costs the SM time it holds: the latency class
                     // then shrinks to the fewest SMs its tasks fit on instead of the fewest that end them soonest (measured
                     // on an eighth of BASELINE configs[2]: up to eight searches in flight each held 4+ SMs at a third of
                     // their issue rate for a tail several times longer than its bulk).
-                    const double t = (t_overlapped ? (smL * tL + (numSMs_ - smL) * tB) / numSMs_ : std::max(tL, tB)) + 3000.0;  // a second launch is not free
+                    const double t = (t_overlapped ? (smL * tL + (db_.numSMs - smL) * tB) / db_.numSMs : std::max(tL, tB)) + 3000.0;  // a second launch is not free
                     if (t < bestT * 0.97) { bestT = t; bestM = m; bestSm = smL; bestL = gL; bestB = gB; }
                 }
             }
@@ -1280,15 +1271,15 @@ bool DeviceDb::plan_class(int type, const std::vector<int>& list, const Run& run
                     const int Rpad = rpad_of(R), rowStride = 32 * Rpad;
                     const size_t smem = (size_t)planes * (A + 1) * rowStride * 4;
                     const int smL = passes * quads;
-                    if (smem > (size_t)smemLimit_ || smL > numSMs_ / 3) continue;
+                    if (smem > (size_t)db_.smemLimit || smL > db_.numSMs / 3) continue;
                     Geometry gL, gB;
                     gL.G = 32; gL.R = R; gL.tableIndex = (int)ti; gL.passes = passes; gL.Rpad = Rpad; gL.rowStride = rowStride;
                     gL.smemBytes = smem; gL.warpsPerPartition = 1; gL.padTop = mode == kModeNW ? 0 : passes * rows - Q; gL.chain = true;
                     // every pass trails the one above by about three chunks of 32 columns
                     const double tL = (tl.len[0] + 31 + 100.0 * (passes - 1)) * step_cycles(flavorClass, 1, R) * 1.08 + 40000.0;
                     double tB = 0;
-                    if (!pick_geometry(Q, A, lanes, tl, m, nT, smemLimit_, numSMs_ - smL, mode, false, flavorClass, &gB, &tB)) continue;
-                    const double t = (t_overlapped ? (smL * tL + (numSMs_ - smL) * tB) / numSMs_ : std::max(tL, tB)) + 3000.0;
+                    if (!pick_geometry(Q, A, lanes, tl, m, nT, db_.smemLimit, db_.numSMs - smL, mode, false, flavorClass, &gB, &tB)) continue;
+                    const double t = (t_overlapped ? (smL * tL + (db_.numSMs - smL) * tB) / db_.numSMs : std::max(tL, tB)) + 3000.0;
                     // (a tenth better at least: a folded or plain latency class of equal speed holds fewer SMs)
                     if (t < bestT * 0.90 || (force && !bestL.chain)) { bestT = t; bestM = m; bestSm = smL; bestL = gL; bestB = gB; }
                 }
@@ -1310,16 +1301,16 @@ bool DeviceDb::plan_class(int type, const std::vector<int>& list, const Run& run
         grp.maxBlocks = maxBlocks;
         grp.smemBytes = g.smemBytes;
         // exclusive placement: ask for enough shared memory that a block of the other group cannot join this SM
-        if (otherSmem > 0 && g.smemBytes + otherSmem <= (size_t)smemLimit_)
-            grp.smemBytes = std::min<size_t>((size_t)smemLimit_, (size_t)smemLimit_ - otherSmem + 1024);
+        if (otherSmem > 0 && g.smemBytes + otherSmem <= (size_t)db_.smemLimit)
+            grp.smemBytes = std::min<size_t>((size_t)db_.smemLimit, (size_t)db_.smemLimit - otherSmem + 1024);
         groups->push_back(std::move(grp));
     };
-    if (bestM == 0) add(0, tasks.size(), gAll, numSMs_, 0, tAll);
+    if (bestM == 0) add(0, tasks.size(), gAll, db_.numSMs, 0, tAll);
     else {
         add(0, bestM, bestL, bestSm, bestB.smemBytes, bestT);   // launched first: takes its SMs
         // every block's first tasks are assigned statically (longest first), so the bulk grid must be fully
         // resident from the start: one block per SM the latency class leaves free
-        add(bestM, tasks.size(), bestB, numSMs_ - bestSm, 0, bestT);
+        add(bestM, tasks.size(), bestB, db_.numSMs - bestSm, 0, bestT);
     }
     return true;
 }
@@ -1339,7 +1330,7 @@ static bool allow_full_smem(int device, const void* fn, int smemLimit) {
 }
 
 // Launches every pass of one group on `stream`.
-bool DeviceDb::launch_group(const Group& grp, int* taskListDevice, cudaStream_t stream, const Run& run) {
+bool SearchContext::launch_group(const Group& grp, int* taskListDevice, cudaStream_t stream, const Run& run) {
     const Geometry& g = grp.g;
     const int type = grp.type, mode = run.s.mode, wantEnd = run.wantEnd, maxScore = run.b.maxEntry;
     if (g.passes > 1 && !g.chain && !ensure_boundary()) return false;
@@ -1360,7 +1351,7 @@ bool DeviceDb::launch_group(const Group& grp, int* taskListDevice, cudaStream_t 
         fn = kernel_tables()[g.tableIndex].fn[type == 0 ? 8 : type * 4 + flavor];  // Packed16 variant compiled for 384 threads
     if (g.chain) fn = kernel_tables()[g.tableIndex].chainFn[type * 4 + flavor];
     if (!fn) { set_error("no kernel for this geometry"); return false; }
-    if (!allow_full_smem(device_, fn, smemLimit_)) return false;
+    if (!allow_full_smem(db_.device, fn, db_.smemLimit)) return false;
     // chained passes: one launch, passes x quads blocks; boundary rows and flags live in a block of their own
     int chainStride = 0;
     int *dChainOffsets = nullptr, *dChainDone = nullptr, *dChainTicket = nullptr;
@@ -1369,18 +1360,18 @@ bool DeviceDb::launch_group(const Group& grp, int* taskListDevice, cudaStream_t 
         std::vector<int> offsets(grp.tasks.size());
         for (size_t k = 0; k < grp.tasks.size(); k++) {
             offsets[k] = chainStride;
-            chainStride += lay_->sortedLen[type == 0 ? 2 * (size_t)grp.tasks[k] : (size_t)grp.tasks[k]] + 32;
+            chainStride += db_.lay->sortedLen[type == 0 ? 2 * (size_t)grp.tasks[k] : (size_t)grp.tasks[k]] + 32;
         }
         chainStride = (chainStride + 63) / 64 * 64;
         const size_t nT = grp.tasks.size(), flags = nT * (size_t)g.passes;
         const size_t ints = nT + flags + 64, words = 2 * (size_t)g.passes * (size_t)chainStride;
         int* block = nullptr;
-        if (!device_alloc(device_, (void**)&block, sizeof(int) * (ints + words))) return false;
+        if (!device_alloc(db_.device, (void**)&block, sizeof(int) * (ints + words))) return false;
         chainScratch_.push_back(block);
         dChainOffsets = block; dChainDone = block + nT; dChainTicket = dChainDone + flags;
         dChainH = reinterpret_cast<uint32_t*>(block + ints); dChainF = dChainH + (size_t)g.passes * chainStride;
         CUDA_TRY(cudaMemsetAsync(block, 0, sizeof(int) * ints, stream));
-        fill_words_kernel<<<std::min<size_t>((words + 1023) / 1024, 4 * (size_t)numSMs_), 256, 0, stream>>>(dChainH, words, type == 0 ? kChainEmpty : kChainEmpty32);
+        fill_words_kernel<<<std::min<size_t>((words + 1023) / 1024, 4 * (size_t)db_.numSMs), 256, 0, stream>>>(dChainH, words, type == 0 ? kChainEmpty : kChainEmpty32);
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaMemcpyAsync(dChainOffsets, offsets.data(), sizeof(int) * nT, cudaMemcpyHostToDevice, stream));  // (pageable: staged before the call returns)
         stats_.chainedTasks = (int)nT;
@@ -1392,14 +1383,14 @@ bool DeviceDb::launch_group(const Group& grp, int* taskListDevice, cudaStream_t 
         p.Q = run.s.Q; p.A = run.s.A; p.gapOpen = run.s.Go; p.gapExt = run.s.Ge; p.mode = mode; p.wantEnd = wantEnd;
         p.G = g.G; p.rowBase = pass * g.G * g.R; p.padTop = g.padTop; p.pass = pass; p.numPasses = g.passes;
         p.rowStride = g.rowStride; p.Rpad = g.Rpad;
-        p.residues = dResidues_; p.offsets = dOffsets_; p.lengths = dLengths_;
-        p.pairStream = dPairStream_; p.pairOffsets = dPairOffsets_; p.numTargets = n_;
-        if (g.folded) { p.folded = 1; p.pairStream = dFoldStream_; p.pairOffsets = dFoldOffsets_; stats_.foldedTasks = (int)grp.tasks.size(); }
+        p.residues = db_.dResidues; p.offsets = db_.dOffsets; p.lengths = db_.dLengths;
+        p.pairStream = db_.dPairStream; p.pairOffsets = db_.dPairOffsets; p.numTargets = db_.n;
+        if (g.folded) { p.folded = 1; p.pairStream = db_.dFoldStream; p.pairOffsets = db_.dFoldOffsets; stats_.foldedTasks = (int)grp.tasks.size(); }
         p.taskList = contiguous ? nullptr : taskListDevice;
         p.taskBase = contiguous && !grp.tasks.empty() ? grp.tasks[0] : 0;
         p.numTasks = (int)grp.tasks.size();
         p.counter = run.dCounters + run.slot++;
-        const size_t half = (size_t)(totalResidues_ + 64);
+        const size_t half = (size_t)(db_.totalResidues + 64);
         p.bndInH = dBndH_ ? dBndH_ + ((pass + 1) & 1) * half : nullptr; p.bndInF = dBndF_ ? dBndF_ + ((pass + 1) & 1) * half : nullptr;
         p.bndOutH = dBndH_ ? dBndH_ + (pass & 1) * half : nullptr; p.bndOutF = dBndF_ ? dBndF_ + (pass & 1) * half : nullptr;
         p.outScore = dScore_; p.outEndQ = dEndQ_; p.outEndT = dEndT_;
@@ -1410,7 +1401,7 @@ bool DeviceDb::launch_group(const Group& grp, int* taskListDevice, cudaStream_t 
         // column: 0 keeps pad cells inside the range of the real ones, so they cannot trip the range tracking.
         p.padLetterScore = type == 0 ? (mode == kModeNW ? 0 : -16384) : 0;
         p.one = 1; p.keyScale = 1 << kRowBits; p.fastEndLimit = fastEndLimit;
-        {   // range tracking of the 16-bit NW / HW / OV sweeps (see DeviceDb::Run for the limits)
+        {   // range tracking of the 16-bit NW / HW / OV sweeps (see SearchContext::Run for the limits)
             const long long margin = (long long)(g.R + 3) * run.step;
             p.rangeHi = run.rangeTracking ? (int)(32767 - margin) : INT_MAX;   // (not tracking: routed by the a-priori bound)
             p.rangeLo = run.rangeTracking ? (int)(run.rangeLo + margin) : INT_MIN;
@@ -1434,7 +1425,7 @@ bool DeviceDb::launch_group(const Group& grp, int* taskListDevice, cudaStream_t 
 
 // Runs the given classes concurrently: every launch group gets a stream of its own (the first one the
 // database's main stream), all of them ordered after `ready` and joined back into the main stream.
-int DeviceDb::run_classes(const std::vector<std::pair<int, const std::vector<int>*>>& classes, const Run& run) {
+int SearchContext::run_classes(const std::vector<std::pair<int, const std::vector<int>*>>& classes, const Run& run) {
     std::vector<Group> groups;
     PhaseTrace trace("run_classes");
     // the class with the most targets first: what it is estimated to take is the time the small ones may hide in
@@ -1470,10 +1461,10 @@ int DeviceDb::run_classes(const std::vector<std::pair<int, const std::vector<int
         int reserved = 0;
         double bigWork = 0;
         for (size_t i = 0; i < groups.size(); i++) {
-            if (want[i] * 4 <= numSMs_ && reserved + want[i] <= numSMs_ / 2) { groups[i].maxBlocks = want[i]; reserved += want[i]; }
+            if (want[i] * 4 <= db_.numSMs && reserved + want[i] <= db_.numSMs / 2) { groups[i].maxBlocks = want[i]; reserved += want[i]; }
             else { big[i] = 1; bigWork += std::max(1.0, groups[i].estCycles * want[i]); }
         }
-        const int left = numSMs_ - reserved;
+        const int left = db_.numSMs - reserved;
         for (size_t i = 0; i < groups.size(); i++) {
             if (!big[i]) continue;
             const int share = std::max(1, (int)(left * std::max(1.0, groups[i].estCycles * want[i]) / bigWork));
@@ -1484,7 +1475,7 @@ int DeviceDb::run_classes(const std::vector<std::pair<int, const std::vector<int
         for (const Group& g : groups)
             fprintf(stderr, "[opal-b200] group type=%d%s tasks=%zu longest=%d G=%d R=%d k=%d passes=%d blocks<=%d est=%.0f kcycles\n", g.type,
                     g.g.folded ? " folded" : g.g.chain ? " chained" : "", g.tasks.size(),
-                    g.tasks.empty() ? 0 : lay_->sortedLen[g.type == 0 && !g.g.folded ? 2 * g.tasks[0] : g.tasks[0]], g.g.G, g.g.R,
+                    g.tasks.empty() ? 0 : db_.lay->sortedLen[g.type == 0 && !g.g.folded ? 2 * g.tasks[0] : g.tasks[0]], g.g.G, g.g.R,
                     g.g.warpsPerPartition, g.g.passes, g.maxBlocks, g.estCycles / 1e3);
     bool badArgument = false;
     auto body = [&]() -> bool {
@@ -1493,7 +1484,7 @@ int DeviceDb::run_classes(const std::vector<std::pair<int, const std::vector<int
         // validated here, before anything indexes the profile with them.
         if (!ensure_uploaded()) return false;
         trace.mark("upload-wait");
-        if (maxCode_ >= run.s.A) { set_error("database holds residue codes >= alphabetLength"); badArgument = true; return false; }
+        if (*db_.hMaxCode >= run.s.A) { set_error("database holds residue codes >= alphabetLength"); badArgument = true; return false; }
         if (!startRecorded_) { CUDA_TRY(cudaEventRecord(evStart_, stream_)); startRecorded_ = true; }  // planning is host work: keep it outside the device window
         if (groups.size() > 1) CUDA_TRY(cudaEventRecord(evFork_, stream_));
         for (size_t gi = 0; gi < groups.size(); gi++) {
@@ -1501,7 +1492,7 @@ int DeviceDb::run_classes(const std::vector<std::pair<int, const std::vector<int
             if (gi > 0) {
                 while (auxStreams_.size() < gi) {
                     cudaStream_t s2; cudaEvent_t e2;
-                    if (!stream_acquire(device_, &s2) || !event_acquire(device_, &e2)) return false;
+                    if (!stream_acquire(db_.device, &s2) || !event_acquire(db_.device, &e2)) return false;
                     auxStreams_.push_back(s2); auxEvents_.push_back(e2);
                 }
                 st = auxStreams_[gi - 1];
@@ -1519,9 +1510,9 @@ int DeviceDb::run_classes(const std::vector<std::pair<int, const std::vector<int
     return body() ? 0 : (badArgument ? OPAL_B200_ERR_ARGUMENT : OPAL_B200_ERR_CUDA);
 }
 
-int DeviceDb::search(const Scoring& s, int wantEnd, const unsigned char* skip, const SearchOut& out, float* deviceMs) {
+int SearchContext::search(const Scoring& s, int wantEnd, const unsigned char* skip, const SearchOut& out, float* deviceMs) {
     stats_ = SearchStats();
-    for (void* b : chainScratch_) device_release(device_, b);  // (the previous search has been waited for)
+    for (void* b : chainScratch_) device_release(db_.device, b);  // (the previous search has been waited for)
     chainScratch_.clear();
     PhaseTrace trace("search");
     if (deviceMs) *deviceMs = 0.f;
@@ -1531,7 +1522,7 @@ int DeviceDb::search(const Scoring& s, int wantEnd, const unsigned char* skip, c
     // holds it (alphabetLength 256) is searched by the 32-bit class, which reads the plain stream.
     if (s.A == 256) {
         if (!ensure_uploaded()) return OPAL_B200_ERR_CUDA;
-        if (maxCode_ >= 255) b.args16 = false;
+        if (*db_.hMaxCode >= 255) b.args16 = false;
     }
     Run run{s, wantEnd, b};
     Routes routes;
@@ -1545,7 +1536,7 @@ int DeviceDb::search(const Scoring& s, int wantEnd, const unsigned char* skip, c
 
 // Every non-skipped target to the 16-bit or the 32-bit class; a target with nothing to align gets its result here.
 // 0 or OPAL_B200_ERR_OVERFLOW (a target that 32 bits cannot hold).
-int DeviceDb::route(const Run& run, const unsigned char* skip, const SearchOut& out, Routes* routes) {
+int SearchContext::route(const Run& run, const unsigned char* skip, const SearchOut& out, Routes* routes) {
     const int Q = run.s.Q, Go = run.s.Go, Ge = run.s.Ge, mode = run.s.mode, maxP = run.b.maxEntry;
     const bool isSW = mode == kModeSW, args16 = run.b.args16, track16 = run.rangeTracking;
     auto& [list16, list32, emptyFrom] = *routes;
@@ -1572,31 +1563,31 @@ int DeviceDb::route(const Run& run, const unsigned char* skip, const SearchOut& 
     auto ok32 = [&](int T) -> bool {
         return isSW ? (maxP > 0 ? (long long)std::min(Q, T) * maxP : 0) < (1LL << 30) : fits(T, 1LL << 30);
     };
-    (args16 ? list16 : list32).reserve((size_t)n_);
-    emptyFrom = n_;
+    (args16 ? list16 : list32).reserve((size_t)db_.n);
+    emptyFrom = db_.n;
     int routeFrom = 0;
     if (!skip && Q > 0) {
         // Nothing skipped: the classes are ranges of the sorted order: [0, b) needs 32 bits, [b, nonEmpty) fits 16;
         // only the empty targets are left to the loop below.
-        const int m = lay_->nonEmpty;
+        const int m = db_.lay->nonEmpty;
         int lo = 0, hi = m;  // first position whose target fits 16 bits
         while (lo < hi) {
             const int mid = (lo + hi) / 2;
-            if (ok16(lay_->sortedLen[mid])) hi = mid; else lo = mid + 1;
+            if (ok16(db_.lay->sortedLen[mid])) hi = mid; else lo = mid + 1;
         }
         int b = lo;
         if (!isSW && (b & 1) && b < m) b++;  // a pair is never split between the classes (see below)
-        if (b > 0 && !ok32(lay_->sortedLen[0])) return OPAL_B200_ERR_OVERFLOW;  // the longest target decides for all
+        if (b > 0 && !ok32(db_.lay->sortedLen[0])) return OPAL_B200_ERR_OVERFLOW;  // the longest target decides for all
         list32.resize((size_t)b);
         for (int p = 0; p < b; p++) list32[p] = p;
         list16.resize((size_t)(m - b));
         for (int p = b; p < m; p++) list16[p - b] = p;
         routeFrom = m;
     }
-    for (int p = routeFrom; p < n_; p++) {
-        const int i = lay_->order[p];
+    for (int p = routeFrom; p < db_.n; p++) {
+        const int i = db_.lay->order[p];
         if (skip && skip[i]) continue;
-        const int T = lay_->sortedLen[p];
+        const int T = db_.lay->sortedLen[p];
         if (T == 0 && out.dSelect) { emptyFrom = std::min(emptyFrom, p); continue; }  // filled on the device
         if (T == 0 || Q <= 0) {  // nothing to align: defined as in oracle/opal_oracle.c
             int sc = 0, eq = Q - 1, et = T - 1;
@@ -1613,7 +1604,7 @@ int DeviceDb::route(const Run& run, const unsigned char* skip, const SearchOut& 
     // The 16-bit class works on whole pairs (sorted targets 2p, 2p+1) and the two classes of NW/HW/OV run
     // concurrently, so a pair is never split between them: if one member needs 32 bits, both go there.
     if (!isSW && !list32.empty() && !list16.empty()) {
-        std::vector<char> wide((size_t)numPairs_, 0);
+        std::vector<char> wide((size_t)db_.numPairs, 0);
         for (int p : list32) wide[p >> 1] = 1;
         std::vector<int> keep16, merged32;
         for (int p : list16) (wide[p >> 1] ? merged32 : keep16).push_back(p);
@@ -1629,17 +1620,17 @@ int DeviceDb::route(const Run& run, const unsigned char* skip, const SearchOut& 
 
 // Launch counters (zeroed), score matrix and query travel in one pinned block, one copy; with a PSSM the block is
 // counters and PSSM (the query letters are not needed).
-bool DeviceDb::upload_args(Run* run) {
+bool SearchContext::upload_args(Run* run) {
     const Scoring& s = run->s;
-    CUDA_TRY(cudaSetDevice(device_));
+    CUDA_TRY(cudaSetDevice(db_.device));
     const size_t scoreBytes = sizeof(int) * (size_t)s.num_entries(), matrixBytes = (scoreBytes + 255) / 256 * 256;
     const size_t countersBytes = sizeof(int) * 256;
     const size_t argsBytes = countersBytes + matrixBytes + (s.byPssm ? 0 : (size_t)s.Q + 16);
     if (argsBytes > argsCapacity_) {
-        device_release(device_, dArgs_); dArgs_ = nullptr;
+        device_release(db_.device, dArgs_); dArgs_ = nullptr;
         pinned_release(hArgs_); hArgs_ = nullptr;
         argsCapacity_ = std::max<size_t>(8192, 2 * argsBytes);
-        if (!device_alloc(device_, (void**)&dArgs_, argsCapacity_) || !pinned_alloc((void**)&hArgs_, argsCapacity_)) { argsCapacity_ = 0; return false; }
+        if (!device_alloc(db_.device, (void**)&dArgs_, argsCapacity_) || !pinned_alloc((void**)&hArgs_, argsCapacity_)) { argsCapacity_ = 0; return false; }
     }
     memset(hArgs_, 0, countersBytes);
     memcpy(hArgs_ + countersBytes, s.entries, scoreBytes);
@@ -1654,7 +1645,7 @@ bool DeviceDb::upload_args(Run* run) {
 // The precision ladder: the 16-bit class (NW / HW / OV: and the 32-bit class beside it), then at 32 bits what 16 bits
 // could not hold.  Results are published after every round, or stay on the device.  False: a CUDA failure; *rc: the
 // search's code otherwise.
-bool DeviceDb::ladder(const Run& run, Routes& routes, const SearchOut& out, float* deviceMs, PhaseTrace& trace, int* rc) {
+bool SearchContext::ladder(const Run& run, Routes& routes, const SearchOut& out, float* deviceMs, PhaseTrace& trace, int* rc) {
     const int Q = run.s.Q, Go = run.s.Go, Ge = run.s.Ge, mode = run.s.mode, wantEnd = run.wantEnd;
     const bool isSW = mode == kModeSW, onDevice = out.dSelect != nullptr;
     auto& [list16, list32, emptyFrom] = routes;
@@ -1698,11 +1689,11 @@ bool DeviceDb::ladder(const Run& run, Routes& routes, const SearchOut& out, floa
             if (!publish(list32, wantEnd, out, nullptr)) *rc = OPAL_B200_ERR_OVERFLOW;
         }
     }
-    if (onDevice && emptyFrom < n_) {  // zero-length targets: the defined result, written where a sweep would have left it
+    if (onDevice && emptyFrom < db_.n) {  // zero-length targets: the defined result, written where a sweep would have left it
         int sc = 0, eq = Q - 1, et = -1;
         if (mode == kModeNW || mode == kModeHW) sc = -Go - (Q - 1) * Ge;
         if (isSW) { eq = 0x7fffffff; et = 0x7fffffff; }
-        fill_empty_kernel<<<std::min(numSMs_, (n_ - emptyFrom + 255) / 256), 256, 0, stream_>>>(dScore_, dEndQ_, dEndT_, emptyFrom, n_, sc, eq, et);
+        fill_empty_kernel<<<std::min(db_.numSMs, (db_.n - emptyFrom + 255) / 256), 256, 0, stream_>>>(dScore_, dEndQ_, dEndT_, emptyFrom, db_.n, sc, eq, et);
         CUDA_TRY(cudaGetLastError());
     }
     trace.mark("publish");
@@ -1711,8 +1702,8 @@ bool DeviceDb::ladder(const Run& run, Routes& routes, const SearchOut& out, floa
 }
 
 // [score | endQ | endT] of every target back to the host: they are adjacent on both sides, one copy.
-bool DeviceDb::fetch(int wantEnd, PhaseTrace& trace) {
-    const size_t nWords = (size_t)std::max(n_, 1);
+bool SearchContext::fetch(int wantEnd, PhaseTrace& trace) {
+    const size_t nWords = (size_t)std::max(db_.n, 1);
     CUDA_TRY(cudaMemcpyAsync(hResults_, dResults_, sizeof(int) * (wantEnd ? 3 : 1) * nWords, cudaMemcpyDeviceToHost, stream_));
     trace.mark("launch");
     CUDA_TRY(cudaStreamSynchronize(stream_));
@@ -1722,13 +1713,13 @@ bool DeviceDb::fetch(int wantEnd, PhaseTrace& trace) {
 
 // The fetched results of `list` go back to caller order: a scatter, split over the host pool for large databases.
 // Targets flagged for 32 bits go to *overflowed (sorted); without it, false when there is any.
-bool DeviceDb::publish(const std::vector<int>& list, int wantEnd, const SearchOut& out, std::vector<int>* overflowed) {
+bool SearchContext::publish(const std::vector<int>& list, int wantEnd, const SearchOut& out, std::vector<int>* overflowed) {
     std::mutex mu;
     bool placed = true;
     parallel_for((long long)list.size(), 65536, [&](long long lo, long long hi) {
         std::vector<int> flagged;
         for (long long k = lo; k < hi; k++) {
-            const int p = list[(size_t)k], i = lay_->order[p];
+            const int p = list[(size_t)k], i = db_.lay->order[p];
             const int sc = hScore_[p];
             if (sc == kScoreOverflow || sc == kScoreNone) { flagged.push_back(p); continue; }
             out.put(i, sc, (wantEnd && hEndQ_[p] != 0x7fffffff) ? hEndQ_[p] : -1, (wantEnd && hEndT_[p] != 0x7fffffff) ? hEndT_[p] : -1);
@@ -1745,10 +1736,10 @@ bool DeviceDb::publish(const std::vector<int>& list, int wantEnd, const SearchOu
 
 // Results on the device (search_topk): the hand-over list of the ladder is gathered there (a count and the flagged
 // positions come back instead of every score).
-bool DeviceDb::collect(int* dSelect, int emptyFrom, std::vector<int>* flagged) {
+bool SearchContext::collect(int* dSelect, int emptyFrom, std::vector<int>* flagged) {
     if (emptyFrom <= 0) return true;
     CUDA_TRY(cudaMemsetAsync(dSelect, 0, sizeof(int), stream_));
-    collect_flagged_kernel<<<std::min(numSMs_ * 4, (emptyFrom + 255) / 256), 256, 0, stream_>>>(dScore_, emptyFrom, dSelect + 1, dSelect);
+    collect_flagged_kernel<<<std::min(db_.numSMs * 4, (emptyFrom + 255) / 256), 256, 0, stream_>>>(dScore_, emptyFrom, dSelect + 1, dSelect);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(hResults_, dSelect, sizeof(int), cudaMemcpyDeviceToHost, stream_));
     CUDA_TRY(cudaStreamSynchronize(stream_));
@@ -1762,15 +1753,15 @@ bool DeviceDb::collect(int* dSelect, int emptyFrom, std::vector<int>* flagged) {
     return true;
 }
 
-int DeviceDb::search_topk(const Scoring& s, int wantEnd, int k, const int* map, int* outIndex, int* outScore, int* outEndQ, int* outEndT) {
-    const int kk = std::min(k, n_);
+int SearchContext::search_topk(const Scoring& s, int wantEnd, int k, const int* map, int* outIndex, int* outScore, int* outEndQ, int* outEndT) {
+    const int kk = std::min(k, db_.n);
     if (kk <= 0) return 0;
     if (s.Q <= 0) {  // degenerate: every result is written by the host anyway
-        std::vector<int> sc((size_t)n_), eq((size_t)n_, -1), et((size_t)n_, -1);
+        std::vector<int> sc((size_t)db_.n), eq((size_t)db_.n, -1), et((size_t)db_.n, -1);
         const int rc = search(s, wantEnd, nullptr, SearchOut::arrays(sc.data(), eq.data(), et.data()), nullptr);
         if (rc) return rc;
-        std::vector<int> idx((size_t)n_);
-        for (int i = 0; i < n_; i++) idx[i] = i;
+        std::vector<int> idx((size_t)db_.n);
+        for (int i = 0; i < db_.n; i++) idx[i] = i;
         auto better = [&](int a, int b) { return sc[a] != sc[b] ? sc[a] > sc[b] : (map ? map[a] < map[b] : a < b); };
         std::partial_sort(idx.begin(), idx.begin() + kk, idx.end(), better);
         for (int j = 0; j < kk; j++) { outIndex[j] = idx[j]; outScore[j] = sc[idx[j]]; outEndQ[j] = wantEnd ? eq[idx[j]] : -1; outEndT[j] = wantEnd ? et[idx[j]] : -1; }
@@ -1778,22 +1769,21 @@ int DeviceDb::search_topk(const Scoring& s, int wantEnd, int k, const int* map, 
     }
     // Device path: the search leaves [score | endQ | endT] in HBM, the k best are selected there (caller indices of a
     // shard ascend with the map, so the key can use them) and 16 k bytes come back.
-    if (cudaSetDevice(device_) != cudaSuccess) { set_error("cudaSetDevice failed"); return OPAL_B200_ERR_CUDA; }
-    const size_t selectInts = (size_t)n_ + 4 * (size_t)kk + 16;
+    if (cudaSetDevice(db_.device) != cudaSuccess) { set_error("cudaSetDevice failed"); return OPAL_B200_ERR_CUDA; }
+    const size_t selectInts = (size_t)db_.n + 4 * (size_t)kk + 16;
     int* dSelect = nullptr;  // [count | flagged positions (n) | k records]
-    if (!device_alloc(device_, (void**)&dSelect, sizeof(int) * selectInts)) return OPAL_B200_ERR_CUDA;
-    if (!ensure_order()) { device_release(device_, dSelect); return OPAL_B200_ERR_CUDA; }
+    if (!device_alloc(db_.device, (void**)&dSelect, sizeof(int) * selectInts)) return OPAL_B200_ERR_CUDA;
     const int rc = search(s, wantEnd, nullptr, SearchOut::on_device(dSelect), nullptr);
-    if (rc) { device_release(device_, dSelect); return rc; }
-    int4* dRecords = reinterpret_cast<int4*>(dSelect + (((size_t)n_ + 4) & ~(size_t)3));
-    topk_select_kernel<<<1, 1024, 0, stream_>>>(dScore_, dEndQ_, dEndT_, dOrder_, n_, kk, wantEnd, dRecords);
+    if (rc) { device_release(db_.device, dSelect); return rc; }
+    int4* dRecords = reinterpret_cast<int4*>(dSelect + (((size_t)db_.n + 4) & ~(size_t)3));
+    topk_select_kernel<<<1, 1024, 0, stream_>>>(dScore_, dEndQ_, dEndT_, db_.dOrder, db_.n, kk, wantEnd, dRecords);
     std::vector<int4> rec((size_t)kk);
     if (cudaGetLastError() != cudaSuccess ||
         cudaMemcpyAsync(rec.data(), dRecords, sizeof(int4) * (size_t)kk, cudaMemcpyDeviceToHost, stream_) != cudaSuccess ||
         cudaStreamSynchronize(stream_) != cudaSuccess) {
-        set_error("top-k selection failed"); device_release(device_, dSelect); return OPAL_B200_ERR_CUDA;
+        set_error("top-k selection failed"); device_release(db_.device, dSelect); return OPAL_B200_ERR_CUDA;
     }
-    device_release(device_, dSelect);
+    device_release(db_.device, dSelect);
     std::sort(rec.begin(), rec.end(), [&](const int4& a, const int4& b) { return a.y != b.y ? a.y > b.y : (map ? map[a.x] < map[b.x] : a.x < b.x); });
     for (int j = 0; j < kk; j++) {
         outIndex[j] = rec[j].x; outScore[j] = rec[j].y;
@@ -1803,45 +1793,45 @@ int DeviceDb::search_topk(const Scoring& s, int wantEnd, int k, const int* map, 
     return 0;
 }
 
-// The device copy of the index map (sorted position -> caller index) that the selection reads, made once; the search
-// contexts borrow it as they borrow the database arrays.
+// The device copy of the index map (sorted position -> caller index) that the selection reads, made once in the
+// database arrays, where every context reads it.
 bool DeviceDb::ensure_order() {
-    if (dOrder_) return true;
-    if (!ensure_uploaded() || !device_alloc(device_, (void**)&dOrder_, sizeof(int) * (size_t)std::max(n_, 1)) ||
-        cudaMemcpyAsync(dOrder_, lay_->order.data(), sizeof(int) * (size_t)n_, cudaMemcpyHostToDevice, stream_) != cudaSuccess ||
-        cudaStreamSynchronize(stream_) != cudaSuccess) {
+    if (db_.dOrder) return true;
+    if (!ensure_uploaded() || !device_alloc(db_.device, (void**)&db_.dOrder, sizeof(int) * (size_t)std::max(db_.n, 1)) ||
+        cudaMemcpyAsync(db_.dOrder, db_.lay->order.data(), sizeof(int) * (size_t)db_.n, cudaMemcpyHostToDevice, stream()) != cudaSuccess ||
+        cudaStreamSynchronize(stream()) != cudaSuccess) {
         set_error("upload of the index map failed");
         return false;
     }
-    for (DeviceDb* c : contexts_) c->dOrder_ = dOrder_;
     return true;
 }
 
 int DeviceDb::check(const Scoring& s) {
     ScoreBounds b;
     if (const int rc = s.validate(&b)) return rc;
-    if (s.Q <= 0 || lay_->nonEmpty == 0) return 0;  // nothing is swept, so no residue code is read (see run_classes)
+    if (s.Q <= 0 || db_.lay->nonEmpty == 0) return 0;  // nothing is swept, so no residue code is read (see run_classes)
     if (!ensure_uploaded()) return OPAL_B200_ERR_CUDA;
-    if (maxCode_ >= s.A) { set_error("database holds residue codes >= alphabetLength"); return OPAL_B200_ERR_ARGUMENT; }
+    if (*db_.hMaxCode >= s.A) { set_error("database holds residue codes >= alphabetLength"); return OPAL_B200_ERR_ARGUMENT; }
     return 0;
 }
 
 // Searches claim the next index in order and stop claiming after a failure, so every search below the lowest failed
-// one has run: its code is the one a loop of single searches would have returned.
-int DeviceDb::in_flight(int num, int inFlight, const std::function<int(DeviceDb*, int)>& job, float* batchMs) {
+// one has run: its code is the one a loop of single searches would have returned.  The upload is waited for before
+// the contexts are made, so none of them waits for it on a thread of its own.
+int DeviceDb::in_flight(int num, int inFlight, const std::function<int(SearchContext&, int)>& job, float* batchMs) {
     if (batchMs) *batchMs = 0.f;
     if (num <= 0) return 0;
     const int K = std::max(1, std::min(std::min(inFlight, num), 16));
-    if (cudaSetDevice(device_) != cudaSuccess) { set_error("cudaSetDevice failed"); return OPAL_B200_ERR_CUDA; }
-    while ((int)contexts_.size() < K - 1) {
-        DeviceDb* c = clone_context();
-        if (!c) return OPAL_B200_ERR_CUDA;
-        contexts_.push_back(c);
-    }
+    if (cudaSetDevice(db_.device) != cudaSuccess) { set_error("cudaSetDevice failed"); return OPAL_B200_ERR_CUDA; }
     if (!ensure_uploaded()) return OPAL_B200_ERR_CUDA;
+    while ((int)contexts_.size() < K) {
+        auto c = std::make_unique<SearchContext>(db_);
+        if (!c->alloc_search_buffers()) return OPAL_B200_ERR_CUDA;
+        contexts_.push_back(std::move(c));
+    }
     cudaEvent_t evBatch = nullptr;
-    if (!event_acquire(device_, &evBatch)) return OPAL_B200_ERR_CUDA;
-    if (cudaEventRecord(evBatch, stream_) != cudaSuccess) { event_release(device_, evBatch); set_error("cudaEventRecord failed"); return OPAL_B200_ERR_CUDA; }
+    if (!event_acquire(db_.device, &evBatch)) return OPAL_B200_ERR_CUDA;
+    if (cudaEventRecord(evBatch, stream()) != cudaSuccess) { event_release(db_.device, evBatch); set_error("cudaEventRecord failed"); return OPAL_B200_ERR_CUDA; }
     std::atomic<int> next(0);
     std::atomic<bool> stop(false);
     std::vector<int> rcs((size_t)num, 0);
@@ -1849,15 +1839,15 @@ int DeviceDb::in_flight(int num, int inFlight, const std::function<int(DeviceDb*
     std::vector<float> lastStop((size_t)K, 0.f);
     std::vector<int> launches((size_t)K, 0), reruns((size_t)K, 0);
     auto worker = [&](int k) {
-        DeviceDb* ctx = k == 0 ? this : contexts_[k - 1];
+        SearchContext& ctx = *contexts_[k];
         while (!stop.load()) {
             const int q = next.fetch_add(1);
             if (q >= num) break;
             const int rc = job(ctx, q);
             if (rc) { rcs[q] = rc; errors[q] = last_error(); stop.store(true); break; }
-            launches[k] += ctx->stats_.kernelLaunches; reruns[k] += ctx->stats_.rerun32;
+            launches[k] += ctx.stats_.kernelLaunches; reruns[k] += ctx.stats_.rerun32;
             float ms = 0.f;
-            if (ctx->startRecorded_ && cudaEventElapsedTime(&ms, evBatch, ctx->evStop_) == cudaSuccess) lastStop[k] = std::max(lastStop[k], ms);
+            if (ctx.startRecorded_ && cudaEventElapsedTime(&ms, evBatch, ctx.evStop_) == cudaSuccess) lastStop[k] = std::max(lastStop[k], ms);
         }
     };
     if (K == 1) worker(0);
@@ -1869,32 +1859,33 @@ int DeviceDb::in_flight(int num, int inFlight, const std::function<int(DeviceDb*
         t_overlapped = false;
         for (auto& t : th) t.join();
     }
-    event_release(device_, evBatch);
+    event_release(db_.device, evBatch);
     for (int q = 0; q < num; q++)
         if (rcs[q]) { set_error(errors[q]); return rcs[q]; }
     if (batchMs) *batchMs = *std::max_element(lastStop.begin(), lastStop.end());
-    stats_.kernelLaunches = stats_.rerun32 = 0;  // batch totals
-    for (int k = 0; k < K; k++) { stats_.kernelLaunches += launches[k]; stats_.rerun32 += reruns[k]; }
+    SearchStats& stats = contexts_[0]->stats_;  // batch totals
+    stats.kernelLaunches = stats.rerun32 = 0;
+    for (int k = 0; k < K; k++) { stats.kernelLaunches += launches[k]; stats.rerun32 += reruns[k]; }
     return 0;
 }
 
 int DeviceDb::search_batch(const std::vector<Scoring>& searches, int wantEnd, int* scores, int* endQ, int* endT, int inFlight,
                            float* batchMs) {
-    return in_flight((int)searches.size(), inFlight, [&](DeviceDb* ctx, int q) {
-        const size_t base = (size_t)q * (size_t)n_;
+    return in_flight((int)searches.size(), inFlight, [&](SearchContext& ctx, int q) {
+        const size_t base = (size_t)q * (size_t)db_.n;
         const SearchOut out = SearchOut::arrays(scores + base, endQ ? endQ + base : nullptr, endT ? endT + base : nullptr);
-        return ctx->search(searches[q], wantEnd, nullptr, out, nullptr);
+        return ctx.search(searches[q], wantEnd, nullptr, out, nullptr);
     }, batchMs);
 }
 
 int DeviceDb::search_batch_topk(const std::vector<Scoring>& searches, int wantEnd, int k, const int* map, int* outIndex, int* outScore,
                                 int* outEndQ, int* outEndT, int inFlight) {
     if (k <= 0 || searches.empty()) return 0;
-    if (cudaSetDevice(device_) != cudaSuccess) { set_error("cudaSetDevice failed"); return OPAL_B200_ERR_CUDA; }
-    if (!ensure_order()) return OPAL_B200_ERR_CUDA;  // before the contexts start: they borrow it
-    return in_flight((int)searches.size(), inFlight, [&](DeviceDb* ctx, int q) {
+    if (cudaSetDevice(db_.device) != cudaSuccess) { set_error("cudaSetDevice failed"); return OPAL_B200_ERR_CUDA; }
+    if (!ensure_order()) return OPAL_B200_ERR_CUDA;
+    return in_flight((int)searches.size(), inFlight, [&](SearchContext& ctx, int q) {
         const size_t base = (size_t)q * (size_t)k;
-        return ctx->search_topk(searches[q], wantEnd, k, map, outIndex + base, outScore + base, outEndQ + base, outEndT + base);
+        return ctx.search_topk(searches[q], wantEnd, k, map, outIndex + base, outScore + base, outEndQ + base, outEndT + base);
     }, nullptr);
 }
 

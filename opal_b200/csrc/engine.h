@@ -143,60 +143,49 @@ std::shared_ptr<const Layout> layout_for(const int* lens, const int* order, int 
 void set_thread_overlapped(bool on);
 struct PhaseTrace;  // phase timings on stderr with OPAL_B200_TRACE=1 (engine.cu)
 
-// A length-sorted (longest first) database resident in one device's HBM.
-class DeviceDb {
+// A length-sorted (longest first) database resident in one device's HBM, built by DeviceDb::build and read-only once
+// its upload has finished.  It is the only owner of these allocations; search contexts read them through a const
+// reference.
+struct DbArrays {
+    int device = 0, n = 0, numSMs = 0, smemLimit = 0;
+    long long totalResidues = 0;
+    std::shared_ptr<const Layout> lay;
+    unsigned char *hBlock = nullptr, *dBlock = nullptr;  // offsets | pair offsets | fold offsets | lengths | max code | residues (pinned / device)
+    uint8_t *hResidues = nullptr, *dResidues = nullptr;  // views: the pinned host copy and the device copy
+    long long *dOffsets = nullptr, *dPairOffsets = nullptr, *dFoldOffsets = nullptr;
+    int *dLengths = nullptr, *dMaxCode = nullptr;
+    uint16_t* dPairStream = nullptr;
+    uint16_t* dFoldStream = nullptr;  // folded stream of the numFold longest targets
+    int numPairs = 0, numFold = 0;
+    int* hMaxCode = nullptr;  // pinned: the largest residue code, copied back by the upload (read once it has finished)
+    int* dOrder = nullptr;    // device copy of lay->order (sorted position -> caller index), made by DeviceDb::ensure_order
+
+    DbArrays() = default;
+    DbArrays(const DbArrays&) = delete;
+    DbArrays& operator=(const DbArrays&) = delete;
+    ~DbArrays();
+};
+
+// One search in flight on a resident database: its stream and events, result and argument blocks, boundary rows and
+// chained-launch scratch.  It reads the database arrays and owns none of them.
+class SearchContext {
 public:
-    static DeviceDb* create(unsigned char* const* db, int n, const int* lens, int device);
-    // Database that is already packed: residues contiguous, longest sequence first; order[p] = caller index of
-    // sorted position p (NULL = identity).  This is the in-memory form of the on-disk format (cli/packed_db.h).
-    static DeviceDb* create_sorted(const unsigned char* residues, const int* sortedLens, const int* order, int n, int device);
-    ~DeviceDb();
-
-    // Several queries against the resident database, up to `inFlight` of them on the device at a time (each on a
-    // search context of its own: streams, result and scratch buffers), so that the tail of one query overlaps the
-    // bulk of the next and host-side planning / publishing overlaps kernels.  Outputs are [search][caller index].
-    int search_batch(const std::vector<Scoring>& searches, int wantEnd, int* scores, int* endQ, int* endT, int inFlight,
-                     float* batchMs);
-    // Blocks until the upload issued by create() has finished (create() returns with it in flight).
+    explicit SearchContext(const DbArrays& db) : db_(db) {}
+    SearchContext(const SearchContext&) = delete;
+    ~SearchContext();
+    bool alloc_search_buffers();
+    // Blocks until the database upload issued on this context's stream has finished (nothing to wait for elsewhere).
     bool ensure_uploaded();
-
     // Score / score+end for every non-skipped target, into `out`.  Stages: Scoring::validate, route (every target to
     // the 16- or the 32-bit class), upload_args, ladder (16 bits, then 32 bits for what 16 could not hold).
     int search(const Scoring& s, int wantEnd, const unsigned char* skip, const SearchOut& out, float* deviceMs);
-
     // Score [+ end] search followed by the selection of the k best targets: score descending, then smallest
-    // map[caller index] (map NULL: the caller index itself).  Writes k (<= size()) caller indices and their records.
+    // map[caller index] (map NULL: the caller index itself).  Writes k (<= n) caller indices and their records.  Reads
+    // the index map made by DeviceDb::ensure_order.
     int search_topk(const Scoring& s, int wantEnd, int k, const int* map, int* outIndex, int* outScore, int* outEndQ, int* outEndT);
-    // search_topk of every search, up to `inFlight` of them on the device at a time (as search_batch); k <= size().
-    // Outputs are [search][k].  0, or the code of the lowest-index search that failed.
-    int search_batch_topk(const std::vector<Scoring>& searches, int wantEnd, int k, const int* map, int* outIndex, int* outScore,
-                          int* outEndQ, int* outEndT, int inFlight);
-    // The checks a search makes before it sweeps: Scoring::validate, then (for a search that sweeps at all) the
-    // database's residue codes against the alphabet length.  0 or an OPAL_B200_ERR_* code.
-    int check(const Scoring& s);
-
-    int size() const { return n_; }
-    long long residues() const { return totalResidues_; }
-    const SearchStats& stats() const { return stats_; }
-    int device() const { return device_; }
-    cudaStream_t stream() const { return stream_; }
-    // sorted position -> caller index, and device-side views (used by the alignment stage)
-    const std::vector<int>& order() const { return lay_->order; }
-    const std::vector<int>& sorted_position() const { return lay_->pos; }
-    const uint8_t* d_residues() const { return dResidues_; }
-    const long long* d_offsets() const { return dOffsets_; }
-    const std::vector<long long>& offsets() const { return lay_->offsets; }
-    const std::vector<int>& sorted_lengths() const { return lay_->sortedLen; }
-    const uint8_t* h_residues() const { return hResidues_; }  // pinned host copy, sorted order
 
 private:
-    DeviceDb() {}
-    static DeviceDb* build(unsigned char* const* db, const unsigned char* packed, const int* lens, const int* order, int n, int device);
-    DeviceDb* clone_context();
-    bool ensure_order();
-    // job(context, q) for every q in [0, num), up to inFlight at a time, each context on a host thread of its own.
-    int in_flight(int num, int inFlight, const std::function<int(DeviceDb*, int)>& job, float* batchMs);
-    bool alloc_search_buffers();
+    friend class DeviceDb;  // build() uploads on the first context's stream; in_flight() reads every context's stats and timing
     struct Group;
     struct Run;     // the search in progress (engine.cu)
     struct Routes;  // its targets by precision class
@@ -211,29 +200,14 @@ private:
     int run_classes(const std::vector<std::pair<int, const std::vector<int>*>>& classes, const Run& run);
     bool ensure_boundary();
 
-    int device_ = 0, n_ = 0, numSMs_ = 0, smemLimit_ = 0;
-    long long totalResidues_ = 0;
-    std::shared_ptr<const Layout> lay_;
-    bool ownsDb_ = true, uploaded_ = false;  // search contexts made by clone_context() borrow the database arrays
-    std::vector<DeviceDb*> contexts_;
-    uint8_t* hResidues_ = nullptr;
-    uint8_t* dResidues_ = nullptr;
-    long long* dOffsets_ = nullptr;
-    int* dLengths_ = nullptr;
+    const DbArrays& db_;
+    bool uploadPending_ = false;  // the database upload was issued on stream_ and has not been waited for
     int *dResults_ = nullptr, *hResults_ = nullptr;  // [score | endQ | endT | task list] device block, [score | endQ | endT] pinned
     int *dScore_ = nullptr, *dEndQ_ = nullptr, *dEndT_ = nullptr, *dTaskList_ = nullptr;  // views
+    int *hScore_ = nullptr, *hEndQ_ = nullptr, *hEndT_ = nullptr;  // views into hResults_
     uint32_t *dBndH_ = nullptr, *dBndF_ = nullptr;
-    uint16_t* dPairStream_ = nullptr;
-    long long* dPairOffsets_ = nullptr;
-    uint16_t* dFoldStream_ = nullptr;    // folded stream of the numFold_ longest targets
-    long long* dFoldOffsets_ = nullptr;
-    int numFold_ = 0;
-    int *dMaxCode_ = nullptr, *hMaxCode_ = nullptr;
-    unsigned char *hBlock_ = nullptr, *dBlock_ = nullptr;  // offsets | pair offsets | lengths | max code | residues (pinned / device)
-    int numPairs_ = 0, maxCode_ = 0;
     unsigned char *dArgs_ = nullptr, *hArgs_ = nullptr;  // launch counters | score matrix | query, or counters | PSSM (device / pinned)
     size_t argsCapacity_ = 0;
-    int *hScore_ = nullptr, *hEndQ_ = nullptr, *hEndT_ = nullptr;  // views into hResults_
     cudaStream_t stream_ = nullptr;
     cudaEvent_t evStart_ = nullptr, evStop_ = nullptr, evFork_ = nullptr;
     std::vector<cudaStream_t> auxStreams_;
@@ -241,7 +215,58 @@ private:
     SearchStats stats_;
     std::vector<void*> chainScratch_;  // device blocks of chained launches (boundary rows, flags), released by the next search
     bool startRecorded_ = false;
-    int* dOrder_ = nullptr;       // device copy of order_ (sorted position -> caller index), made by the first top-k search, borrowed by the contexts
+};
+
+// A resident database and the search contexts that run on it.
+class DeviceDb {
+public:
+    static DeviceDb* create(unsigned char* const* db, int n, const int* lens, int device);
+    // Database that is already packed: residues contiguous, longest sequence first; order[p] = caller index of
+    // sorted position p (NULL = identity).  This is the in-memory form of the on-disk format (cli/packed_db.h).
+    static DeviceDb* create_sorted(const unsigned char* residues, const int* sortedLens, const int* order, int n, int device);
+
+    // Several queries against the resident database, up to `inFlight` of them on the device at a time (each on a
+    // search context of its own: streams, result and scratch buffers), so that the tail of one query overlaps the
+    // bulk of the next and host-side planning / publishing overlaps kernels.  Outputs are [search][caller index].
+    int search_batch(const std::vector<Scoring>& searches, int wantEnd, int* scores, int* endQ, int* endT, int inFlight,
+                     float* batchMs);
+    // Blocks until the upload issued by create() has finished (create() returns with it in flight).
+    bool ensure_uploaded() { return contexts_[0]->ensure_uploaded(); }
+
+    // SearchContext::search on the first context.
+    int search(const Scoring& s, int wantEnd, const unsigned char* skip, const SearchOut& out, float* deviceMs) {
+        return contexts_[0]->search(s, wantEnd, skip, out, deviceMs);
+    }
+
+    // For every search: the score [+ end] search followed by the selection of the k best targets (score descending,
+    // then smallest map[caller index]; map NULL: the caller index itself), up to `inFlight` of them on the device at
+    // a time (as search_batch); k <= size().  Outputs are [search][k] caller indices and their records.  0, or the
+    // code of the lowest-index search that failed.
+    int search_batch_topk(const std::vector<Scoring>& searches, int wantEnd, int k, const int* map, int* outIndex, int* outScore,
+                          int* outEndQ, int* outEndT, int inFlight);
+    // The checks a search makes before it sweeps: Scoring::validate, then (for a search that sweeps at all) the
+    // database's residue codes against the alphabet length.  0 or an OPAL_B200_ERR_* code.
+    int check(const Scoring& s);
+
+    int size() const { return db_.n; }
+    long long residues() const { return db_.totalResidues; }
+    const SearchStats& stats() const { return contexts_[0]->stats_; }
+    int device() const { return db_.device; }
+    // What the alignment stage reads: the database arrays, and the stream of the first context to run on.
+    const DbArrays& arrays() const { return db_; }
+    cudaStream_t stream() const { return contexts_[0]->stream_; }
+
+private:
+    DeviceDb() {}
+    static DeviceDb* build(unsigned char* const* db, const unsigned char* packed, const int* lens, const int* order, int n, int device);
+    bool ensure_order();
+    // job(context, q) for every q in [0, num), up to inFlight at a time, each context on a host thread of its own.
+    int in_flight(int num, int inFlight, const std::function<int(SearchContext&, int)>& job, float* batchMs);
+
+    DbArrays db_;
+    // [0]: made with the database, which is uploaded on its stream; in_flight adds more.  Declared after db_, so every
+    // context has synchronized its streams and released its blocks before the database arrays go.
+    std::vector<std::unique_ptr<SearchContext>> contexts_;
 };
 
 double measure_dpx_peak(int device, int mix, double* threadInstrPerSec, float* ms);  // mix 0 = SW recurrence, 1 = NW / HW / OV
