@@ -186,6 +186,39 @@ int opalb200_db_search_batch_topk_pssm(OpalB200Db* handle, int numSearches, cons
                                        int alphabetLength, int gapOpen, int gapExt, int searchType, int k,
                                        int* indices, struct OpalSearchResult* results[], int* found, int inFlight);
 
+/*
+ * Scores a list of (query, database entry) pairs instead of every query against the whole database: the second stage of
+ * a search pipeline (rescoring the candidates a prefilter proposes, all-vs-all inside clusters, re-aligning earlier
+ * hits).  Pair p scores queries[pairQuery[p]] (queryLengths[pairQuery[p]] residues) against database entry
+ * pairTarget[p] (caller index).  Its result is exactly what opalSearchDatabase gives for that query against a
+ * one-sequence database holding that entry -- score, end-location tie-breaking, the defined results of empty queries
+ * and targets, overflow -- which is also entry pairTarget[p] of opalb200_db_search for that query on this handle.
+ * Pairs may come in any order and may repeat; a query may appear in any number of pairs, or in none.  The work, the
+ * copies and the host time grow with numPairs and the residues of the pairs' targets, not with the database size.
+ * All queries share the scoring arguments (as opalb200_db_search).  searchType is 0 or 1; scores, endQuery and
+ * endTarget have numPairs entries, indexed by p (endQuery / endTarget may be NULL for searchType 0).  deviceMs
+ * (nullable) receives the CUDA-event time from the first launch to the last kernel end.  numPairs = 0 (with counts
+ * >= 0) returns 0 and reads and writes nothing else.
+ * Every argument is checked before anything runs, and on any failure nothing is written (deviceMs included): counts
+ * must be >= 0, the arrays non-NULL when their count is > 0, searchType 0 or 1; every pairQuery[p] must lie in [0, numQueries) and every pairTarget[p] in
+ * [0, dbLength) (else OPAL_ERR_INVALID_ARGUMENT, opalb200_last_error() naming the first bad pair); then every query goes
+ * through the checks of a single search, and the code of the lowest-index query that fails is returned.  On a handle
+ * dealt over several devices, each pair runs on the device that owns its target, the devices concurrently.
+ */
+int opalb200_db_search_pairs(OpalB200Db* handle, int numQueries, const unsigned char* const queries[],
+                             const int queryLengths[], int numPairs, const int pairQuery[], const int pairTarget[],
+                             int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength,
+                             int searchType, int mode, int* scores, int* endQuery, int* endTarget, float* deviceMs);
+/*
+ * opalb200_db_search_pairs into opalSearchDatabase's records: results[p] (distinct records) receives pair p's result at
+ * any of the three search levels, OPAL_SEARCH_ALIGNMENT included, with opalSearchDatabase's reuse rule (a record that
+ * already holds a score -- and an end location, above OPAL_SEARCH_SCORE -- is not recomputed).  Same checks and codes.
+ */
+int opalb200_db_search_pairs_results(OpalB200Db* handle, int numQueries, const unsigned char* const queries[],
+                                     const int queryLengths[], int numPairs, const int pairQuery[], const int pairTarget[],
+                                     int gapOpen, int gapExt, const int* scoreMatrix, int alphabetLength,
+                                     struct OpalSearchResult* results[], int searchType, int mode);
+
 /* Statistics of the last search on this handle: kernels launched, targets re-run in 32 bits, and the
  * geometry of the last launched class (threads per target pair, query rows per thread, passes over the
  * query, resident warps per SM scheduler partition), and the number of concurrent launch groups. Any pointer may be NULL. */

@@ -102,6 +102,16 @@ struct DbHandle {
     ~DbHandle() { for (DeviceDb* d : shards) delete d; }
     int parts() const { return (int)shards.size(); }
     int caller_index(int s, int local) const { return index.empty() ? local : index[s][local]; }
+    // caller index -> (shard, local index) on a handle of several shards, made on first use (the pairs calls)
+    std::once_flag ownersOnce;
+    std::vector<int> shardOf, localOf;
+    void owners() {
+        std::call_once(ownersOnce, [this] {
+            shardOf.assign((size_t)n, 0); localOf.assign((size_t)n, 0);
+            for (size_t s = 0; s < index.size(); s++)
+                for (size_t k = 0; k < index[s].size(); k++) { shardOf[index[s][k]] = (int)s; localOf[index[s][k]] = (int)k; }
+        });
+    }
     void collect_stats() {
         stats = shards[0]->stats();
         for (size_t s = 1; s < shards.size(); s++) {
@@ -678,6 +688,120 @@ int opalb200_db_search_batch_topk_pssm(OpalB200Db* hh, int numSearches, const un
         searches.push_back(Scoring::with_pssm(queries ? queries[q] : nullptr, pssms[q], queryLengths[q], alphabetLength, gapOpen, gapExt,
                                               modes[q]));
     return db_search_batch_topk(hh, searches, searchType, k, indices, results, found, inFlight);
+}
+
+// Both pairs calls: the arrays call (scores / endQuery / endTarget by pair) or the records call (`results`).  Every
+// argument and every query is checked before anything runs; each pair runs on the device that owns its target, and the
+// outputs are written once every shard has succeeded.
+static int db_search_pairs(OpalB200Db* hh, int numQueries, const unsigned char* const queries[], const int queryLengths[], int numPairs,
+                           const int pairQuery[], const int pairTarget[], int gapOpen, int gapExt, const int* scoreMatrix,
+                           int alphabetLength, int searchType, int mode, int* scores, int* endQuery, int* endTarget, bool records,
+                           OpalSearchResult* const* results, float* deviceMs) {
+    if (!hh) return OPAL_ERR_NO_SIMD_SUPPORT;
+    DeviceGuard guard;
+    DbHandle* h = reinterpret_cast<DbHandle*>(hh);
+    auto bad = [](const std::string& what) { set_error(what); return OPAL_ERR_INVALID_ARGUMENT; };
+    if (numQueries < 0 || numPairs < 0) return bad("numQueries and numPairs must be >= 0");
+    if (numPairs == 0) return 0;  // nothing to score: no further argument is read, nothing is written
+    if (numQueries > 0 && (!queries || !queryLengths)) return bad("queries / queryLengths is NULL");
+    if (!pairQuery || !pairTarget) return bad("pairQuery / pairTarget is NULL");
+    if (records) {
+        if (!results) return bad("results is NULL");
+        if (searchType < OPAL_SEARCH_SCORE || searchType > OPAL_SEARCH_ALIGNMENT) return bad("searchType must be 0, 1 or 2");
+    } else {
+        if (searchType != OPAL_SEARCH_SCORE && searchType != OPAL_SEARCH_SCORE_END) return bad("searchType must be 0 or 1");
+        if (!scores || (searchType == OPAL_SEARCH_SCORE_END && (!endQuery || !endTarget)))
+            return bad("scores / endQuery / endTarget is NULL");
+    }
+    for (int p = 0; p < numPairs; p++) {
+        if (pairQuery[p] < 0 || pairQuery[p] >= numQueries)
+            return bad("pair " + std::to_string(p) + ": pairQuery " + std::to_string(pairQuery[p]) + " is outside [0, numQueries)");
+        if (pairTarget[p] < 0 || pairTarget[p] >= h->n)
+            return bad("pair " + std::to_string(p) + ": pairTarget " + std::to_string(pairTarget[p]) + " is outside [0, dbLength)");
+    }
+    std::vector<Scoring> searches;
+    for (int q = 0; q < numQueries; q++)
+        searches.push_back(Scoring::with_matrix(queries[q], queryLengths[q], scoreMatrix, alphabetLength, gapOpen, gapExt, mode));
+    for (const Scoring& s : searches)
+        for (int sh = 0; sh < h->parts(); sh++)
+            if (const int rc = h->shards[sh]->check(s)) return rc;
+
+    // the pairs that need work, dealt to the shards that own their targets (records: opalSearchDatabase's reuse rule)
+    const int parts = h->parts(), wantEnd = searchType != OPAL_SEARCH_SCORE;
+    const bool dealt = !h->index.empty();
+    if (dealt) h->owners();
+    auto shard_of = [&](int p) { return dealt ? h->shardOf[pairTarget[p]] : 0; };
+    auto local_of = [&](int p) { return dealt ? h->localOf[pairTarget[p]] : pairTarget[p]; };
+    std::vector<std::vector<int>> mine((size_t)parts);
+    for (int p = 0; p < numPairs; p++) {
+        const OpalSearchResult* r = results ? results[p] : nullptr;
+        if (r && r->scoreSet && (searchType == OPAL_SEARCH_SCORE || (r->endLocationQuery >= 0 && r->endLocationTarget >= 0))) continue;
+        mine[shard_of(p)].push_back(p);
+    }
+    std::vector<int> sc((size_t)numPairs), eq((size_t)numPairs), et((size_t)numPairs);  // by pair
+    std::vector<float> ms((size_t)parts, 0.f);
+    int rc = on_shards(parts, [&](int s) -> int {
+        const std::vector<int>& ks = mine[s];
+        const int m = (int)ks.size();
+        if (m == 0) return 0;
+        std::vector<int> pq((size_t)m), pt((size_t)m), lsc((size_t)m), leq((size_t)m), let((size_t)m);
+        for (int j = 0; j < m; j++) { pq[j] = pairQuery[ks[j]]; pt[j] = local_of(ks[j]); }
+        const int r = h->shards[s]->search_pairs(searches, wantEnd, m, pq.data(), pt.data(), SearchOut::arrays(lsc.data(), leq.data(), let.data()),
+                                                 &ms[s]);
+        if (r) return r;
+        for (int j = 0; j < m; j++) { sc[ks[j]] = lsc[j]; eq[ks[j]] = leq[j]; et[ks[j]] = let[j]; }
+        return 0;
+    });
+    h->collect_stats();
+    if (rc) return rc;
+    if (deviceMs) *deviceMs = *std::max_element(ms.begin(), ms.end());  // the devices run concurrently
+    for (int s = 0; s < parts; s++)
+        for (int p : mine[s]) {
+            if (!records) {
+                scores[p] = sc[p];
+                if (endQuery) endQuery[p] = wantEnd ? eq[p] : -1;
+                if (endTarget) endTarget[p] = wantEnd ? et[p] : -1;
+            } else {
+                OpalSearchResult* r = results[p];  // reference src/opal.cpp:1561-1564, 420-426, 869-905
+                r->scoreSet = 1; r->score = sc[p]; r->endLocationQuery = eq[p]; r->endLocationTarget = et[p];
+            }
+        }
+    if (!records) return 0;
+    if (searchType != OPAL_SEARCH_ALIGNMENT) {  // :1508-1515, reused records included
+        for (int p = 0; p < numPairs; p++) {
+            OpalSearchResult* r = results[p];
+            r->alignment = NULL; r->alignmentLength = -1; r->startLocationQuery = r->startLocationTarget = -1;
+        }
+        return 0;
+    }
+    // start + alignment of every pair on the device that owns its target: one set per query (a target may repeat in a set)
+    return on_shards(parts, [&](int s) -> int {
+        std::vector<std::vector<int>> subset((size_t)numQueries);
+        std::vector<std::vector<OpalSearchResult*>> res((size_t)numQueries);
+        for (int p = 0; p < numPairs; p++)
+            if (shard_of(p) == s) { subset[pairQuery[p]].push_back(local_of(p)); res[pairQuery[p]].push_back(results[p]); }
+        std::vector<AlignSet> sets;
+        for (int q = 0; q < numQueries; q++)
+            if (!subset[q].empty()) sets.push_back({&searches[q], res[q].data(), (int)subset[q].size(), subset[q].data()});
+        if (sets.empty()) return 0;
+        DeviceDb* d = h->shards[s];
+        return d->ensure_uploaded() ? align_database(d->arrays(), d->stream(), sets) : OPAL_B200_ERR_CUDA;
+    });
+}
+
+int opalb200_db_search_pairs(OpalB200Db* handle, int numQueries, const unsigned char* const queries[], const int queryLengths[],
+                             int numPairs, const int pairQuery[], const int pairTarget[], int gapOpen, int gapExt,
+                             const int* scoreMatrix, int alphabetLength, int searchType, int mode, int* scores, int* endQuery,
+                             int* endTarget, float* deviceMs) {
+    return db_search_pairs(handle, numQueries, queries, queryLengths, numPairs, pairQuery, pairTarget, gapOpen, gapExt, scoreMatrix,
+                           alphabetLength, searchType, mode, scores, endQuery, endTarget, false, nullptr, deviceMs);
+}
+
+int opalb200_db_search_pairs_results(OpalB200Db* handle, int numQueries, const unsigned char* const queries[], const int queryLengths[],
+                                     int numPairs, const int pairQuery[], const int pairTarget[], int gapOpen, int gapExt,
+                                     const int* scoreMatrix, int alphabetLength, OpalSearchResult* results[], int searchType, int mode) {
+    return db_search_pairs(handle, numQueries, queries, queryLengths, numPairs, pairQuery, pairTarget, gapOpen, gapExt, scoreMatrix,
+                           alphabetLength, searchType, mode, nullptr, nullptr, nullptr, true, results, nullptr);
 }
 
 void opalb200_db_last_stats(const OpalB200Db* h, int* kernelLaunches, int* rerun32, int* G, int* R, int* passes,

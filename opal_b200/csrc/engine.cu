@@ -10,6 +10,7 @@
 #include <emmintrin.h>
 
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -22,6 +23,7 @@
 #include <unordered_map>
 
 #include "r_list.h"
+#include "pairs_kernel.cuh"
 #include "search_kernel.cuh"
 
 namespace opalb200 {
@@ -1887,6 +1889,352 @@ int DeviceDb::search_batch_topk(const std::vector<Scoring>& searches, int wantEn
         const size_t base = (size_t)q * (size_t)k;
         return ctx.search_topk(searches[q], wantEnd, k, map, outIndex + base, outScore + base, outEndQ + base, outEndT + base);
     }, nullptr);
+}
+
+// ------------------------------------------------------------------ pairs path
+#define CUDA_TRY_RC(expr)                                                                    \
+    do {                                                                                     \
+        cudaError_t _e = (expr);                                                             \
+        if (_e != cudaSuccess) {                                                             \
+            set_error(std::string(#expr) + ": " + cudaGetErrorString(_e));                   \
+            return OPAL_B200_ERR_CUDA;                                                       \
+        }                                                                                    \
+    } while (0)
+
+// One precision class of a pairs call, grouped and planned: tasks of one query are consecutive (longest target first),
+// blocks serve runs of them (PairBlock), and every query has its strip geometry (PairQuery).
+struct PairsSearch::Class {
+    int type = 0, rIndex = 0, maxG = 1, maxPasses = 1;
+    std::vector<PairQuery> queryTab;
+    std::vector<PairTask> tasks;
+    std::vector<PairBlock> blocks;
+    long long streamEntries = 0, bndWords = 0;
+};
+
+PairsSearch::~PairsSearch() {
+    cudaSetDevice(db_.device);
+    cudaStreamSynchronize(stream_);  // nothing may still be using the blocks when they go back to the cache
+    for (void* p : device_) device_release(db_.device, p);
+    for (void* p : pinned_) pinned_release(p);
+    event_release(db_.device, evStart_); event_release(db_.device, evStop_);
+}
+
+void* PairsSearch::alloc(size_t bytes) {
+    void* p = nullptr;
+    if (!device_alloc(db_.device, &p, bytes)) return nullptr;
+    device_.push_back(p);
+    return p;
+}
+
+// One pinned block, one copy.
+bool PairsSearch::upload(const std::vector<unsigned char>& block, unsigned char** dBlock, unsigned char** hBlock) {
+    void* h = nullptr;
+    if (!pinned_alloc(&h, block.size())) return false;
+    pinned_.push_back(h);
+    memcpy(h, block.data(), block.size());
+    *hBlock = static_cast<unsigned char*>(h);
+    if (!(*dBlock = static_cast<unsigned char*>(alloc(block.size())))) return false;
+    CUDA_TRY(cudaMemcpyAsync(*dBlock, h, block.size(), cudaMemcpyHostToDevice, stream_));
+    return true;
+}
+
+// Geometry and tables of one class.  The strip height is one per launch (it is a template parameter): the one the B200
+// step-time model (step_cycles, three warps per partition) prices lowest over every task of the class.  Per query, the
+// group size G is the smallest power of two whose G x R rows cover the query, within what shared memory holds.
+bool PairsSearch::plan(int type, const std::vector<Scoring>& queries, int wantEnd, const std::vector<std::vector<int>>& byQuery,
+                       const int* pos, Class* c) {
+    const Scoring& s0 = queries[0];
+    const int lanes = type == 0 ? 2 : 1, A = s0.A, warps = kPairsThreads / 32;
+    const int flavorClass = s0.mode == kModeSW ? (wantEnd ? 0 : 1) : 2;
+    const std::vector<int>& sortedLen = db_.lay->sortedLen;
+    auto geometry = [&](int ri, int Q, int* G, int* passes) {
+        const int R = kPairsR[ri];
+        auto smem = [&](int g) { return (size_t)lanes * (A + 1) * ((g * pairs_rpad(R) + 31) / 32 * 32) * 4; };
+        int g = 1;
+        while (g < 32 && g * R < Q) g *= 2;
+        while (g > 1 && smem(g) > (size_t)db_.smemLimit) g /= 2;
+        *G = g;
+        *passes = (Q + g * R - 1) / (g * R);
+        return smem(g) <= (size_t)db_.smemLimit;
+    };
+    double bestCost = 1e300;
+    c->rIndex = -1;
+    for (int ri = 0; ri < 2; ri++) {
+        double cost = 0;
+        bool fits = true;
+        for (size_t q = 0; q < byQuery.size() && fits; q++) {
+            if (byQuery[q].empty()) continue;
+            int G = 1, passes = 1;
+            fits = geometry(ri, queries[q].Q, &G, &passes);
+            double steps = 0;
+            for (size_t j = 0; j < byQuery[q].size(); j += lanes) steps += sortedLen[pos[byQuery[q][j]]] + G - 1;
+            cost += passes * steps * step_cycles(flavorClass, 3, kPairsR[ri]) * G / 32.0;
+        }
+        if (fits && cost < bestCost) { bestCost = cost; c->rIndex = ri; }
+    }
+    if (c->rIndex < 0) { set_error("alphabet too large for the shared-memory query profile"); return false; }
+    c->type = type;
+    const int R = kPairsR[c->rIndex];
+    // Blocks of up to `rounds` tasks per warp: enough blocks that every SM takes several (one is resident at a time), few
+    // enough that the profile build is paid for many tasks.
+    long long warpTasks = 0;
+    for (size_t q = 0; q < byQuery.size(); q++) {
+        int G = 1, passes = 1;
+        geometry(c->rIndex, queries[q].Q, &G, &passes);
+        warpTasks += ((long long)byQuery[q].size() + lanes * (32 / G) - 1) / (lanes * (32 / G));
+    }
+    const int rounds = (int)std::max<long long>(1, std::min<long long>(4, warpTasks / ((long long)db_.numSMs * warps * 8)));
+    long long col = 32, bnd = 0, queryOff = 0;
+    std::vector<double> work;
+    for (size_t q = 0; q < byQuery.size(); q++) {
+        const std::vector<int>& ks = byQuery[q];
+        const long long off = queryOff;
+        queryOff += std::max(queries[q].Q, 0);
+        if (ks.empty()) continue;
+        PairQuery pq;
+        pq.Q = queries[q].Q;
+        geometry(c->rIndex, pq.Q, &pq.G, &pq.passes);
+        pq.padTop = s0.mode == kModeNW ? 0 : pq.passes * pq.G * R - pq.Q;  // HW / OV: the last query row at the bottom of the last pass
+        pq.queryOff = off;
+        const int qIndex = (int)c->queryTab.size();
+        c->queryTab.push_back(pq);
+        c->maxG = std::max(c->maxG, pq.G);
+        c->maxPasses = std::max(c->maxPasses, pq.passes);
+        const int firstTask = (int)c->tasks.size();
+        for (size_t j = 0; j < ks.size(); j += lanes) {
+            PairTask tk;
+            const bool two = lanes == 2 && j + 1 < ks.size();
+            tk.slot[0] = ks[j]; tk.slot[1] = two ? ks[j + 1] : -1;
+            tk.tgt[0] = pos[ks[j]]; tk.tgt[1] = two ? pos[ks[j + 1]] : pos[ks[j]];
+            tk.T[0] = sortedLen[tk.tgt[0]]; tk.T[1] = two ? sortedLen[tk.tgt[1]] : 0;
+            tk.col = type == 0 ? col : 0;
+            if (type == 0) col += tk.T[0] + 32;
+            tk.bnd = pq.passes > 1 ? bnd : 0;
+            if (pq.passes > 1) bnd += tk.T[0];
+            c->tasks.push_back(tk);
+        }
+        const int nt = (int)c->tasks.size() - firstTask, perRound = warps * (32 / pq.G), per = perRound * rounds;
+        for (int k = 0; k < nt; k += per) {
+            const int cnt = std::min(per, nt - k);
+            c->blocks.push_back({qIndex, firstTask + k, cnt, 0});
+            work.push_back((double)pq.passes * (c->tasks[firstTask + k].T[0] + pq.G) * ((cnt + perRound - 1) / perRound));
+        }
+    }
+    c->streamEntries = col + 32;
+    c->bndWords = bnd + 32;
+    // the heaviest blocks first, so that the last blocks to start are short ones
+    std::vector<int> order(c->blocks.size());
+    for (size_t k = 0; k < order.size(); k++) order[k] = (int)k;
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return work[a] > work[b]; });
+    std::vector<PairBlock> sorted(c->blocks.size());
+    for (size_t k = 0; k < order.size(); k++) sorted[k] = c->blocks[order[k]];
+    c->blocks.swap(sorted);
+    return true;
+}
+
+// Uploads a class's tables and launches it (16 bits: after the gather of its paired stream).
+bool PairsSearch::launch(const Class& c, const std::vector<Scoring>& queries, int wantEnd, const ScoreBounds& b, bool rangeTracking,
+                         long long step, long long rangeLo, const Tables& d) {
+    const Scoring& s0 = queries[0];
+    const int mode = s0.mode, R = kPairsR[c.rIndex];
+    const PairQuery* dQueryTab = d.queryTab;
+    const PairTask* dTasks = d.tasks;
+    const PairBlock* dBlocks = d.blocks;
+    PairsParams p;
+    memset(&p, 0, sizeof(p));
+    if (c.type == 0) {
+        uint16_t* dStream = static_cast<uint16_t*>(alloc(sizeof(uint16_t) * (size_t)c.streamEntries));
+        if (!dStream) return false;
+        if (!launch_gather_pairs(dTasks, (int)c.tasks.size(), db_.dResidues, db_.dOffsets, dStream, stream_)) {
+            set_error("gather of the paired stream failed");
+            return false;
+        }
+        p.stream = dStream;
+    }
+    if (c.maxPasses > 1) {
+        p.bndHalf = c.bndWords;
+        p.bndH = alloc(2 * sizeof(uint32_t) * (size_t)c.bndWords);
+        p.bndF = alloc(2 * sizeof(uint32_t) * (size_t)c.bndWords);
+        if (!p.bndH || !p.bndF) return false;
+    }
+    const int flavor = mode == kModeSW ? (wantEnd ? kFlavorSWEnd : kFlavorSWScore) : kFlavorGlobal;
+    const void* fn = pairs_kernel_fn(c.rIndex, c.type, flavor);
+    if (!allow_full_smem(db_.device, fn, db_.smemLimit)) return false;
+    p.queries = dQueries_; p.matrix = dMatrix_;
+    p.A = s0.A; p.gapOpen = s0.Go; p.gapExt = s0.Ge; p.mode = mode; p.wantEnd = wantEnd;
+    p.queryTab = dQueryTab; p.blockTab = dBlocks; p.tasks = dTasks;
+    p.residues = db_.dResidues; p.offsets = db_.dOffsets;
+    p.outScore = dOut_; p.outEndQ = dOut_ + numPairs_; p.outEndT = dOut_ + 2 * (size_t)numPairs_;
+    // as launch_group: the SW overflow limit, the "no residue" letter and the range tracking of the 16-bit sweeps
+    p.overflowLimit = c.type == 0 ? 32767 - std::max(b.maxEntry, 0) - 1 : (1 << 30);
+    p.padLetterScore = c.type == 0 ? (mode == kModeNW ? 0 : -16384) : 0;
+    const long long margin = (long long)(R + 3) * step;
+    p.rangeHi = rangeTracking ? (int)(32767 - margin) : INT_MAX;
+    p.rangeLo = rangeTracking ? (int)(rangeLo + margin) : INT_MIN;
+    p.one = 1;
+    const size_t smem = (size_t)(c.type == 0 ? 2 : 1) * (s0.A + 1) * ((c.maxG * pairs_rpad(R) + 31) / 32 * 32) * 4;
+    void* args[] = {&p};
+    CUDA_TRY(cudaLaunchKernel(fn, dim3((unsigned)c.blocks.size()), dim3(kPairsThreads), args, smem, stream_));
+    return true;
+}
+
+int PairsSearch::run(const std::vector<Scoring>& queries, int wantEnd, int numPairs, const int* pairQuery, const int* pairTarget,
+                     const SearchOut& out, float* deviceMs, SearchStats* stats) {
+    if (deviceMs) *deviceMs = 0.f;
+    if (numPairs <= 0) return 0;
+    CUDA_TRY_RC(cudaSetDevice(db_.device));
+    const Scoring& s0 = queries[0];  // alphabet, matrix, gaps and mode are the same for every query
+    const int Go = s0.Go, Ge = s0.Ge, mode = s0.mode, nq = (int)queries.size();
+    const bool isSW = mode == kModeSW;
+    ScoreBounds b;
+    if (const int rc = s0.validate(&b)) return rc;
+    if (s0.A == 256 && *db_.hMaxCode >= 255) b.args16 = false;  // code 255 cannot ride in the 16-bit stream (see search())
+    // the routing rule of SearchContext::route and the range limits of SearchContext::Run, for a pair of lengths (Q, T)
+    const long long step = (long long)Go + Ge + b.absEntry, rangeLo = mode == kModeNW ? -28000 : -16383;
+    const bool rangeTracking = !isSW && b.args16 && 40 * step <= 6000;
+    auto fits = [&](int Q, int T, long long lim) {
+        const long long lo = 3LL * Go + ((long long)Q + T) * Ge + b.absEntry;
+        const long long hi = (b.maxEntry > 0 ? (long long)std::min(Q, T) * b.maxEntry : 0) + Go + b.absEntry;
+        return lo <= lim && hi <= lim;
+    };
+    auto ok16 = [&](int Q, int T) {
+        if (isSW) return b.args16;
+        if (!rangeTracking) return b.args16 && fits(Q, T, 16000);
+        const long long border = (long long)Go + (mode == kModeNW ? (long long)std::max(Q, T) : mode == kModeHW ? (long long)Q : 0LL) * Ge;
+        return -border >= rangeLo + 40 * step;
+    };
+    auto ok32 = [&](int Q, int T) { return isSW ? (b.maxEntry > 0 ? (long long)std::min(Q, T) * b.maxEntry : 0) < (1LL << 30) : fits(Q, T, 1LL << 30); };
+
+    // ---- route every pair, group the classes by query (longest target first)
+    std::vector<int> pos((size_t)numPairs);
+    std::vector<char> fixed((size_t)numPairs, 0);
+    std::vector<std::vector<int>> by16((size_t)nq), by32((size_t)nq);
+    for (int k = 0; k < numPairs; k++) {
+        const int q = pairQuery[k], p = db_.lay->pos[pairTarget[k]], T = db_.lay->sortedLen[p], Q = queries[q].Q;
+        pos[k] = p;
+        if (T == 0 || Q <= 0) fixed[k] = 1;  // nothing to align: the defined result, below
+        else if (ok16(Q, T)) by16[q].push_back(k);
+        else if (ok32(Q, T)) by32[q].push_back(k);
+        else return OPAL_B200_ERR_OVERFLOW;
+    }
+    auto longest_first = [&](std::vector<int>& ks) {
+        std::stable_sort(ks.begin(), ks.end(), [&](int a, int c) { return db_.lay->sortedLen[pos[a]] > db_.lay->sortedLen[pos[c]]; });
+    };
+    bool any16 = false, any32 = false;
+    for (int q = 0; q < nq; q++) {
+        longest_first(by16[q]); longest_first(by32[q]);
+        any16 |= !by16[q].empty(); any32 |= !by32[q].empty();
+    }
+    SearchStats st;
+    numPairs_ = numPairs;
+    if (any16 || any32) {
+        Class c16;
+        if (any16 && !plan(0, queries, wantEnd, by16, pos.data(), &c16)) return OPAL_B200_ERR_CUDA;
+        // ---- one upload: [matrix | queries | the 16-bit class's query table, tasks, blocks]
+        std::vector<unsigned char> block;
+        auto put = [&](const void* src, size_t bytes) {
+            const size_t at = block.size();
+            block.resize((at + bytes + 15) / 16 * 16, 0);
+            if (bytes) memcpy(block.data() + at, src, bytes);
+            return at;
+        };
+        const size_t atMatrix = put(s0.entries, sizeof(int) * (size_t)s0.num_entries());
+        const size_t atQueries = block.size();
+        for (const Scoring& s : queries)
+            if (s.Q > 0) block.insert(block.end(), s.query, s.query + s.Q);  // back to back: PairQuery::queryOff
+        put(nullptr, 0);
+        // (every part starts on a 16-byte boundary: the tables are found at the offsets put() returns)
+        auto put_tables = [&](const Class& c) {
+            return std::array<size_t, 3>{put(c.queryTab.data(), sizeof(PairQuery) * c.queryTab.size()),
+                                         put(c.tasks.data(), sizeof(PairTask) * c.tasks.size()),
+                                         put(c.blocks.data(), sizeof(PairBlock) * c.blocks.size())};
+        };
+        auto tables_at = [](const unsigned char* dBase, const std::array<size_t, 3>& at) {
+            return Tables{reinterpret_cast<const PairQuery*>(dBase + at[0]), reinterpret_cast<const PairTask*>(dBase + at[1]),
+                          reinterpret_cast<const PairBlock*>(dBase + at[2])};
+        };
+        const std::array<size_t, 3> at16 = put_tables(c16);
+        unsigned char *dBlock = nullptr, *hBlock = nullptr;
+        int* hOut = nullptr;
+        if (!event_acquire(db_.device, &evStart_) || !event_acquire(db_.device, &evStop_)) return OPAL_B200_ERR_CUDA;
+        if (!upload(block, &dBlock, &hBlock)) return OPAL_B200_ERR_CUDA;
+        dMatrix_ = reinterpret_cast<const int*>(dBlock + atMatrix);
+        dQueries_ = dBlock + atQueries;
+        const size_t outInts = 4 * (size_t)numPairs + 1;
+        if (!(dOut_ = static_cast<int*>(alloc(sizeof(int) * outInts)))) return OPAL_B200_ERR_CUDA;
+        if (!pinned_alloc((void**)&hOut, sizeof(int) * outInts)) return OPAL_B200_ERR_CUDA;
+        pinned_.push_back(hOut);
+        int* dCount = dOut_ + 3 * (size_t)numPairs;
+        CUDA_TRY_RC(cudaMemsetAsync(dOut_, 0, sizeof(int) * (3 * (size_t)numPairs + 1), stream_));  // (0 is never "re-run me")
+        CUDA_TRY_RC(cudaEventRecord(evStart_, stream_));
+        // ---- 16 bits, then the collection of what they could not hold
+        if (any16) {
+            if (!launch(c16, queries, wantEnd, b, rangeTracking, step, rangeLo, tables_at(dBlock, at16))) return OPAL_B200_ERR_CUDA;
+            st.kernelLaunches += 2;
+            st.R = kPairsR[c16.rIndex]; st.G = c16.maxG; st.passes = c16.maxPasses; st.warpsPerPartition = 3; st.groups = 1;
+            collect_flagged_kernel<<<std::min(db_.numSMs * 4, (numPairs + 255) / 256), 256, 0, stream_>>>(dOut_, numPairs, dCount + 1, dCount);
+            CUDA_TRY_RC(cudaGetLastError());
+            CUDA_TRY_RC(cudaMemcpyAsync(hOut, dCount, sizeof(int), cudaMemcpyDeviceToHost, stream_));
+            CUDA_TRY_RC(cudaStreamSynchronize(stream_));
+            const int flagged = hOut[0];
+            if (flagged > 0) {
+                CUDA_TRY_RC(cudaMemcpyAsync(hOut, dCount + 1, sizeof(int) * (size_t)flagged, cudaMemcpyDeviceToHost, stream_));
+                CUDA_TRY_RC(cudaStreamSynchronize(stream_));
+                std::vector<char> touched((size_t)nq, 0);
+                for (int f = 0; f < flagged; f++) { const int k = hOut[f]; by32[pairQuery[k]].push_back(k); touched[pairQuery[k]] = 1; }
+                for (int q = 0; q < nq; q++) if (touched[q]) longest_first(by32[q]);
+                any32 = true;
+                st.rerun32 = flagged;
+            }
+        }
+        // ---- 32 bits: the pairs routed there and the re-runs
+        if (any32) {
+            Class c32;
+            if (!plan(1, queries, wantEnd, by32, pos.data(), &c32)) return OPAL_B200_ERR_CUDA;
+            block.clear();
+            const std::array<size_t, 3> at32 = put_tables(c32);
+            unsigned char *dPlan32 = nullptr, *hPlan32 = nullptr;
+            if (!upload(block, &dPlan32, &hPlan32)) return OPAL_B200_ERR_CUDA;
+            if (!launch(c32, queries, wantEnd, b, rangeTracking, step, rangeLo, tables_at(dPlan32, at32))) return OPAL_B200_ERR_CUDA;
+            st.kernelLaunches++;
+        }
+        CUDA_TRY_RC(cudaEventRecord(evStop_, stream_));
+        // ---- the per-pair results back in one copy
+        CUDA_TRY_RC(cudaMemcpyAsync(hOut, dOut_, sizeof(int) * (wantEnd ? 3 : 1) * (size_t)numPairs, cudaMemcpyDeviceToHost, stream_));
+        CUDA_TRY_RC(cudaStreamSynchronize(stream_));
+        if (deviceMs) CUDA_TRY_RC(cudaEventElapsedTime(deviceMs, evStart_, evStop_));
+        for (int k = 0; k < numPairs; k++)
+            if (!fixed[k] && (hOut[k] == kScoreOverflow || hOut[k] == kScoreNone)) return OPAL_B200_ERR_OVERFLOW;
+        const int *hEndQ = hOut + numPairs, *hEndT = hOut + 2 * (size_t)numPairs;
+        for (int k = 0; k < numPairs; k++)
+            if (!fixed[k])
+                out.put(k, hOut[k], (wantEnd && hEndQ[k] != 0x7fffffff) ? hEndQ[k] : -1, (wantEnd && hEndT[k] != 0x7fffffff) ? hEndT[k] : -1);
+    }
+    for (int k = 0; k < numPairs; k++) {
+        if (!fixed[k]) continue;
+        const int Q = queries[pairQuery[k]].Q, T = db_.lay->sortedLen[pos[k]];
+        int sc = 0, eq = Q - 1, et = T - 1;  // as SearchContext::route (oracle/opal_oracle.c)
+        if (Q > 0 && (mode == kModeNW || mode == kModeHW)) sc = -Go - (Q - 1) * Ge;
+        else if (Q <= 0 && T > 0 && mode == kModeNW) sc = -Go - (T - 1) * Ge;
+        if (isSW) { eq = -1; et = -1; }
+        out.put(k, sc, wantEnd ? eq : -1, wantEnd ? et : -1);
+    }
+    if (stats) *stats = st;
+    return 0;
+}
+
+int DeviceDb::search_pairs(const std::vector<Scoring>& queries, int wantEnd, int numPairs, const int* pairQuery, const int* pairTarget,
+                           const SearchOut& out, float* deviceMs) {
+    if (cudaSetDevice(db_.device) != cudaSuccess) { set_error("cudaSetDevice failed"); return OPAL_B200_ERR_CUDA; }
+    if (!ensure_uploaded()) return OPAL_B200_ERR_CUDA;
+    SearchStats st;
+    int rc;
+    {
+        PairsSearch ps(db_, stream());
+        rc = ps.run(queries, wantEnd, numPairs, pairQuery, pairTarget, out, deviceMs, &st);
+    }
+    contexts_[0]->stats_ = st;
+    return rc;
 }
 
 // ------------------------------------------------------------------ DPX roofline probe

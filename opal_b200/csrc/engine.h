@@ -217,6 +217,48 @@ private:
     bool startRecorded_ = false;
 };
 
+// The pairs path: many queries, each scored against its own list of database entries (pairs_kernel.cuh).  It reads the
+// database arrays through a const reference and owns only the buffers of its call, which it releases when it goes.
+// Stages: route every pair (the defined result of an empty query or target, or the 16- or the 32-bit class), group the
+// classes' pairs by query and plan their geometry, one upload of [matrix | queries | tables], the 16-bit launch, the
+// device-side collection of what 16 bits could not hold, the 32-bit launch, one copy of the per-pair results back.
+struct PairTask;
+struct PairQuery;
+struct PairBlock;
+class PairsSearch {
+public:
+    PairsSearch(const DbArrays& db, cudaStream_t stream) : db_(db), stream_(stream) {}
+    PairsSearch(const PairsSearch&) = delete;
+    ~PairsSearch();
+    // Pair k scores queries[pairQuery[k]] against database entry pairTarget[k] (the database's caller index); its result
+    // goes to out.put(k, ...).  The queries share the alphabet, the matrix, the gap penalties and the mode, and have
+    // passed DeviceDb::check.  0 or an OPAL_B200_ERR_* code (nothing is written unless it is 0).
+    int run(const std::vector<Scoring>& queries, int wantEnd, int numPairs, const int* pairQuery, const int* pairTarget,
+            const SearchOut& out, float* deviceMs, SearchStats* stats);
+
+private:
+    struct Class;  // the pairs of one precision class, grouped and planned (engine.cu)
+    struct Tables { const PairQuery* queryTab; const PairTask* tasks; const PairBlock* blocks; };  // a class's tables on the device
+    bool plan(int type, const std::vector<Scoring>& queries, int wantEnd, const std::vector<std::vector<int>>& byQuery,
+              const int* pos, Class* c);
+    bool launch(const Class& c, const std::vector<Scoring>& queries, int wantEnd, const ScoreBounds& b, bool rangeTracking,
+                long long step, long long rangeLo, const Tables& d);
+    bool upload(const std::vector<unsigned char>& block, unsigned char** dBlock, unsigned char** hBlock);
+    void* alloc(size_t bytes);
+
+    const DbArrays& db_;
+    cudaStream_t stream_;
+    std::vector<void*> device_, pinned_;  // this call's blocks
+    cudaEvent_t evStart_ = nullptr, evStop_ = nullptr;
+    const int* dMatrix_ = nullptr;
+    const uint8_t* dQueries_ = nullptr;
+    int *dOut_ = nullptr;  // [score | endQ | endT | flagged count | flagged slots], numPairs each
+    int numPairs_ = 0;
+};
+bool launch_gather_pairs(const PairTask* tasks, int numTasks, const uint8_t* residues, const long long* offsets, uint16_t* stream,
+                         cudaStream_t st);
+const void* pairs_kernel_fn(int rIndex, int type, int flavor);  // pairs.cu: [strip height index][Packed16 / Scalar32][flavor]
+
 // A resident database and the search contexts that run on it.
 class DeviceDb {
 public:
@@ -247,6 +289,9 @@ public:
     // The checks a search makes before it sweeps: Scoring::validate, then (for a search that sweeps at all) the
     // database's residue codes against the alphabet length.  0 or an OPAL_B200_ERR_* code.
     int check(const Scoring& s);
+    // PairsSearch::run on the first context's stream, once the upload has finished; the call's statistics become stats().
+    int search_pairs(const std::vector<Scoring>& queries, int wantEnd, int numPairs, const int* pairQuery, const int* pairTarget,
+                     const SearchOut& out, float* deviceMs);
 
     int size() const { return db_.n; }
     long long residues() const { return db_.totalResidues; }

@@ -62,6 +62,10 @@ class OpalB200(OpalCLibrary):
         L.opalb200_db_search_batch_topk.restype = ci
         L.opalb200_db_search_batch_topk_pssm.argtypes = [vp, ci, vp, vp, vp, vp, ci, ci, ci, ci, ci, vp, vp, ctypes.POINTER(ci), ci]
         L.opalb200_db_search_batch_topk_pssm.restype = ci
+        L.opalb200_db_search_pairs.argtypes = [vp, ci, vp, vp, ci, vp, vp, ci, ci, vp, ci, ci, ci, vp, vp, vp, vp]
+        L.opalb200_db_search_pairs.restype = ci
+        L.opalb200_db_search_pairs_results.argtypes = [vp, ci, vp, vp, ci, vp, vp, ci, ci, vp, ci, vp, ci, ci]
+        L.opalb200_db_search_pairs_results.restype = ci
         L.opalb200_db_last_stats.argtypes = [vp] + [ctypes.POINTER(ci)] * 7
         L.opalb200_db_last_stats.restype = None
         L.opalb200_db_last_folded.argtypes = [vp]
@@ -353,6 +357,53 @@ class ResidentDb:
         return self._batch_topk(lambda idx, rp, found: self.eng.lib.opalb200_db_search_batch_topk_pssm(
             self.handle, ns, None if qbufs is None else qptrs.ctypes.data, ptrs.ctypes.data, qlens.ctypes.data, mdb.ctypes.data, A,
             int(gap_open), int(gap_ext), int(search_type), int(k), idx, rp, found, int(in_flight)), ns, k)
+
+    # ---- (query, target) pairs: pair p scores queries[pair_query[p]] against database entry pair_target[p]
+    @staticmethod
+    def _pairs_args(queries, pair_query, pair_target):
+        """(arrays kept alive, query pointers, query lengths, pair_query, pair_target, numPairs)"""
+        qs = [np.ascontiguousarray(q, dtype=np.uint8) for q in queries]
+        bufs = [q if q.size else np.zeros(1, dtype=np.uint8) for q in qs]
+        ptrs = np.array([b.ctypes.data for b in bufs] or [0], dtype=np.uint64)
+        qlens = np.array([q.size for q in qs] or [0], dtype=np.int32)
+        pq = np.ascontiguousarray(pair_query, dtype=np.int32).ravel()
+        pt = np.ascontiguousarray(pair_target, dtype=np.int32).ravel()
+        if pq.size != pt.size:
+            raise ValueError("pair_query and pair_target must have the same length")
+        return bufs, ptrs, qlens, (pq if pq.size else np.zeros(1, dtype=np.int32)), (pt if pt.size else np.zeros(1, dtype=np.int32)), int(pq.size)
+
+    def search_pairs(self, queries, pair_query, pair_target, gap_open, gap_ext, score_matrix, alphabet_length, search_type, mode):
+        """opalb200_db_search_pairs. Returns (rc, scores, endQuery, endTarget, device_ms); arrays are indexed by pair."""
+        keep, ptrs, qlens, pq, pt, m = self._pairs_args(queries, pair_query, pair_target)
+        sm = np.ascontiguousarray(score_matrix, dtype=np.int32).ravel()
+        sc = np.zeros(max(m, 1), dtype=np.int32)
+        eq = np.full(max(m, 1), -1, dtype=np.int32)
+        et = np.full(max(m, 1), -1, dtype=np.int32)
+        ms = ctypes.c_float(0)
+        if isinstance(mode, str):
+            mode = MODES[mode]
+        rc = self.eng.lib.opalb200_db_search_pairs(
+            self.handle, len(keep), ptrs.ctypes.data, qlens.ctypes.data, m, pq.ctypes.data, pt.ctypes.data, int(gap_open), int(gap_ext),
+            sm.ctypes.data, int(alphabet_length), int(search_type), int(mode), sc.ctypes.data, eq.ctypes.data, et.ctypes.data,
+            ctypes.byref(ms))
+        del keep
+        return rc, sc[:m], eq[:m], et[:m], float(ms.value)
+
+    def search_pairs_results(self, queries, pair_query, pair_target, gap_open, gap_ext, score_matrix, alphabet_length, search_type,
+                             mode, results=None):
+        """opalb200_db_search_pairs_results: one record per pair (`results` = prefilled records to reuse). Returns (rc, results)."""
+        keep, ptrs, qlens, pq, pt, m = self._pairs_args(queries, pair_query, pair_target)
+        sm = np.ascontiguousarray(score_matrix, dtype=np.int32).ravel()
+        if results is None:
+            results = new_results(m)
+        rp = result_pointers(results) if m else np.zeros(1, dtype=np.uint64)
+        if isinstance(mode, str):
+            mode = MODES[mode]
+        rc = self.eng.lib.opalb200_db_search_pairs_results(
+            self.handle, len(keep), ptrs.ctypes.data, qlens.ctypes.data, m, pq.ctypes.data, pt.ctypes.data, int(gap_open), int(gap_ext),
+            sm.ctypes.data, int(alphabet_length), rp.ctypes.data, int(search_type), int(mode))
+        del keep
+        return rc, results
 
     def devices(self):
         return int(self.eng.lib.opalb200_db_devices(self.handle))
